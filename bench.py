@@ -4,6 +4,7 @@ uncompressed data, with the HBM roofline of the dominant kernel and the referenc
 timed on the same box.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--size-gb G]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: dexqv (statistics scan, code construction,
 encode) of a synthetic .quiva shard followed by undexqv of the result, the decoder finding the
@@ -15,6 +16,9 @@ value   uncompressed GB/s summed over both directions (2*U / t), inputs resident
         with CUDA events on the library's stream, max over ranks.
 e2e     the same step through the host-buffer C ABI (dx_dexqv_host / dx_undexqv_host): pinned
         host -> device copies of the inputs and device -> host copies of the results included.
+
+--dump-outputs DIR writes what the last timed step produced (see dump_outputs) so that two builds
+can be compared output for output; the inputs are seeded, so equal arguments give equal inputs.
 
 Control flow rule (round 1 died of breaking it): every collective is issued from the top level of
 run_ours() through `Comm`, by every rank, unconditionally.  Nothing under `if rank == 0` may
@@ -122,6 +126,48 @@ def workload_config(args):
                         ".quiva per GPU (5 QV streams)",
             "uncompressed_bytes_per_gpu": int(args.size_gb * GB), "shards": args.gpus,
             "l2": "inputs (2 GB) exceed the 126 MB L2; no explicit flush"}
+
+
+# --dump-outputs: per output and rank, a seeded sample of up to 4 Mi bytes (float32, 16 MB) and the
+# exact sums of up to 1 Mi contiguous blocks (float64, 8 MB), divided by the number of ranks: two
+# outputs stay under 64 MB in all.  The sample shows where bytes differ; the block sums cover every
+# byte.  The sample positions are drawn from [0, next power of two >= length) and those past the
+# end dropped, so outputs of different lengths in the same power-of-two range are sampled at the
+# same positions, and their samples agree element by element up to the shorter one.
+DUMP_SAMPLE, DUMP_BLOCKS = 1 << 22, 1 << 20
+
+
+def dump_outputs(outdir, outputs, rank, world):
+    """outputs: {name: 1-D uint8 tensor}.  Writes <name>_sample.npy, <name>_block_sums.npy and
+    lengths.npy (the byte length of each output, in order) into outdir; with several ranks every
+    file name ends in _rank<r>."""
+    import numpy as np
+    import torch
+    os.makedirs(outdir, exist_ok=True)
+    tag = f"_rank{rank}" if world > 1 else ""
+    lengths = []
+    for name, t in outputs.items():
+        n = t.numel()
+        lengths.append(n)
+        k = DUMP_SAMPLE // world
+        if n <= k:
+            pos = np.arange(n)
+        else:
+            # k draws below the power of two, repeats merged (a permutation of the range, as
+            # choice(replace=False) makes for small ranges, would cost up to 1 GB of host memory)
+            top = 1 << (n - 1).bit_length()
+            pos = np.unique(np.random.default_rng(rank).integers(0, top, k))
+            pos = pos[pos < n]
+        sample = t[torch.from_numpy(pos).to(t.device)].to(torch.float32).cpu().numpy()
+        b = max(1, -(-n // (DUMP_BLOCKS // world)))          # block length: at most that many blocks
+        full = t[: n - n % b].view(-1, b)
+        sums = [full[i: i + 4096].to(torch.int32).sum(1).cpu().numpy() for i in range(0, full.shape[0], 4096)]
+        if n % b:
+            sums.append(np.array([int(t[n - n % b:].to(torch.int32).sum())]))
+        np.save(os.path.join(outdir, f"{name}_sample{tag}.npy"), sample)
+        np.save(os.path.join(outdir, f"{name}_block_sums{tag}.npy"),
+                np.concatenate(sums).astype(np.float64) if sums else np.zeros(0))
+    np.save(os.path.join(outdir, f"lengths{tag}.npy"), np.array(lengths, dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -510,6 +556,9 @@ def run_ours(args, env=None, out=print):
     sampler.begin()
     ms = env.timed_ms(k_steps)
     sampler.end()
+    if args.dump_outputs:                          # before the timings below overwrite the buffers
+        dump_outputs(args.dump_outputs, {"dexqv": sh.enc[: sh.st["img_len"]],
+                                         "undexqv": sh.back[: sh.st["out_len"]]}, rank, world)
     comm.barrier()
     clocks = sampler.stop()
     launches = ctx.launch_count()
@@ -748,7 +797,13 @@ def parse_args(argv=None):
     ap.add_argument("--cpu-sample-mb", type=float, default=64.0, help="per process")
     ap.add_argument("--no-extras", action="store_true", help="skip the dexta/undexta side numbers")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write samples of the last timed step's .dexqv image and decoded text as .npy")
     args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU path's outputs; the reference arm writes none")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     return args
 

@@ -17,10 +17,3 @@ def orc():
     from oracle import orc as _orc
     _orc.lib()
     return _orc
-
-
-@pytest.fixture(scope="session")
-def ref(orc):
-    if not orc.have_ref():
-        pytest.skip("oracle/_ref reference tools not built (no /root/reference here)")
-    return orc

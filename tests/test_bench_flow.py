@@ -234,3 +234,51 @@ def test_single_rank_flow_and_config_matches_reference_arm(orc, monkeypatch):
     # the two arms must print the same config object (the driver compares them)
     assert d["config"] == bench.workload_config(bench.parse_args(["--impl", "reference", "--size-gb", "0.02"]))
     assert d["roofline"]["traffic_source"] is None or "profiles/" in d["roofline"]["traffic_source"]
+
+
+def test_dump_outputs_hold_the_timed_paths_image_and_text(orc, monkeypatch, tmp_path):
+    """--dump-outputs: the stand-in's image is header + text and its decode is the text, both
+    small enough for the sample to be the whole output.  (The stand-in gives the same output at
+    every step, so this checks what is dumped and how, not from which step.)"""
+    sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setenv("RANK", "0"); monkeypatch.setenv("WORLD_SIZE", "1"); monkeypatch.setenv("LOCAL_RANK", "0")
+    with pytest.raises(SystemExit):
+        bench.parse_args(["--impl", "reference", "--dump-outputs", str(tmp_path)])
+    args = bench.parse_args(["--steps", "2", "--size-gb", "0.02", "--parity-mb", "8", "--no-cpu",
+                             "--no-extras", "--dump-outputs", str(tmp_path)])
+    bench.run_ours(args, env=FakeEnv(1), out=[].append)
+    text = FakeEnv(1).make_quiva(100, 0.02e9)[0].numpy()
+    files = sorted(os.listdir(tmp_path))
+    assert files == ["dexqv_block_sums.npy", "dexqv_sample.npy", "lengths.npy",
+                     "undexqv_block_sums.npy", "undexqv_sample.npy"]
+    assert sum(os.path.getsize(tmp_path / f) for f in files) <= 64 << 20
+    img, dec = np.load(tmp_path / "dexqv_sample.npy"), np.load(tmp_path / "undexqv_sample.npy")
+    assert img.dtype == dec.dtype == np.float32
+    assert np.array_equal(dec, text) and np.array_equal(img[len(img) - len(text):], text)
+    assert np.load(tmp_path / "lengths.npy").tolist() == [len(img), len(text)]
+    for name, want in (("dexqv", img), ("undexqv", dec)):
+        sums = np.load(tmp_path / f"{name}_block_sums.npy")
+        assert sums.dtype == np.float64 and sums.sum() == want.astype(np.int64).sum()
+
+
+def test_dump_outputs_sample_large_outputs_the_same_way_every_time(monkeypatch, tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    import torch
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 1000)
+    monkeypatch.setattr(bench, "DUMP_BLOCKS", 64)
+    t = torch.from_numpy(np.random.default_rng(3).integers(0, 256, 100_003, dtype=np.uint8))
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"x": t}, rank=1, world=2)
+    a = {f: np.load(tmp_path / "a" / f) for f in sorted(os.listdir(tmp_path / "a"))}
+    assert sorted(a) == ["lengths_rank1.npy", "x_block_sums_rank1.npy", "x_sample_rank1.npy"]
+    for f, v in a.items():
+        assert np.array_equal(v, np.load(tmp_path / "b" / f)), f
+    assert 250 <= len(a["x_sample_rank1.npy"]) <= 500 and len(a["x_block_sums_rank1.npy"]) <= 32
+    assert a["x_block_sums_rank1.npy"].sum() == int(t.sum()) and a["lengths_rank1.npy"].tolist() == [100_003]
+    # a shorter output in the same power-of-two range is sampled at the same positions
+    bench.dump_outputs(str(tmp_path / "c"), {"x": t[:90_000]}, rank=1, world=2)
+    c = np.load(tmp_path / "c" / "x_sample_rank1.npy")
+    assert 0 < len(c) < len(a["x_sample_rank1.npy"])
+    assert np.array_equal(c, a["x_sample_rank1.npy"][: len(c)])

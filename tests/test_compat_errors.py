@@ -4,12 +4,16 @@ and errors follow the reference's two conventions (DB.h:28-47): batch = message 
 -DINTERACTIVE = message in Ebuffer + documented error value.  No codec work runs here: without a
 GPU the codec calls must fail loudly in either convention."""
 import ctypes
+import json
 import os
 import subprocess
 import sys
 import textwrap
 
 import pytest
+
+from tests import refgold
+from tests.refgold import check
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIBDIR = os.path.join(ROOT, "dextractor_b200")
@@ -147,16 +151,21 @@ def test_batch_codec_calls_exit_without_a_gpu(tmp_path):
     assert "no usable CUDA device" in r.stderr
 
 
-def test_path_helpers_match_the_reference(ref):
+def _ref_lib(orc, name):
+    """the reference's own DB.c + QV.c as compiled into oracle/_ref, or None where it is not built"""
+    path = os.path.join(ROOT, "oracle", "_ref", name)
+    return ctypes.CDLL(path) if orc.have_ref() and os.path.exists(path) else None
+
+
+def test_path_helpers_match_the_reference(orc):
     """PathTo / Root / Catenate / Numbered_Suffix (DB.c:112-202) of libdexcompat.so against the
-    reference's own, compiled from DB.c into oracle/_ref/libdbqv_ref.so."""
-    path = os.path.join(ROOT, "oracle", "_ref", "libdbqv_ref.so")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref/libdbqv_ref.so not built")
-    R, L = ctypes.CDLL(path), _load("libdexcompat.so")
+    reference's own, compiled from DB.c into oracle/_ref/libdbqv_ref.so (or their stored results)."""
+    R, L = _ref_lib(orc, "libdbqv_ref.so"), _load("libdexcompat.so")
     libc = ctypes.CDLL(None)
     libc.free.argtypes = [ctypes.c_void_p]
     for lib in (R, L):
+        if lib is None:
+            continue
         lib.PathTo.restype = lib.Root.restype = ctypes.c_void_p
         lib.PathTo.argtypes = [ctypes.c_char_p]
         lib.Root.argtypes = [ctypes.c_char_p, ctypes.c_char_p]
@@ -169,36 +178,34 @@ def test_path_helpers_match_the_reference(ref):
         bufs = [ctypes.create_string_buffer(x) if isinstance(x, bytes) else x for x in a]
         p = getattr(lib, fn)(*[ctypes.cast(b, ctypes.c_char_p) if b is not None else None for b in bufs])
         if not p:
-            return None
+            return repr(None)
         s = ctypes.string_at(p)
         libc.free(p)
-        return s
+        return repr(s)
 
     names = [b"x", b"x.fasta", b"x.FASTA", b"dir/x.fasta", b"/x.fasta", b"/abs/dir.d/x.y.z", b".fasta",
              b"a.fasta.fasta", b"dir.fasta/x", b"", b"trailing/", b"x.quiva", b"./x", b"../x.dexqv"]
     for n in names:
-        assert owned(L, "PathTo", n) == owned(R, "PathTo", n), n
+        check(f"PathTo {n!r}", owned(L, "PathTo", n), lambda: owned(R, "PathTo", n), R is not None)
         for suf in (b".fasta", b".quiva", b".dexqv", b"", None):
-            assert owned(L, "Root", n, suf) == owned(R, "Root", n, suf), (n, suf)
+            check(f"Root {n!r} {suf!r}", owned(L, "Root", n, suf), lambda: owned(R, "Root", n, suf), R is not None)
     for a in ((b".", b"/", b"x", b".dexqv"), (b"", b"", b"", b""), (b"/abs", b"/", b"r" * 500, b".q")):
-        assert L.Catenate(*a) == R.Catenate(*a)
+        check(f"Catenate {a!r}", repr(L.Catenate(*a)), lambda: repr(R.Catenate(*a)), R is not None)
     for a in ((b"_", 17, b".las"), (b"", -3, b""), (b"x" * 300, 2**31 - 1, b"y")):
-        assert L.Numbered_Suffix(*a) == R.Numbered_Suffix(*a)
+        check(f"Numbered_Suffix {a!r}", repr(L.Numbered_Suffix(*a)), lambda: repr(R.Numbered_Suffix(*a)), R is not None)
     assert L.Catenate(None, b"", b"", b"") is None and L.Numbered_Suffix(None, 1, b"") is None
 
 
-def test_line_reader_matches_the_interactive_reference(ref, shim, tmp_path):
+def test_line_reader_matches_the_interactive_reference(orc, shim, tmp_path):
     """Read_Lines of libdexcompat_i.so beside the reference's own (QV.c:751-798 compiled with
-    -DINTERACTIVE into oracle/_ref/libdbqv_ref_i.so): same return values, same lines, same line
-    counter, same Ebuffer text, call by call over well-formed and broken inputs."""
-    path = os.path.join(ROOT, "oracle", "_ref", "libdbqv_ref_i.so")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref/libdbqv_ref_i.so not built")
-    R = ctypes.CDLL(path)
-    R.Read_Lines.argtypes = [ctypes.c_void_p, ctypes.c_int]
-    R.QVentry.restype = ctypes.c_void_p
+    -DINTERACTIVE into oracle/_ref/libdbqv_ref_i.so, or its stored results): same return values,
+    same lines, same line counter, same Ebuffer text, call by call over well-formed and broken inputs."""
+    R = _ref_lib(orc, "libdbqv_ref_i.so")
+    if R is not None:
+        R.Read_Lines.argtypes = [ctypes.c_void_p, ctypes.c_int]
+        R.QVentry.restype = ctypes.c_void_p
+        rbuf = (ctypes.c_char * 1000).in_dll(R, "Ebuffer")
     shim.L.QVentry.restype = ctypes.c_void_p
-    rbuf = (ctypes.c_char * 1000).in_dll(R, "Ebuffer")
     files = {
         "good": b"@m/1/0_4 RQ=0.850\nabcd\nefgh\nijkl\nmnop\nqrst\n@m/2/0_2 RQ=0.8\nab\ncd\nef\ngh\nij\n",
         "ragged": b"@h\nabc\nab\nabc\nabc\nabc\n",
@@ -208,26 +215,31 @@ def test_line_reader_matches_the_interactive_reference(ref, shim, tmp_path):
         "empty": b"",
         "long": b"@h\n" + b"".join(bytes([70 + k]) * 120_000 + b"\n" for k in range(5)),
     }
+
+    def step(lib, ebuf, f, nl):
+        ebuf.value = b""
+        a = lib.Read_Lines(f, nl)
+        # the first line read sits at QVentry(); the reference keeps the newline, so compare up to it
+        line = refgold.sha(ctypes.string_at(lib.QVentry(), a)) if a >= 0 else None
+        return json.dumps([a, ebuf.value.decode("latin-1"), lib.Get_QV_Line(), line])
+
     for name, data in files.items():
         p = tmp_path / name
         p.write_bytes(data)
-        fr, fo = shim.open(p), shim.open(p)
-        R.Set_QV_Line(0); shim.L.Set_QV_Line(0)
-        for step in range(8):
-            nl = 1 if step % 2 == 0 else 5
-            rbuf.value = b""; shim.ebuf.value = b""
-            a, b = R.Read_Lines(fr, nl), shim.L.Read_Lines(fo, nl)
-            assert a == b, (name, step, a, b)
-            assert rbuf.value == shim.ebuf.value, (name, step)
-            assert R.Get_QV_Line() == shim.L.Get_QV_Line(), (name, step)
-            if a >= 0:
-                # the first line read sits at QVentry(); the reference keeps the newline, so compare up to it
-                ra = ctypes.string_at(R.QVentry(), a)
-                rb = ctypes.string_at(shim.L.QVentry(), a)
-                assert ra == rb, (name, step)
-            if a < 0:
+        fo = shim.open(p)
+        fr = shim.open(p) if R is not None else None
+        shim.L.Set_QV_Line(0)
+        if R is not None:
+            R.Set_QV_Line(0)
+        for k in range(8):
+            nl = 1 if k % 2 == 0 else 5
+            got = step(shim.L, shim.ebuf, fo, nl)
+            check(f"Read_Lines {name} {k}", got, lambda: step(R, rbuf, fr, nl), R is not None)
+            if json.loads(got)[0] < 0:
                 break
-        shim.libc.fclose(fr); shim.libc.fclose(fo)
+        shim.libc.fclose(fo)
+        if fr is not None:
+            shim.libc.fclose(fr)
     shim.L.QVentry.restype = ctypes.c_char_p
 
 
@@ -237,16 +249,14 @@ class _QVcoding(ctypes.Structure):                          # QV.h:31-42
 
 
 @pytest.mark.parametrize("seed", range(6))
-def test_coding_header_io_matches_the_reference_functions(ref, tmp_path, seed):
+def test_coding_header_io_matches_the_reference_functions(orc, tmp_path, seed):
     """Read_QVcoding + Write_QVcoding of libdexcompat.so (host work) beside the reference's own
-    functions on real .dexqv files: same delChar / subChar / flip / prefix, same file position after
-    the read, same bytes written back -- and those are the bytes of the file's header."""
+    functions (or their stored results) on real .dexqv files: same delChar / subChar / flip / prefix,
+    same file position after the read, same bytes written back -- and those are the bytes of the
+    file's header."""
     from tests import fuzz
-    path = os.path.join(ROOT, "oracle", "_ref", "libdbqv_ref.so")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref/libdbqv_ref.so not built")
     text, _ = fuzz.fuzz_quiva(seed)
-    data = ref.dexqv(text, lossy=bool(seed & 1))
+    data = orc.dexqv(text, lossy=bool(seed & 1))
     src = tmp_path / "f.dexqv"
     src.write_bytes(data)
     libc = ctypes.CDLL(None)
@@ -256,8 +266,8 @@ def test_coding_header_io_matches_the_reference_functions(ref, tmp_path, seed):
         fn.argtypes = [ctypes.c_void_p]
     libc.fseek.argtypes = [ctypes.c_void_p, ctypes.c_long, ctypes.c_int]
     libc.ftell.restype = ctypes.c_long
-    seen = []
-    for lib in (ctypes.CDLL(path), _load("libdexcompat.so")):
+
+    def header_io(lib):
         lib.Read_QVcoding.restype = ctypes.POINTER(_QVcoding)
         lib.Read_QVcoding.argtypes = [ctypes.c_void_p]
         lib.Write_QVcoding.argtypes = [ctypes.c_void_p, ctypes.POINTER(_QVcoding)]
@@ -271,9 +281,16 @@ def test_coding_header_io_matches_the_reference_functions(ref, tmp_path, seed):
         g = libc.fopen(str(out).encode(), b"w")
         lib.Write_QVcoding(g, c)
         libc.fclose(g)
-        seen.append((c.contents.delChar, c.contents.subChar, c.contents.flip, c.contents.prefix,
-                     pos, out.read_bytes()))
+        seen = (c.contents.delChar, c.contents.subChar, c.contents.flip, c.contents.prefix.decode("latin-1"),
+                pos, out.read_bytes())
         lib.Free_QVcoding(c)                                 # frees prefix too (QV.c:1324-1334)
         libc.fclose(f)
-    assert seen[0] == seen[1]
-    assert seen[0][5] == data[2:seen[0][4]]
+        return seen
+
+    def value(seen):
+        return json.dumps([*seen[:5], refgold.sha(seen[5])])
+
+    R = _ref_lib(orc, "libdbqv_ref.so")
+    mine = header_io(_load("libdexcompat.so"))
+    check(f"QVcoding header io seed={seed}", value(mine), lambda: value(header_io(R)), R is not None)
+    assert mine[5] == data[2:mine[4]]

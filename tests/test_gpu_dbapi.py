@@ -1,6 +1,8 @@
 """The in-memory QV.h calls the way the Dazzler DB code uses them (SURVEY 8f rows 1-2), through
 libdexcompat.so on the GPU, call by call against the reference's own functions compiled into
-oracle/_ref/libdbqv_ref.so:
+oracle/_ref/libdbqv_ref.so or, where they are not built, against their stored results
+(tests/golden/reference_digests.json); the .qvs files the other tests read are then written by
+libdexcompat.so, whose writer the first test finds byte-equal to the reference's:
 
   * dex2DB's write path (dex2DB.c:506-567, 604-622): QVcoding_Scan1(0,...) reset, QVcoding_Scan1 per
     read, Create_QVcoding, prefix ".qvs", Write_QVcoding, Compress_Next_QVentry1 per read with
@@ -11,12 +13,15 @@ oracle/_ref/libdbqv_ref.so:
   * the batch form of the same (dx_qv_load_entries_dev): every entry of a .qvs in one call.
 """
 import ctypes as C
+import json
 import os
 
 import numpy as np
 import pytest
 
 from dextractor_b200 import synth
+from tests import refgold
+from tests.refgold import check
 
 pytestmark = pytest.mark.gpu
 
@@ -61,11 +66,11 @@ def _lib(path):
 
 
 @pytest.fixture(scope="module")
-def libs():
+def libs(orc):
+    """(libdexcompat.so, the reference's libdbqv_ref.so or None where it is not built)"""
     ref = os.path.join(ROOT, "oracle", "_ref", "libdbqv_ref.so")
-    if not os.path.exists(ref):
-        pytest.skip("oracle/_ref/libdbqv_ref.so not built (no /root/reference here)")
-    return _lib(os.path.join(ROOT, "dextractor_b200", "libdexcompat.so")), _lib(ref)
+    have = orc.have_ref() and os.path.exists(ref)
+    return _lib(os.path.join(ROOT, "dextractor_b200", "libdexcompat.so")), (_lib(ref) if have else None)
 
 
 def _reads(seed, lengths):
@@ -105,39 +110,49 @@ def _read_entry(L, f, coding, rlen):
 
 
 def test_dex2db_write_order_and_load_qventry(libs, tmp_path):
+    """against the reference's own calls, or where they are not built, against what they gave
+    (tests/golden/reference_digests.json): the .qvs bytes, every coff, every entry read back"""
     gpu, ref = libs
     rng = np.random.default_rng(9)
     lengths = [int(x) for x in rng.integers(1, 9000, size=70)] + [1, 2, 3, 4, 31, 32, 33]
     reads = _reads(9, lengths)
-    out = {}
-    for name, L in (("gpu", gpu), ("ref", ref)):
+
+    def write(name, L):
         path = tmp_path / f"{name}.qvs"
         f = libc.fopen(str(path).encode(), b"w")
         coff = _write_block(L, f, reads)
         end = libc.ftello(f)
         libc.fclose(f)
-        out[name] = (path.read_bytes(), coff, end)
-    assert out["gpu"][1] == out["ref"][1], "ftello after Compress_Next_QVentry1 differs (DAZZ_READ.coff)"
-    assert out["gpu"][0] == out["ref"][0], "the .qvs bytes differ"
+        return path, coff, end
 
-    # Load_QVentry: Read_QVcoding once, then fseeko(coff) + Uncompress_Next_QVentry in any order
-    path = tmp_path / "ref.qvs"
-    coff = out["ref"][1]
+    mine = write("gpu", gpu)
+    theirs = write("ref", ref) if ref is not None else None
+    check("dex2DB coff", json.dumps([mine[1], mine[2]]), lambda: json.dumps([theirs[1], theirs[2]]),
+          ref is not None)                               # ftello after Compress_Next_QVentry1 (DAZZ_READ.coff)
+    check("dex2DB .qvs", mine[0].read_bytes(), lambda: theirs[0].read_bytes(), ref is not None)
+
+    # Load_QVentry: Read_QVcoding once, then fseeko(coff) + Uncompress_Next_QVentry in any order, on
+    # the reference's file (or, without it, ours: the check above found the two equal)
+    path, coff = (theirs or mine)[:2]
     order = list(rng.permutation(len(reads)))
-    got = {}
-    for name, L in (("gpu", gpu), ("ref", ref)):
+
+    def load(L):
         f = libc.fopen(str(path).encode(), b"r")
         cd = L.Read_QVcoding(f)
         assert cd
         res = []
         for i in order:
             libc.fseeko(f, coff[i], 0)
-            res.append(_read_entry(L, f, cd, len(reads[i][0])))
+            rc, lines, pos = _read_entry(L, f, cd, len(reads[i][0]))
+            res.append(json.dumps([rc, refgold.sha(b"\n".join(lines)), pos]))
         libc.fclose(f)
-        got[name] = res
+        return res
+
+    got = load(gpu)
+    want = load(ref) if ref is not None else None
     for k, i in enumerate(order):
-        assert got["gpu"][k] == got["ref"][k], f"entry {i}"
-        assert got["ref"][k][0] == 0
+        check(f"Load_QVentry {i}", got[k], lambda: want[k], ref is not None)
+        assert json.loads(got[k])[0] == 0
 
 
 def test_two_codings_in_one_qvs(libs, tmp_path):
@@ -151,9 +166,11 @@ def test_two_codings_in_one_qvs(libs, tmp_path):
     heads, coffs = [], []
     for b in blocks:
         heads.append(libc.ftello(f))
-        coffs.append(_write_block(ref, f, b))
+        coffs.append(_write_block(ref or gpu, f, b))       # the reference writes it where it is built
     libc.fclose(f)
     for name, L in (("gpu", gpu), ("ref", ref)):
+        if L is None:
+            continue
         f = libc.fopen(str(path).encode(), b"r")
         codings = []
         for h in heads:
@@ -188,7 +205,7 @@ def test_batched_load_of_a_qvs(libs, tmp_path):
     reads = _reads(33, lengths)
     path = tmp_path / "b.qvs"
     f = libc.fopen(str(path).encode(), b"w")
-    coff = _write_block(ref, f, reads)
+    coff = _write_block(ref or gpu, f, reads)         # the reference writes it where it is built
     libc.fclose(f)
     data = path.read_bytes()
     cd, prefix, used = dxl.read_coding(data)

@@ -35,9 +35,14 @@ def test_fixture_is_what_the_manifest_says(name):
 
 
 @pytest.mark.parametrize("name", FILES)
-def test_reference_decodes_the_fixture_to_the_text(ref, name):
+def test_reference_decodes_the_fixture_to_the_text(orc, name):
+    """the reference undexqv (oracle/_ref) decodes the fixture to the text; where it is not built,
+    the oracle must give the text the reference gave when the fixture was made (decoded_sha256)"""
     b = open(os.path.join(HERE, name), "rb").read()
-    assert ref.ref_tool("undexqv", b)[0] == _text(ref)
+    if orc.have_ref():
+        assert orc.ref_tool("undexqv", b)[0] == _text(orc)
+    else:
+        assert hashlib.sha256(orc.undexqv(b)).hexdigest() == MAN["decoded_sha256"]
 
 
 @pytest.mark.gpu
