@@ -35,9 +35,12 @@ struct DxPhases
 //  errors, context, arena
 // ================================================================================================
 
+// every DX_E_CAP failure clears the size kept for dx_needed_bytes, so a caller never reallocates from
+// what an earlier call needed; dx_fail_cap then sets it when the call knows its size
 int dx_fail(dx_ctx *ctx, int code, const char *fmt, ...)
 { if (ctx != NULL)
-    { va_list ap;
+    { if (code == DX_E_CAP) ctx->need_bytes = 0;
+      va_list ap;
       va_start(ap,fmt);
       vsnprintf(ctx->err,sizeof(ctx->err),fmt,ap);
       va_end(ap);
@@ -47,8 +50,9 @@ int dx_fail(dx_ctx *ctx, int code, const char *fmt, ...)
 
 // the output buffer is too small: the size the call needs is kept for dx_needed_bytes
 int dx_fail_cap(dx_ctx *ctx, size_t need, size_t cap)
-{ ctx->need_bytes = need;
-  return dx_fail(ctx,DX_E_CAP,"output needs %zu bytes, buffer has %zu",need,cap);
+{ dx_fail(ctx,DX_E_CAP,"output needs %zu bytes, buffer has %zu",need,cap);
+  ctx->need_bytes = need;
+  return DX_E_CAP;
 }
 
 int dx_cuda_fail(dx_ctx *ctx, cudaError_t e, const char *what)
@@ -195,7 +199,7 @@ extern "C" int dx_profile_report(dx_ctx *ctx, char *buf, size_t cap)
   size_t at = 0;
   for (const Acc &a : acc)
     { int w = snprintf(buf+at,cap-at,"%s %d %.6f\n",a.name,a.calls,a.ms);
-      if (w < 0 || (size_t) w >= cap-at) return DX_E_CAP;
+      if (w < 0 || (size_t) w >= cap-at) return dx_fail(ctx,DX_E_CAP,"profile report needs more than %zu bytes",cap);
       at += (size_t) w;
     }
   return DX_OK;
@@ -1194,13 +1198,18 @@ extern "C" int dx_dexqv_dev(dx_ctx *ctx, const uint8_t *d_text, size_t n, int lo
     const uint16_t key = 0x55aa;                                         // dexqv.c:105-106
     memcpy(fh.data(),&key,2);
     if ((rc = dx_qv_write_coding(cd,(const char *) head.data(),(int) (sl - head.data()),
-                                 fh.data()+2,fh.size()-2,&hlen)) != DX_OK) goto done;
+                                 fh.data()+2,fh.size()-2,&hlen)) != DX_OK)
+      { dx_fail(ctx,rc,"could not write the coding header");
+        goto done;
+      }
     hlen += 2;
   }
-  if (hlen > cap) { rc = dx_fail(ctx,DX_E_CAP,"output buffer too small"); goto done; }
+  if (hlen > cap) { rc = dx_fail(ctx,DX_E_CAP,"output buffer too small for the coding header"); goto done; }
   if ((rc = upload(ctx,d_out,fh.data(),hlen)) != DX_OK) goto done;
   if ((rc = dx_qv_encode_dev(ctx,d_text,n,cd,lossy,0,d_out+hlen,cap-hlen,&body,NULL,NULL,0)) != DX_OK)
-    goto done;
+    { if (rc == DX_E_CAP && ctx->need_bytes > 0) ctx->need_bytes += hlen;   // the body's need: add the header
+      goto done;
+    }
   if ((rc = dx_sync(ctx)) != DX_OK) goto done;
   *out_len = hlen + body;
 done:
@@ -1576,6 +1585,11 @@ static int plan_undexqv(dx_ctx *ctx, const uint8_t *d_in, size_t n, const int64_
           if ((rc = download(ctx,d_stat,N,stat)) != DX_OK) return rc;
           for (size_t i = 0; i < N; i++)
             if (stat[i]) return dx_fail(ctx,DX_E_TRUNC,"Could not read more bits (Decode), entry %zu",i+1);
+          std::vector<int64_t> soff;                            // entry i must end where entry i+1 starts
+          if ((rc = download(ctx,plan.d_soff,N*6,soff)) != DX_OK) return rc;
+          for (size_t i = 0; i < N; i++)
+            if (soff[6*i+5] != ((i + 1 < N) ? h_entry_off[i+1] : (int64_t) n))
+              return dx_fail(ctx,DX_E_FORMAT,"entry %zu: its streams do not end at the next entry",i+1);
         }
       plan.ix_fs = fs;
       plan.ix_end.resize(N);
@@ -1851,7 +1865,11 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
       int32_t *h_rlen  = (int32_t *) dx_hpin_get(ctx,N*4);
       int32_t *h_order = (int32_t *) dx_hpin_get(ctx,N*4);
       int32_t *d_order = (int32_t *) dx_arena_get(ctx,N*4);
-      if (!h_rlen || !h_order || !d_order) return DX_E_NOMEM;
+      int64_t *d_endat = (int64_t *) dx_arena_get(ctx,N*8);  // entry i ends where entry i+1 starts
+      if (!h_rlen || !h_order || !d_order || !d_endat) return DX_E_NOMEM;
+      const int64_t image_end = (int64_t) n;
+      if (N > 1) DX_CUDA(ctx,cudaMemcpyAsync(d_endat,h_entry_off+1,(N-1)*8,cudaMemcpyHostToDevice,ctx->stream));
+      DX_CUDA(ctx,cudaMemcpyAsync(d_endat+N-1,&image_end,8,cudaMemcpyHostToDevice,ctx->stream));
       DX_CUDA(ctx,cudaMemcpyAsync(h_rlen,pa.rlen,N*4,cudaMemcpyDeviceToHost,ctx->stream));
       DX_CUDA(ctx,cudaMemcpyAsync(&h_tail->total,d_opre+N,8,cudaMemcpyDeviceToHost,ctx->stream));
       DX_CUDA(ctx,cudaMemcpyAsync(&h_tail->flag,d_flag,4,cudaMemcpyDeviceToHost,ctx->stream));
@@ -1865,7 +1883,7 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
       const int64_t n_coop = ticket_plan(ctx,h_rlen,N,h_order);
       DX_CUDA(ctx,cudaMemcpyAsync(d_order,h_order,N*4,cudaMemcpyHostToDevice,ctx->stream));
       if ((rc = dxk_qv_decode6x(ctx,d_in,n,d_tab4,coding.delchar,coding.subchar,upper,1,(int64_t) N,pa.fs,pa.rlen,
-                                d_ent,d_prefix,plen,d_out,NULL,d_stat1,NULL,d_order,NULL,n_coop)) != DX_OK) return rc;
+                                d_ent,d_prefix,plen,d_out,NULL,d_stat1,NULL,d_order,NULL,n_coop,d_endat)) != DX_OK) return rc;
       DX_CUDA(ctx,cudaMemcpyAsync(&h_tail->flag,d_stat1,4,cudaMemcpyDeviceToHost,ctx->stream));
       DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
       ph.mark("decode");
@@ -2134,8 +2152,15 @@ extern "C" int dx_undexqv_dev(dx_ctx *ctx, const uint8_t *d_in, size_t n, int up
         }
     }
   else if (plan.v2)
-    rc = dxk_qv_decode5(ctx,d_in,n,plan.d_tab4,cd.delchar,cd.subchar,upper,1,(int64_t) N,
-                        plan.d_start,plan.d_rlen,d_ent,plan.d_prefix,plan.plen,d_out,NULL,d_stat);
+    { int64_t *d_endat = NULL;                                 // known offsets: entry i ends where i+1 starts
+      if (h_entry_off != NULL && plan.ix_end.size() == N)
+        { if ((d_endat = (int64_t *) dx_arena_get(ctx,N*8)) == NULL) return DX_E_NOMEM;
+          if ((rc = upload(ctx,d_endat,plan.ix_end.data(),N)) != DX_OK) return rc;
+        }
+      rc = dxk_qv_decode5x(ctx,d_in,n,plan.d_tab4,cd.delchar,cd.subchar,upper,1,(int64_t) N,
+                           plan.d_start,plan.d_rlen,d_ent,plan.d_prefix,plan.plen,d_out,NULL,d_stat,
+                           NULL,NULL,NULL,d_endat);
+    }
   else
     rc = dxk_qv_decode(ctx,d_in,n,plan.d_tab,cd.delchar,cd.subchar,cd.flip,upper,d_ent,plan.d_soff,
                        (int64_t) N,plan.d_prefix,plan.plen,d_out,d_stat);

@@ -208,12 +208,15 @@ int dxk_qv_decode5(dx_ctx *ctx, const uint8_t *d_in, size_t n, const QvDecTables
                    const char *d_prefix, int plen, uint8_t *d_out, int64_t *d_soff, int32_t *d_status);
 
 // ... with a per-entry byte limit (an entry that would read past it is reported as bad) and a
-// ticket -> entry order (long entries first); either may be NULL
+// ticket -> entry order (long entries first); either may be NULL.  d_endat (known entry offsets):
+// the byte each entry must end at exactly, the next entry's offset -- an entry whose streams end
+// anywhere else is reported as bad; NULL: not checked
 int dxk_qv_decode5x(dx_ctx *ctx, const uint8_t *d_in, size_t n, const QvDecTables4 *d_tab,
                     int delchar, int subchar, int upper, int write, int64_t count,
                     const int64_t *d_start, const int32_t *d_rlen, const QvDecEntry *d_ent,
                     const char *d_prefix, int plen, uint8_t *d_out, int64_t *d_soff, int32_t *d_status,
-                    const int64_t *d_limit, const int32_t *d_order, const int64_t *d_toff);
+                    const int64_t *d_limit, const int32_t *d_order, const int64_t *d_toff,
+                    const int64_t *d_endat = NULL);
 
 // dx_qv_decode6.cu : one LANE per entry for tickets [n_coop, count), the warp-per-entry kernel for
 // tickets [0, n_coop) (the longest entries); write = 1 or 2
@@ -221,7 +224,8 @@ int dxk_qv_decode6x(dx_ctx *ctx, const uint8_t *d_in, size_t n, const QvDecTable
                     int delchar, int subchar, int upper, int write, int64_t count,
                     const int64_t *d_start, const int32_t *d_rlen, const QvDecEntry *d_ent,
                     const char *d_prefix, int plen, uint8_t *d_out, int64_t *d_soff, int32_t *d_status,
-                    const int64_t *d_limit, const int32_t *d_order, const int64_t *d_toff, int64_t n_coop);
+                    const int64_t *d_limit, const int32_t *d_order, const int64_t *d_toff, int64_t n_coop,
+                    const int64_t *d_endat = NULL);
 
 // move speculatively decoded lines (scratch image d_tmp, entry e at d_src[e], < 0 = skip) to their
 // final place and write the header lines

@@ -65,6 +65,7 @@ struct Dec5Args
   int32_t       *status;       // [count] (walk) or [1] (decode)
   const int64_t *limit;        // per entry: first byte the entry may not reach (NULL: the image end)
   const int32_t *order;        // ticket -> entry (long entries first), NULL: identity
+  const int64_t *endat;        // per entry: the byte its streams must end at (known offsets), NULL: any
   unsigned long long *ticket;
   unsigned long long *dbg;     // optional counters [table][0 rounds, 1 windows, 2 streams, 3 restarts]
 };
@@ -611,6 +612,7 @@ k_qv_decode5(Dec5Args a)
       while (false);
       if (lane == 0)
         { if (at > lim) bad = 1;
+          if (a.endat != NULL && at != a.endat[e]) bad = 1;     // the streams do not fill the entry
           if (a.soff != NULL)
             for (int k = 0; k < 6; k++) a.soff[e*6 + k] = o[k];
           if (a.write == 1) { if (bad) atomicExch(a.status,1); }
@@ -686,21 +688,23 @@ int dxk_qv_decode5x(dx_ctx *ctx, const uint8_t *d_in, size_t n, const QvDecTable
                     int delchar, int subchar, int upper, int write, int64_t count,
                     const int64_t *d_start, const int32_t *d_rlen, const QvDecEntry *d_ent,
                     const char *d_prefix, int plen, uint8_t *d_out, int64_t *d_soff, int32_t *d_status,
-                    const int64_t *d_limit, const int32_t *d_order, const int64_t *d_toff);
+                    const int64_t *d_limit, const int32_t *d_order, const int64_t *d_toff,
+                    const int64_t *d_endat);
 
 int dxk_qv_decode5(dx_ctx *ctx, const uint8_t *d_in, size_t n, const QvDecTables4 *d_tab,
                    int delchar, int subchar, int upper, int write, int64_t count,
                    const int64_t *d_start, const int32_t *d_rlen, const QvDecEntry *d_ent,
                    const char *d_prefix, int plen, uint8_t *d_out, int64_t *d_soff, int32_t *d_status)
 { return dxk_qv_decode5x(ctx,d_in,n,d_tab,delchar,subchar,upper,write,count,d_start,d_rlen,d_ent,d_prefix,plen,
-                         d_out,d_soff,d_status,NULL,NULL,NULL);
+                         d_out,d_soff,d_status,NULL,NULL,NULL,NULL);
 }
 
 int dxk_qv_decode5x(dx_ctx *ctx, const uint8_t *d_in, size_t n, const QvDecTables4 *d_tab,
                     int delchar, int subchar, int upper, int write, int64_t count,
                     const int64_t *d_start, const int32_t *d_rlen, const QvDecEntry *d_ent,
                     const char *d_prefix, int plen, uint8_t *d_out, int64_t *d_soff, int32_t *d_status,
-                    const int64_t *d_limit, const int32_t *d_order, const int64_t *d_toff)
+                    const int64_t *d_limit, const int32_t *d_order, const int64_t *d_toff,
+                    const int64_t *d_endat)
 { if (count == 0) return DX_OK;
   unsigned long long *d_ticket = (unsigned long long *) dx_arena_get(ctx,8);
   if (d_ticket == NULL) return DX_E_NOMEM;
@@ -711,7 +715,7 @@ int dxk_qv_decode5x(dx_ctx *ctx, const uint8_t *d_in, size_t n, const QvDecTable
   a.count = count; a.start = d_start; a.rlen = d_rlen; a.ent = d_ent;
   a.prefix = d_prefix; a.plen = plen; a.out = d_out; a.soff = d_soff; a.status = d_status;
   a.ticket = d_ticket;
-  a.limit = d_limit; a.order = d_order; a.toff = d_toff;
+  a.limit = d_limit; a.order = d_order; a.toff = d_toff; a.endat = d_endat;
   a.dbg = NULL;
   const size_t smem = sizeof(Shared5);
   DX_CUDA(ctx,cudaFuncSetAttribute(k_qv_decode5,cudaFuncAttributeMaxDynamicSharedMemorySize,(int) smem));

@@ -67,6 +67,7 @@ struct Dec6Args
   int32_t       *status;       // [count] (write == 2) or [1] (write == 1)
   const int64_t *limit;        // per entry: first byte the entry may not reach (NULL: the image end)
   const int32_t *order;        // ticket -> entry (long entries first), NULL: identity
+  const int64_t *endat;        // per entry: the byte its streams must end at (known offsets), NULL: any
 };
 
 // shared memory: the tables, then per warp an input ring and an output ring
@@ -656,6 +657,7 @@ k_qv_decode6(Dec6Args a)
   __syncwarp(live);
   if (Ls >= 0) ln.out.sync_partial();
   if (at > lim || Ls < 0) ln.bad = 1;
+  if (a.endat != NULL && at != a.endat[e]) ln.bad = 1;     // the streams do not fill the entry
   if (a.soff != NULL)
     for (int k = done + 1; k < 6; k++) a.soff[e*6 + k] = at;
   if (a.write == 1) { if (ln.bad) atomicExch(a.status,1); }
@@ -670,20 +672,21 @@ int dxk_qv_decode6x(dx_ctx *ctx, const uint8_t *d_in, size_t n, const QvDecTable
                     int delchar, int subchar, int upper, int write, int64_t count,
                     const int64_t *d_start, const int32_t *d_rlen, const QvDecEntry *d_ent,
                     const char *d_prefix, int plen, uint8_t *d_out, int64_t *d_soff, int32_t *d_status,
-                    const int64_t *d_limit, const int32_t *d_order, const int64_t *d_toff, int64_t n_coop)
+                    const int64_t *d_limit, const int32_t *d_order, const int64_t *d_toff, int64_t n_coop,
+                    const int64_t *d_endat)
 { if (count == 0) return DX_OK;
   int rc;
   if (n_coop > count) n_coop = count;
   if (n_coop > 0 &&
       (rc = dxk_qv_decode5x(ctx,d_in,n,d_tab,delchar,subchar,upper,write,n_coop,d_start,d_rlen,d_ent,d_prefix,plen,
-                            d_out,d_soff,d_status,d_limit,d_order,d_toff)) != DX_OK) return rc;
+                            d_out,d_soff,d_status,d_limit,d_order,d_toff,d_endat)) != DX_OK) return rc;
   if (n_coop >= count) return DX_OK;
   Dec6Args a;
   a.in = d_in; a.n = (int64_t) n; a.tab = d_tab;
   a.delchar = delchar; a.subchar = subchar; a.upper = upper; a.write = write;
   a.first = n_coop; a.count = count; a.start = d_start; a.rlen = d_rlen; a.ent = d_ent;
   a.toff = d_toff; a.prefix = d_prefix; a.plen = plen; a.out = d_out; a.soff = d_soff; a.status = d_status;
-  a.limit = d_limit; a.order = d_order;
+  a.limit = d_limit; a.order = d_order; a.endat = d_endat;
   // one CTA per SM (the tables take 102 KB): as many warps per CTA as it takes to have every entry
   // in flight at once, up to 16; more entries than that run in waves, longest first
   const int64_t nwarps = (count - n_coop + 31) / 32;
