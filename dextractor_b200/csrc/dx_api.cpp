@@ -484,12 +484,13 @@ struct PkWalkUser { int fieldbytes; const uint8_t *d_in; size_t n; };
 static int pk_walk_one(dx_ctx *ctx, void *user, int64_t q, int64_t *end, int64_t *slot)
 { PkWalkUser *u = (PkWalkUser *) user;
   std::vector<uint8_t> f;
-  int rc = peek(ctx,u->d_in,u->n,(size_t) q,8,f);
+  int rc = peek(ctx,u->d_in,u->n,(size_t) q,(size_t) u->fieldbytes,f);
   if (rc != DX_OK) return rc;
   *slot = 0;
-  if (f.size() < 8) { *end = -1; return DX_OK; }
+  if ((int) f.size() < u->fieldbytes) { *end = -1; return DX_OK; }
   const int64_t rlen = (int64_t) le32(f.data()+4) - le32(f.data());
-  *end = (rlen < 0) ? -1 : q + u->fieldbytes + ((rlen + 3) >> 2);
+  if (rlen < 0) return dx_fail(ctx,DX_E_FORMAT,"negative read length in entry header");
+  *end = q + u->fieldbytes + ((rlen + 3) >> 2);
   return DX_OK;
 }
 
@@ -1477,7 +1478,8 @@ static int qv_walk_one(dx_ctx *ctx, void *user, int64_t q, int64_t *end, int64_t
   *slot = (int64_t) (u->side.size() / 6);
   if ((int) f.size() < fb) { *end = -1; return DX_OK; }
   const int32_t rlen = qv_field(f.data(),1,fb,u->flip) - qv_field(f.data(),0,fb,u->flip);
-  if (rlen < 0 || rlen >= (1 << 24)) { *end = -1; return DX_OK; }
+  if (rlen < 0) return dx_fail(ctx,DX_E_FORMAT,"negative read length in entry header");
+  if (rlen >= (1 << 24)) { *end = -1; return DX_OK; }
   int64_t *d_start = (int64_t *) dx_arena_get(ctx,8);
   int32_t *d_rlen  = (int32_t *) dx_arena_get(ctx,4);
   int64_t *d_soff  = (int64_t *) dx_arena_get(ctx,48);

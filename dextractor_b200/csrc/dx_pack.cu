@@ -48,7 +48,8 @@ __device__ __forceinline__ bool snr_field(const uint8_t *t, int64_t &p, int64_t 
     return false;
   const int32_t k = ip*100 + (t[p+1]-'0')*10 + (t[p+2]-'0');
   p += 3;
-  if (p < end && t[p] >= '0' && t[p] <= '9') return false;          // more decimals: host path
+  if (p < end && ((t[p] >= '0' && t[p] <= '9') || t[p] == 'e' || t[p] == 'E'))
+    return false;                                                    // more decimals or an exponent: host path
   const float f = (float) ((double) k / 100.0);                      // what %f into a float yields
   cnr = (f > 99.99) ? 9999u : (uint32_t) ((double) f * 100.);
   cnr &= 0xffffu;
