@@ -464,7 +464,7 @@ int dxk_qv_probe(dx_ctx *ctx, const uint8_t *d_text, QvEntries ent, const dx_qv_
       DX_LAUNCHED(ctx,"k_pick_delchar");
     }
   if (need_sub)
-    { k_probe_sub<<<1,1024,0,ctx->stream>>>(d_text,ent,carry->totchar,d_sub_in,d_probe);
+    { DX_PROF_BEGIN(ctx); k_probe_sub<<<1,1024,0,ctx->stream>>>(d_text,ent,carry->totchar,d_sub_in,d_probe);
       DX_LAUNCHED(ctx,"k_probe_sub");
     }
   DX_CUDA(ctx,cudaMemcpyAsync(h_probe,d_probe,sizeof(QvProbe),cudaMemcpyDeviceToHost,ctx->stream));

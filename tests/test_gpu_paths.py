@@ -372,27 +372,48 @@ def test_pipelined_host_decode_on_small_windows(routed, orc, chunk):
     assert ctx.undexqv(enc, cap=len(want) + 4096) == want
 
 
+_scan_inputs: list = []
+
+
+def _scan_shape_inputs():
+    """(label, text, restatement) of the files the counting modes are checked on, computed once"""
+    import torch
+    from tests import fuzz
+    from tests import scan_shapes as S
+    if not _scan_inputs:
+        texts = [(f"fuzz_{seed}", fuzz.fuzz_quiva(seed)[0]) for seed in (0, 3, 5, 8, 13, 21)]
+        texts += [(n, QUIVA[n]) for n in ("long_runs", "late_n", "lognormal_40", "no_n_tags")]
+        W = torch.cuda.get_device_properties(0).multi_processor_count * S.HIST_WARPS_PER_SM
+        for name in sorted(S.SHAPES) + ["delchar_order"]:
+            texts += [(f"{name}/{lab}", t) for lab, t in S.make(name, W if name == "delchar_order" else None)]
+        _scan_inputs.extend((lab, t, S.scan_with_carry(t)) for lab, t in texts)
+    return _scan_inputs
+
+
 @pytest.mark.parametrize("mode", [0, 1, 2, 3, 4])
 def test_run_histogram_counting_modes(ctx, orc, mode):
     """k_qv_hist_run counts a batch of (symbol, run length) items in five ways (route hist_mode):
     every one must give Histogram_Seqs / Histogram_Runs' numbers (QV.c:702-724) on files of random
-    shape -- run densities 0 ... 0.995, runs beyond 255, run characters that appear late."""
+    shape -- run densities 0 ... 0.995, runs beyond 255, run characters that appear late -- and on
+    the crafted files of tests/scan_shapes.py, whose inputs sit on the boundaries of the pass-1
+    kernels (counter wraps, queue rounds, the first tag past the first wave of warps, the 100 000
+    crossing, empty entries).  sub_prefix is checked against the numpy restatement."""
     import torch
-    from tests import fuzz
     ctx.route("default")
     ctx.route("hist_mode", mode)
     try:
-        texts = [fuzz.fuzz_quiva(seed)[0] for seed in (0, 3, 5, 8, 13, 21)]
-        texts += [QUIVA[n] for n in ("long_runs", "late_n", "lognormal_40", "no_n_tags")]
-        for i, text in enumerate(texts):
+        for label, text, want in _scan_shape_inputs():
             t = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
             st = ctx.qv_scan_dev(t.data_ptr(), len(text))
             ref = orc.qv_scan(text)
-            assert (st.delchar, st.subchar, st.totchar) == (ref.delchar, ref.subchar, ref.totchar), i
+            assert (st.delchar, st.subchar, st.totchar) == (ref.delchar, ref.subchar, ref.totchar), label
+            assert st.nentries == ref.nentries == want["nentries"], label
             for k, nm in enumerate(["del_", "ins", "mrg", "sub"]):
-                assert list(st.hist[k]) == list(getattr(ref, nm)), (i, nm)
-            assert [x + 1 for x in st.hist[4]] == list(ref.delrun), i
-            assert [x + 1 for x in st.hist[5]] == list(ref.subrun), i
+                assert list(st.hist[k]) == list(getattr(ref, nm)), (label, nm)
+            assert [x + 1 for x in st.hist[4]] == list(ref.delrun), label
+            assert [x + 1 for x in st.hist[5]] == list(ref.subrun), label
+            assert all(st.hist[k][0] == 0 and st.hist[k][10] == 0 for k in range(4)), label
+            assert list(st.sub_prefix) == [int(x) for x in want["sub_prefix"]], label
     finally:
         ctx.route("default")
 
