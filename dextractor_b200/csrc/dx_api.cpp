@@ -1348,6 +1348,39 @@ static bool build_dec_tables4(const dx_qv_coding *c, QvDecTables4 *t)
   return true;
 }
 
+// bits a position takes at least: the shortest ins code plus the shortest mrg code (never run-length coded)
+static int qv_minbits(const dx_qv_coding &c)
+{ int minbits = 0;
+  for (int k = 2; k <= 3; k++)
+    { int mn = 32;
+      for (int x = 0; x < 256; x++)
+        if (c.tab[k].lens[x] > 0 && c.tab[k].lens[x] < mn) mn = c.tab[k].lens[x];
+      minbits += (mn == 32) ? 0 : mn;
+    }
+  return minbits;
+}
+
+// A small asynchronous transfer between pinned host memory and the device on ctx->stream; by_kernel: by
+// dxk_fetch, not queued behind the large copies of the pipelined host decode (see k_fetch, dx_frame.cu).
+static int qv_copy(dx_ctx *ctx, bool by_kernel, void *dst, const void *src, size_t bytes)
+{ if (by_kernel) return dxk_fetch(ctx,dst,src,bytes);
+  if (bytes > 0) DX_CUDA(ctx,cudaMemcpyAsync(dst,src,bytes,cudaMemcpyDefault,ctx->stream));
+  return DX_OK;
+}
+
+// The 12-bit decode tables of a coding, copied to d_tab4 through a temporary buffer (h4 == NULL, synchronous)
+// or by qv_copy from pinned h4.  *fits = false: more long codes than the tables hold, nothing is copied.
+static int qv_tables4(dx_ctx *ctx, const dx_qv_coding *c, QvDecTables4 *h4, bool by_kernel,
+                      QvDecTables4 *d_tab4, bool *fits)
+{ QvDecTables4 *h = h4 ? h4 : (QvDecTables4 *) malloc(sizeof(QvDecTables4));
+  if (h == NULL) return DX_E_NOMEM;
+  int rc = DX_OK;
+  *fits = build_dec_tables4(c,h);
+  if (*fits) rc = h4 ? qv_copy(ctx,by_kernel,d_tab4,h,sizeof(QvDecTables4)) : upload(ctx,d_tab4,h,1);
+  if (h4 == NULL) free(h);
+  return rc;
+}
+
 struct QvPlan
 { std::vector<QvDecEntry> ent;
   bool         v2;            // parallel decoders usable (tables fit shared memory)
@@ -1497,49 +1530,64 @@ static int qv_walk_one(dx_ctx *ctx, void *user, int64_t q, int64_t *end, int64_t
   return DX_OK;
 }
 
+// The head of a .dexqv image, read from host bytes.  New layout: 0x55aa (either byte order) in front
+// of the coding header; old layout: the file starts with the coding header itself (key 0x33cc) and
+// beg/end/qv are uint16 (undexqv.c:103-110).
+struct QvHead
+{ uint16_t          key;
+  bool              newv;         // the new layout
+  dx_qv_coding      coding;
+  std::vector<char> prefix = std::vector<char>(100001);   // NUL-terminated
+  int               plen;
+  size_t            first;        // first byte behind the coding header
+};
+
+// DX_E_TRUNC: fewer than 2 bytes; DX_E_KEY: no .dexqv key; else what dx_qv_read_coding returns.  No
+// message: the fast paths decline such an image silently, the general path says what is wrong.
+static int qv_read_head(const uint8_t *h, size_t len, QvHead &hd)
+{ if (len < 2) return DX_E_TRUNC;
+  memcpy(&hd.key,h,2);
+  hd.newv = (hd.key == 0x55aa || hd.key == 0xaa55);
+  if (!hd.newv && !(hd.key == 0x33cc || hd.key == 0xcc33)) return DX_E_KEY;
+  const size_t keylen = hd.newv ? 2 : 0;
+  size_t used = 0;
+  const int rc = dx_qv_read_coding(h + keylen,len - keylen,&hd.coding,hd.prefix.data(),(int) hd.prefix.size(),&used);
+  if (rc != DX_OK) return rc;
+  hd.plen = (int) strlen(hd.prefix.data());
+  hd.first = keylen + used;
+  return DX_OK;
+}
+
 static int plan_undexqv(dx_ctx *ctx, const uint8_t *d_in, size_t n, const int64_t *h_entry_off,
                         int64_t nentries, int32_t well_in, bool need_streams, int upper, QvPlan &plan)
 { int rc;
   std::vector<uint8_t> head;
   if ((rc = peek(ctx,d_in,n,0,2 + 16384 + 100000,head)) != DX_OK) return rc;
   if (head.size() < 2) return dx_fail(ctx,DX_E_TRUNC,"System error, read failed!");
-  uint16_t key; memcpy(&key,head.data(),2);
-  // new layout: 0x55aa (either byte order) in front of the coding header; old layout: the file starts
-  // with the coding header itself (key 0x33cc) and beg/end/qv are uint16 (undexqv.c:103-110)
-  const bool newv = (key == 0x55aa || key == 0xaa55);
-  if (!newv && !(key == 0x33cc || key == 0xcc33))
-    return dx_fail(ctx,DX_E_KEY,"not a .dexqv file (endian key 0x%04x)",(unsigned) key);
-  const size_t keylen = newv ? 2 : 0;
-  std::vector<char> prefix(100001);
-  size_t used = 0;
-  if ((rc = dx_qv_read_coding(head.data()+keylen,head.size()-keylen,&plan.coding,prefix.data(),
-                              (int) prefix.size(),&used)) != DX_OK)
-    return dx_fail(ctx,rc,"Could not read the coding header (Read_QVcoding)");
+  QvHead hd;
+  if ((rc = qv_read_head(head.data(),head.size(),hd)) == DX_E_KEY)
+    return dx_fail(ctx,DX_E_KEY,"not a .dexqv file (endian key 0x%04x)",(unsigned) hd.key);
+  if (rc != DX_OK) return dx_fail(ctx,rc,"Could not read the coding header (Read_QVcoding)");
+  plan.coding = hd.coding;
   // A file of the other byte order (every stream word flipped, QV.c:553-568) or of the old layout is
   // rare: it takes the sequential kernels, which flip words as they read them, and finds its
   // entries by walking them one after the other.  Slow (a launch per entry), but the reference's bytes.
-  const bool legacy = (plan.coding.flip != 0) || !newv;
-  const int fieldbytes = newv ? 12 : 6;
+  const bool legacy = (plan.coding.flip != 0) || !hd.newv;
+  const int fieldbytes = hd.newv ? 12 : 6;
   if (legacy) { h_entry_off = NULL; nentries = 0; }
-  const size_t first = keylen + used;
+  const size_t first = hd.first;
   DxPhases ph(ctx);
-  plan.plen = (int) strlen(prefix.data());
+  plan.plen = hd.plen;
   plan.d_soff = NULL; plan.d_start = NULL; plan.d_rlen = NULL; plan.d_tab = NULL;
   plan.spec = false; plan.d_tmp = NULL; plan.tmp_n = 0; plan.src.clear();
 
-  { // 12-bit shared-memory tables for the parallel kernels; a coding they cannot hold (more long
-    // codes than the sub-tables take) is decoded by the sequential kernels of dx_qv_decode.cu
-    QvDecTables4 *h4 = (QvDecTables4 *) malloc(sizeof(QvDecTables4));
-    if (h4 == NULL) return DX_E_NOMEM;
-    plan.v2 = (ctx->route[DXR_DECODER] != 1) && !legacy && build_dec_tables4(&plan.coding,h4);
-    plan.d_tab4 = NULL;
-    if (plan.v2)
-      { plan.d_tab4 = (QvDecTables4 *) dx_arena_get(ctx,sizeof(QvDecTables4));
-        rc = plan.d_tab4 ? upload(ctx,plan.d_tab4,h4,1) : DX_E_NOMEM;
-      }
-    free(h4);
-    if (rc != DX_OK) return rc;
-  }
+  plan.v2 = false; plan.d_tab4 = NULL;
+  if (ctx->route[DXR_DECODER] != 1 && !legacy)
+    { // 12-bit shared-memory tables for the parallel kernels; a coding they cannot hold (more long
+      // codes than the sub-tables take) is decoded by the sequential kernels of dx_qv_decode.cu
+      if ((plan.d_tab4 = (QvDecTables4 *) dx_arena_get(ctx,sizeof(QvDecTables4))) == NULL) return DX_E_NOMEM;
+      if ((rc = qv_tables4(ctx,&plan.coding,NULL,false,plan.d_tab4,&plan.v2)) != DX_OK) return rc;
+    }
   if (!plan.v2)
     { QvDecTables *h_tab = (QvDecTables *) malloc(sizeof(QvDecTables));
       if (h_tab == NULL) return DX_E_NOMEM;
@@ -1551,7 +1599,7 @@ static int plan_undexqv(dx_ctx *ctx, const uint8_t *d_in, size_t n, const int64_
     }
   plan.d_prefix = (char *) dx_arena_get(ctx,(size_t) plan.plen + 1);
   if (!plan.d_prefix) return DX_E_NOMEM;
-  if ((rc = upload(ctx,plan.d_prefix,prefix.data(),(size_t) plan.plen)) != DX_OK) return rc;
+  if ((rc = upload(ctx,plan.d_prefix,hd.prefix.data(),(size_t) plan.plen)) != DX_OK) return rc;
 
   struct Hdr { int32_t well, beg, end, qv; };
   std::vector<Hdr> hdrs;
@@ -1669,13 +1717,7 @@ static int plan_undexqv(dx_ctx *ctx, const uint8_t *d_in, size_t n, const int64_
           }
           // ... and a candidate whose length field cannot fit before its limit even at the
           // shortest code of the two streams that are never run-length coded is not decoded at all
-          { int minbits = 0;
-            for (int k = 2; k <= 3; k++)
-              { int mn = 32;
-                for (int x = 0; x < 256; x++)
-                  if (plan.coding.tab[k].lens[x] > 0 && plan.coding.tab[k].lens[x] < mn) mn = plan.coding.tab[k].lens[x];
-                minbits += (mn == 32) ? 0 : mn;
-              }
+          { const int minbits = qv_minbits(plan.coding);
             std::vector<int32_t> rl;
             size_t skipped = 0;
             if ((rc = download(ctx,d_rlen,N,rl)) != DX_OK) return rc;
@@ -1780,6 +1822,131 @@ static int plan_undexqv(dx_ctx *ctx, const uint8_t *d_in, size_t n, const int64_
   return DX_OK;
 }
 
+// pinned landing place of a byte total and a flag that a planning step hands back to the host
+struct QvTail { int64_t total; int32_t flag; int32_t pad; };
+
+static bool alloc_plan(dx_ctx *ctx, size_t N, QvPlanArrays &pa)
+{ pa.fs    = (int64_t *)  dx_arena_get(ctx,N*8);
+  pa.rlen  = (int32_t *)  dx_arena_get(ctx,N*4);
+  pa.delta = (uint32_t *) dx_arena_get(ctx,N*4);
+  pa.beg   = (int32_t *)  dx_arena_get(ctx,N*4);
+  pa.end   = (int32_t *)  dx_arena_get(ctx,N*4);
+  pa.qv    = (int32_t *)  dx_arena_get(ctx,N*4);
+  return pa.fs && pa.rlen && pa.delta && pa.beg && pa.end && pa.qv;
+}
+
+// ------------------------------------------------------------------------------------------------
+//  Discovered entries, for undexqv_fast (a whole image) and undexqv_pipe (one window at a time), in
+//  the order a caller runs the steps: qv_cands_prep enqueues the candidates' context and limits,
+//  qv_cands_plan brings what the ticket plan needs to the host, qv_cands_decode decodes every
+//  candidate into a scratch image laid out by the candidates' own lengths; with their ends on the
+//  host dx_chain_walk picks the entries (h_cand / h_well), qv_layout lays out their text, and the
+//  caller checks its size and moves the lines into place (k_qv_assemble).  by_kernel: the small
+//  transfers go through dxk_fetch (qv_copy).
+// ------------------------------------------------------------------------------------------------
+struct QvCands
+{ size_t       N;
+  const int64_t *d_q;                     // the candidates' field positions
+  QvTail      *h_tail;
+  QvPlanArrays pa;
+  uint32_t    *d_tlen;
+  int64_t     *d_limit, *d_toff, *d_soff, *h_q, *h_soff;
+  int32_t     *d_ffrun, *d_stat, *d_order, *h_ffrun, *h_rlen, *h_order, *h_stat;
+  uint8_t     *d_last, *h_last;
+  int32_t     *h_cand, *h_well;           // the chain: entry m is candidate h_cand[m], of well h_well[m]
+  int64_t      n_coop;
+  uint8_t     *d_tmp;                     // the scratch image
+  size_t       tmp_n;
+  QvDecEntry  *d_ent;                     // qv_layout: the entries' table and where their lines are in d_tmp
+  int64_t     *d_src;
+};
+
+static int qv_cands_prep(dx_ctx *ctx, const uint8_t *d_in, size_t n, size_t first, const int64_t *d_q, int64_t nc,
+                         int minbits, QvTail *h_tail, QvCands &c)
+{ const size_t N = (size_t) nc;
+  c.N = N; c.d_q = d_q; c.h_tail = h_tail;
+  c.d_tlen  = (uint32_t *) dx_arena_get(ctx,N*4);
+  c.d_limit = (int64_t *)  dx_arena_get(ctx,N*8);
+  c.d_ffrun = (int32_t *)  dx_arena_get(ctx,N*4);
+  c.d_last  = (uint8_t *)  dx_arena_get(ctx,N);
+  c.d_toff  = (int64_t *)  dx_arena_get(ctx,(N+1)*8);
+  c.d_soff  = (int64_t *)  dx_arena_get(ctx,N*48);
+  c.d_stat  = (int32_t *)  dx_arena_get(ctx,N*4);
+  c.d_order = (int32_t *)  dx_arena_get(ctx,N*4);
+  c.h_q     = (int64_t *)  dx_hpin_get(ctx,N*8);
+  c.h_ffrun = (int32_t *)  dx_hpin_get(ctx,N*4);
+  c.h_last  = (uint8_t *)  dx_hpin_get(ctx,N);
+  c.h_rlen  = (int32_t *)  dx_hpin_get(ctx,N*4);
+  c.h_order = (int32_t *)  dx_hpin_get(ctx,N*4);
+  c.h_soff  = (int64_t *)  dx_hpin_get(ctx,N*48);
+  c.h_stat  = (int32_t *)  dx_hpin_get(ctx,N*4);
+  c.h_cand  = (int32_t *)  dx_hpin_get(ctx,N*4);
+  c.h_well  = (int32_t *)  dx_hpin_get(ctx,N*4);
+  if (!alloc_plan(ctx,N,c.pa) || !c.d_tlen || !c.d_limit || !c.d_ffrun || !c.d_last || !c.d_toff || !c.d_soff ||
+      !c.d_stat || !c.d_order || !c.h_q || !c.h_ffrun || !c.h_last || !c.h_rlen || !c.h_order || !c.h_soff ||
+      !c.h_stat || !c.h_cand || !c.h_well) return DX_E_NOMEM;
+  const int rc = dxk_qv_cand_prep(ctx,d_in,n,first,d_q,nc,4,minbits,c.pa,c.d_tlen,c.d_limit,c.d_ffrun,c.d_last);
+  return (rc != DX_OK) ? rc : dxk_scan_u32(ctx,c.d_tlen,nc,c.d_toff);
+}
+
+// (the synchronisation also covers whatever the caller enqueued after qv_cands_prep)
+static int qv_cands_plan(dx_ctx *ctx, QvCands &c, bool by_kernel)
+{ const size_t N = c.N;
+  int rc;
+  if ((rc = qv_copy(ctx,by_kernel,c.h_q,c.d_q,N*8)) != DX_OK ||
+      (rc = qv_copy(ctx,by_kernel,c.h_ffrun,c.d_ffrun,N*4)) != DX_OK ||
+      (rc = qv_copy(ctx,by_kernel,c.h_last,c.d_last,N)) != DX_OK ||
+      (rc = qv_copy(ctx,by_kernel,c.h_rlen,c.pa.rlen,N*4)) != DX_OK ||
+      (rc = qv_copy(ctx,by_kernel,&c.h_tail->total,c.d_toff+N,8)) != DX_OK) return rc;
+  DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
+  c.tmp_n = (size_t) c.h_tail->total;
+  c.n_coop = ticket_plan(ctx,c.h_rlen,N,c.h_order);
+  return qv_copy(ctx,by_kernel,c.d_order,c.h_order,N*4);
+}
+
+static int qv_cands_decode(dx_ctx *ctx, const uint8_t *d_in, size_t n, const QvDecTables4 *d_tab4,
+                           const dx_qv_coding &cd, int upper, QvCands &c)
+{ c.d_tmp = (uint8_t *) dx_arena_get(ctx,c.tmp_n + 64);
+  if (c.d_tmp == NULL) return DX_E_NOMEM;
+  return dxk_qv_decode6x(ctx,d_in,n,d_tab4,cd.delchar,cd.subchar,upper,2,(int64_t) c.N,c.pa.fs,c.pa.rlen,NULL,NULL,0,
+                         c.d_tmp,c.d_soff,c.d_stat,c.d_limit,c.d_order,c.d_toff,c.n_coop);
+}
+
+// the text layout of the chain's M entries; *total: its bytes (d_flag[0], zero on entry: unusable read length)
+static int qv_layout(dx_ctx *ctx, QvCands &c, size_t M, int plen, int32_t *d_flag, bool by_kernel, size_t *total)
+{ int32_t *d_cand  = (int32_t *) dx_arena_get(ctx,M*4 + 4);
+  int32_t *d_wells = (int32_t *) dx_arena_get(ctx,M*4 + 4);
+  int32_t *d_well  = (int32_t *) dx_arena_get(ctx,M*4 + 4);
+  uint32_t *d_len  = (uint32_t *) dx_arena_get(ctx,M*4 + 4);
+  int64_t *d_opre  = (int64_t *) dx_arena_get(ctx,(M+1)*8);
+  c.d_src = (int64_t *) dx_arena_get(ctx,M*8 + 8);
+  c.d_ent = (QvDecEntry *) dx_arena_get(ctx,(M+1)*sizeof(QvDecEntry));
+  if (!d_cand || !d_wells || !d_well || !d_len || !d_opre || !c.d_src || !c.d_ent) return DX_E_NOMEM;
+  int rc;
+  if ((rc = qv_copy(ctx,by_kernel,d_cand,c.h_cand,M*4)) != DX_OK ||
+      (rc = qv_copy(ctx,by_kernel,d_wells,c.h_well,M*4)) != DX_OK ||
+      (rc = dxk_qv_text_len(ctx,(int64_t) M,d_cand,c.pa,NULL,d_wells,0,plen,d_len,d_well,d_flag)) != DX_OK ||
+      (rc = dxk_scan_u32(ctx,d_len,(int64_t) M,d_opre)) != DX_OK ||
+      (rc = dxk_qv_build_ent(ctx,(int64_t) M,d_cand,c.pa,d_well,d_opre,d_len,c.d_toff,c.d_ent,c.d_src,NULL,NULL)) != DX_OK ||
+      (rc = qv_copy(ctx,by_kernel,&c.h_tail->total,d_opre+M,8)) != DX_OK ||
+      (rc = qv_copy(ctx,by_kernel,&c.h_tail->flag,d_flag,4)) != DX_OK) return rc;
+  DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
+  if (c.h_tail->flag) return dx_fail(ctx,DX_E_FORMAT,"unusable read length in an entry header");
+  *total = (size_t) c.h_tail->total;
+  return DX_OK;
+}
+
+// ctx->last_index (dx_keep_index): entry i's table row, first stream byte and first byte behind it
+static void set_last_index(dx_ctx *ctx, size_t N, const QvDecEntry *ent, const int64_t *stream_off,
+                           const int64_t *end_off)
+{ std::vector<dx_index_row> &ix = *(std::vector<dx_index_row> *) ctx->last_index;
+  ix.resize(N);
+  for (size_t i = 0; i < N; i++)
+    { ix[i].stream_off = stream_off[i]; ix[i].end_off = end_off[i];
+      ix[i].text_off = ent[i].text_off; ix[i].rlen = ent[i].end - ent[i].beg; ix[i].well = ent[i].well;
+    }
+}
+
 // ------------------------------------------------------------------------------------------------
 //  The usual case of dx_undexqv_dev with everything but the verification of the entry chain on the
 //  device (dx_qv_plan.cu): well numbers and text offsets are prefix sums, the host sees a few
@@ -1796,17 +1963,11 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
   if (ctx->route[DXR_DECODER] == 1 || ctx->route[DXR_NO_SPEC] || ctx->route[DXR_NO_FAST]) return DX_OK;
   std::vector<uint8_t> head;
   if ((rc = peek(ctx,d_in,n,0,2 + 16384 + 100000,head)) != DX_OK) return rc;
-  if (head.size() < 2) return DX_OK;
-  uint16_t key; memcpy(&key,head.data(),2);
-  if (!(key == 0x55aa || key == 0xaa55)) return DX_OK;
-  dx_qv_coding coding;
-  std::vector<char> prefix(100001);
-  size_t used = 0;
-  if (dx_qv_read_coding(head.data()+2,head.size()-2,&coding,prefix.data(),(int) prefix.size(),&used) != DX_OK ||
-      coding.flip)
-    return DX_OK;
-  const size_t first = 2 + used;
-  const int plen = (int) strlen(prefix.data());
+  QvHead hd;
+  if (qv_read_head(head.data(),head.size(),hd) != DX_OK || !hd.newv || hd.coding.flip) return DX_OK;
+  const dx_qv_coding &coding = hd.coding;
+  const size_t first = hd.first;
+  const int plen = hd.plen;
   QvDecTables4 *h4 = (QvDecTables4 *) dx_hpin_get(ctx,sizeof(QvDecTables4));
   if (h4 == NULL) return DX_E_NOMEM;
   QvDecTables4 *d_tab4 = (QvDecTables4 *) dx_arena_get(ctx,sizeof(QvDecTables4));
@@ -1816,33 +1977,18 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
   // the decode tables are host work (~0.1 ms): with a known entry index they are built while the
   // planning kernels run
   bool tables_ok = true;
-  auto make_tables = [&]() -> int
-    { tables_ok = build_dec_tables4(&coding,h4);
-      if (tables_ok)
-        DX_CUDA(ctx,cudaMemcpyAsync(d_tab4,h4,sizeof(QvDecTables4),cudaMemcpyHostToDevice,ctx->stream));
-      return DX_OK;
-    };
+  auto make_tables = [&]() -> int { return qv_tables4(ctx,&coding,h4,false,d_tab4,&tables_ok); };
   // ... and while the candidate index runs when there is none
   struct Deferred { decltype(make_tables) *fn; int rc; } deferred = { &make_tables, DX_OK };
   char *h_prefix = (char *) dx_hpin_get(ctx,(size_t) plen + 1);
   if (h_prefix == NULL) return DX_E_NOMEM;
-  memcpy(h_prefix,prefix.data(),(size_t) plen + 1);
+  memcpy(h_prefix,hd.prefix.data(),(size_t) plen + 1);
   DX_CUDA(ctx,cudaMemcpyAsync(d_prefix,h_prefix,(size_t) plen + 1,cudaMemcpyHostToDevice,ctx->stream));
   DX_CUDA(ctx,cudaMemsetAsync(d_flag,0,16,ctx->stream));
   int32_t *d_stat1 = d_flag + 1;                        // decode status of the final launch
   ph.mark("tables");
 
-  auto alloc_plan = [&](size_t N, QvPlanArrays &pa) -> bool
-    { pa.fs   = (int64_t *)  dx_arena_get(ctx,N*8);
-      pa.rlen = (int32_t *)  dx_arena_get(ctx,N*4);
-      pa.delta= (uint32_t *) dx_arena_get(ctx,N*4);
-      pa.beg  = (int32_t *)  dx_arena_get(ctx,N*4);
-      pa.end  = (int32_t *)  dx_arena_get(ctx,N*4);
-      pa.qv   = (int32_t *)  dx_arena_get(ctx,N*4);
-      return pa.fs && pa.rlen && pa.delta && pa.beg && pa.end && pa.qv;
-    };
-  struct Tail { int64_t total; int32_t flag; int32_t pad; };
-  Tail *h_tail = (Tail *) dx_hpin_get(ctx,sizeof(Tail));
+  QvTail *h_tail = (QvTail *) dx_hpin_get(ctx,sizeof(QvTail));
   if (h_tail == NULL) return DX_E_NOMEM;
 
   if (h_entry_off != NULL)
@@ -1856,7 +2002,7 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
       uint32_t *d_len   = (uint32_t *) dx_arena_get(ctx,N*4);
       int32_t *d_well   = (int32_t *) dx_arena_get(ctx,N*4);
       QvDecEntry *d_ent = (QvDecEntry *) dx_arena_get(ctx,N*sizeof(QvDecEntry));
-      if (!alloc_plan(N,pa) || !d_estart || !d_wpre || !d_opre || !d_len || !d_well || !d_ent) return DX_E_NOMEM;
+      if (!alloc_plan(ctx,N,pa) || !d_estart || !d_wpre || !d_opre || !d_len || !d_well || !d_ent) return DX_E_NOMEM;
       DX_CUDA(ctx,cudaMemcpyAsync(d_estart,h_entry_off,N*8,cudaMemcpyHostToDevice,ctx->stream));
       if ((rc = dxk_qv_known_prep(ctx,d_in,n,d_estart,(int64_t) N,pa,d_flag)) != DX_OK) return rc;
       if ((rc = dxk_scan_u32(ctx,pa.delta,(int64_t) N,d_wpre)) != DX_OK) return rc;
@@ -1892,15 +2038,12 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
       ph.report("undexqv (index known)");
       if (h_tail->flag) return dx_fail(ctx,DX_E_TRUNC,"Could not read more bits (Decode)");
       if (ctx->keep_index)
-        { std::vector<dx_index_row> &ix = *(std::vector<dx_index_row> *) ctx->last_index;
-          std::vector<QvDecEntry> he; std::vector<int64_t> hfs;
+        { std::vector<QvDecEntry> he; std::vector<int64_t> hfs;
           if ((rc = download(ctx,d_ent,N,he)) != DX_OK) return rc;
           if ((rc = download(ctx,pa.fs,N,hfs)) != DX_OK) return rc;
-          ix.resize(N);
-          for (size_t i = 0; i < N; i++)
-            { ix[i].stream_off = hfs[i]; ix[i].end_off = (i + 1 < N) ? h_entry_off[i+1] : (int64_t) n;
-              ix[i].text_off = he[i].text_off; ix[i].rlen = he[i].end - he[i].beg; ix[i].well = he[i].well;
-            }
+          std::vector<int64_t> end_off(h_entry_off + 1,h_entry_off + N);
+          end_off.push_back((int64_t) n);
+          set_last_index(ctx,N,he.data(),hfs.data(),end_off.data());
         }
       *out_len = (size_t) h_tail->total;
       *handled = true;
@@ -1922,26 +2065,8 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
   ph.mark("index");
   const size_t N = (size_t) nc;
   if (N == 0) return DX_OK;                             // empty or all entries missed: general path
-  int minbits = 0;
-  for (int k = 2; k <= 3; k++)
-    { int mn = 32;
-      for (int x = 0; x < 256; x++)
-        if (coding.tab[k].lens[x] > 0 && coding.tab[k].lens[x] < mn) mn = coding.tab[k].lens[x];
-      minbits += (mn == 32) ? 0 : mn;
-    }
-  QvPlanArrays pa;
-  uint32_t *d_tlen  = (uint32_t *) dx_arena_get(ctx,N*4);
-  int64_t  *d_limit = (int64_t *)  dx_arena_get(ctx,N*8);
-  int32_t  *d_ffrun = (int32_t *)  dx_arena_get(ctx,N*4);
-  uint8_t  *d_last  = (uint8_t *)  dx_arena_get(ctx,N);
-  int64_t  *d_toff  = (int64_t *)  dx_arena_get(ctx,(N+1)*8);
-  int64_t  *d_soff  = (int64_t *)  dx_arena_get(ctx,N*48);
-  int32_t  *d_stat  = (int32_t *)  dx_arena_get(ctx,N*4);
-  int32_t  *d_order = (int32_t *)  dx_arena_get(ctx,N*4);
-  if (!alloc_plan(N,pa) || !d_tlen || !d_limit || !d_ffrun || !d_last || !d_toff || !d_soff || !d_stat || !d_order)
-    return DX_E_NOMEM;
-  if ((rc = dxk_qv_cand_prep(ctx,d_in,n,first,d_q,nc,4,minbits,pa,d_tlen,d_limit,d_ffrun,d_last)) != DX_OK) return rc;
-  if ((rc = dxk_scan_u32(ctx,d_tlen,nc,d_toff)) != DX_OK) return rc;
+  QvCands c;
+  if ((rc = qv_cands_prep(ctx,d_in,n,first,d_q,nc,qv_minbits(coding),h_tail,c)) != DX_OK) return rc;
   // The layout of the text IF the entries are exactly the candidates k_qv_direct_prep keeps (not within
   // 13 bytes of a later one, fields in the range of real headers) and every well delta but the first is below 255
   // (no 0xff delta bytes; true of real data, where consecutive wells are a few holes apart): wells and text
@@ -1957,52 +2082,27 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
   int32_t *d_flag2 = d_flag + 2;                        // unusable length in some candidate
   uint8_t *d_keep = (uint8_t *) dx_arena_get(ctx,N + 4);         // 1: part of that layout
   if (!d_wpre || !d_opre || !d_len || !d_well || !d_ent || !d_rlen_d || !d_keep) return DX_E_NOMEM;
-  if ((rc = dxk_qv_direct_prep(ctx,d_q,nc,pa,d_rlen_d,d_keep)) != DX_OK) return rc;
-  if ((rc = dxk_scan_u32(ctx,pa.delta,nc,d_wpre)) != DX_OK) return rc;
-  if ((rc = dxk_qv_text_len(ctx,nc,NULL,pa,d_wpre,NULL,well_in,plen,d_len,d_well,d_flag2,d_rlen_d)) != DX_OK) return rc;
+  if ((rc = dxk_qv_direct_prep(ctx,d_q,nc,c.pa,d_rlen_d,d_keep)) != DX_OK) return rc;
+  if ((rc = dxk_scan_u32(ctx,c.pa.delta,nc,d_wpre)) != DX_OK) return rc;
+  if ((rc = dxk_qv_text_len(ctx,nc,NULL,c.pa,d_wpre,NULL,well_in,plen,d_len,d_well,d_flag2,d_rlen_d)) != DX_OK) return rc;
   if ((rc = dxk_scan_u32(ctx,d_len,nc,d_opre)) != DX_OK) return rc;
-  if ((rc = dxk_qv_build_ent(ctx,nc,NULL,pa,d_well,d_opre,d_len,NULL,d_ent,NULL,NULL,NULL)) != DX_OK) return rc;
-  int64_t *h_q     = (int64_t *) dx_hpin_get(ctx,N*8);
-  int32_t *h_ffrun = (int32_t *) dx_hpin_get(ctx,N*4);
-  uint8_t *h_last  = (uint8_t *) dx_hpin_get(ctx,N);
-  int32_t *h_rlen  = (int32_t *) dx_hpin_get(ctx,N*4);
-  int32_t *h_order = (int32_t *) dx_hpin_get(ctx,N*4);
-  int64_t *h_soff  = (int64_t *) dx_hpin_get(ctx,N*48);
-  int32_t *h_stat  = (int32_t *) dx_hpin_get(ctx,N*4);
-  int32_t *h_cand  = (int32_t *) dx_hpin_get(ctx,N*4);
-  int32_t *h_well  = (int32_t *) dx_hpin_get(ctx,N*4);
-  int64_t *h_tot   = (int64_t *) dx_hpin_get(ctx,16);
-  uint8_t *h_keep  = (uint8_t *) dx_hpin_get(ctx,N);
-  if (!h_q || !h_ffrun || !h_last || !h_rlen || !h_order || !h_soff || !h_stat || !h_cand || !h_well || !h_tot || !h_keep)
-    return DX_E_NOMEM;
+  if ((rc = dxk_qv_build_ent(ctx,nc,NULL,c.pa,d_well,d_opre,d_len,NULL,d_ent,NULL,NULL,NULL)) != DX_OK) return rc;
+  int64_t *h_tot  = (int64_t *) dx_hpin_get(ctx,16);
+  uint8_t *h_keep = (uint8_t *) dx_hpin_get(ctx,N);
+  if (!h_tot || !h_keep) return DX_E_NOMEM;
   DX_CUDA(ctx,cudaMemcpyAsync(h_keep,d_keep,N,cudaMemcpyDeviceToHost,ctx->stream));
-  DX_CUDA(ctx,cudaMemcpyAsync(h_q,d_q,N*8,cudaMemcpyDeviceToHost,ctx->stream));
-  DX_CUDA(ctx,cudaMemcpyAsync(h_ffrun,d_ffrun,N*4,cudaMemcpyDeviceToHost,ctx->stream));
-  DX_CUDA(ctx,cudaMemcpyAsync(h_last,d_last,N,cudaMemcpyDeviceToHost,ctx->stream));
-  DX_CUDA(ctx,cudaMemcpyAsync(h_rlen,pa.rlen,N*4,cudaMemcpyDeviceToHost,ctx->stream));
-  DX_CUDA(ctx,cudaMemcpyAsync(&h_tail->total,d_toff+N,8,cudaMemcpyDeviceToHost,ctx->stream));
   DX_CUDA(ctx,cudaMemcpyAsync(h_tot,d_opre+N,8,cudaMemcpyDeviceToHost,ctx->stream));
   DX_CUDA(ctx,cudaMemcpyAsync(&h_tail->flag,d_flag2,4,cudaMemcpyDeviceToHost,ctx->stream));
-  DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
+  if ((rc = qv_cands_plan(ctx,c,false)) != DX_OK) return rc;
   ph.mark("prep");
-  const int64_t n_coop = ticket_plan(ctx,h_rlen,N,h_order);
-  DX_CUDA(ctx,cudaMemcpyAsync(d_order,h_order,N*4,cudaMemcpyHostToDevice,ctx->stream));
-  const size_t tmp_n = (size_t) h_tail->total;
   const int64_t direct_total = h_tot[0];
-  bool direct = !ctx->route[DXR_NO_DIRECT] && n_coop == (int64_t) N && h_tail->flag == 0 &&
+  bool direct = !ctx->route[DXR_NO_DIRECT] && c.n_coop == (int64_t) N && h_tail->flag == 0 &&
                 direct_total >= 0 && (size_t) direct_total <= cap;
-  uint8_t *d_tmp = NULL;
-  auto spec_decode = [&]() -> int
-    { d_tmp = (uint8_t *) dx_arena_get(ctx,tmp_n + 64);
-      if (d_tmp == NULL) return DX_E_NOMEM;
-      return dxk_qv_decode6x(ctx,d_in,n,d_tab4,coding.delchar,coding.subchar,upper,2,nc,pa.fs,pa.rlen,NULL,NULL,0,
-                             d_tmp,d_soff,d_stat,d_limit,d_order,d_toff,n_coop);
-    };
   if (direct)
-    rc = dxk_qv_decode6x(ctx,d_in,n,d_tab4,coding.delchar,coding.subchar,upper,3,nc,pa.fs,d_rlen_d,d_ent,d_prefix,plen,
-                         d_out,d_soff,d_stat,d_limit,d_order,NULL,n_coop);
+    rc = dxk_qv_decode6x(ctx,d_in,n,d_tab4,coding.delchar,coding.subchar,upper,3,nc,c.pa.fs,d_rlen_d,d_ent,d_prefix,plen,
+                         d_out,c.d_soff,c.d_stat,c.d_limit,c.d_order,NULL,c.n_coop);
   else
-    rc = spec_decode();
+    rc = qv_cands_decode(ctx,d_in,n,d_tab4,coding,upper,c);
   if (rc != DX_OK) return rc;
   if (direct && !ctx->keep_index)
     { // the usual end of the call: the device checks that the decode confirmed the layout (the chain
@@ -2011,7 +2111,8 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
       int32_t *h_chk = (int32_t *) dx_hpin_get(ctx,8);
       if (!d_chk || !h_chk) return DX_E_NOMEM;
       DX_CUDA(ctx,cudaMemsetAsync(d_chk,0,8,ctx->stream));
-      if ((rc = dxk_qv_chain_check(ctx,d_q,nc,d_keep,d_rlen_d,d_stat,d_soff,d_last,d_ffrun,first,n,d_chk)) != DX_OK) return rc;
+      if ((rc = dxk_qv_chain_check(ctx,d_q,nc,d_keep,d_rlen_d,c.d_stat,c.d_soff,c.d_last,c.d_ffrun,first,n,d_chk)) != DX_OK)
+        return rc;
       DX_CUDA(ctx,cudaMemcpyAsync(h_chk,d_chk,8,cudaMemcpyDeviceToHost,ctx->stream));
       DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
       ph.mark("decode");
@@ -2025,25 +2126,21 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
           return DX_OK;
         }
     }
-  DX_CUDA(ctx,cudaMemcpyAsync(h_soff,d_soff,N*48,cudaMemcpyDeviceToHost,ctx->stream));
-  DX_CUDA(ctx,cudaMemcpyAsync(h_stat,d_stat,N*4,cudaMemcpyDeviceToHost,ctx->stream));
+  DX_CUDA(ctx,cudaMemcpyAsync(c.h_soff,c.d_soff,N*48,cudaMemcpyDeviceToHost,ctx->stream));
+  DX_CUDA(ctx,cudaMemcpyAsync(c.h_stat,c.d_stat,N*4,cudaMemcpyDeviceToHost,ctx->stream));
   DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
   ph.mark("decode");
 
-  // the chain (dx_chain.h): a candidate is the next entry iff the bytes between the end of the previous
-  // entry and its fields are 0xff ... 0xff, d with d != 0xff
-  size_t M = 0, kept = 0;
+  // the chain (dx_chain.h) over the whole image
+  const DxChainIn ci = { c.h_q, c.h_ffrun, c.h_last, c.h_stat, c.h_soff, h_keep, (int64_t) N, (int64_t) first, (int64_t) n };
+  int64_t m = 0;
   bool as_assumed = true;                 // the entries are the candidates of the assumed layout, with its deltas
-  for (size_t i = 0; i < N; i++) kept += (h_keep[i] != 0);
-  { DxChainIn ci = { h_q, h_ffrun, h_last, h_stat, h_soff, h_keep, (int64_t) N, (int64_t) first, (int64_t) n };
-    int64_t m = 0;
-    if (!dx_chain_walk(ci,well_in,h_cand,h_well,&m,&as_assumed)) return DX_OK;          // general path
-    M = (size_t) m;
-  }
+  if (!dx_chain_walk(ci,well_in,c.h_cand,c.h_well,&m,&as_assumed)) return DX_OK;          // general path
+  const size_t M = (size_t) m;
   ph.mark("chain");
+  size_t total = (size_t) direct_total;
   if (direct && as_assumed)
-    { h_tail->total = direct_total;
-      if (ctx->route[DXR_DEBUG])
+    { if (ctx->route[DXR_DEBUG])
         fprintf(stderr,"[dexb200 debug] undexqv: %zu candidates, %zu entries, decoded in place\n",N,M);
     }
   else
@@ -2052,45 +2149,29 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
           // (soff / status do not depend on where the text goes)
           if (ctx->route[DXR_DEBUG])
             fprintf(stderr,"[dexb200 debug] undexqv: %zu candidates (%zu in the assumed layout), %zu entries: "
-                           "not as assumed, decoding again\n",N,kept,M);
-          if ((rc = spec_decode()) != DX_OK) return rc;
+                           "not as assumed, decoding again\n",N,N - (size_t) std::count(h_keep,h_keep + N,0),M);
+          if ((rc = qv_cands_decode(ctx,d_in,n,d_tab4,coding,upper,c)) != DX_OK) return rc;
           direct = false;
         }
-      int32_t *d_cand = (int32_t *) dx_arena_get(ctx,M*4 + 4);
-      int32_t *d_wells = (int32_t *) dx_arena_get(ctx,M*4 + 4);
-      int64_t *d_src  = (int64_t *) dx_arena_get(ctx,M*8 + 8);
-      if (!d_cand || !d_wells || !d_src) return DX_E_NOMEM;
-      if (M > 0)
-        { DX_CUDA(ctx,cudaMemcpyAsync(d_cand,h_cand,M*4,cudaMemcpyHostToDevice,ctx->stream));
-          DX_CUDA(ctx,cudaMemcpyAsync(d_wells,h_well,M*4,cudaMemcpyHostToDevice,ctx->stream));
-        }
-      if ((rc = dxk_qv_text_len(ctx,(int64_t) M,d_cand,pa,NULL,d_wells,0,plen,d_len,d_well,d_flag)) != DX_OK) return rc;
-      if ((rc = dxk_scan_u32(ctx,d_len,(int64_t) M,d_opre)) != DX_OK) return rc;
-      if ((rc = dxk_qv_build_ent(ctx,(int64_t) M,d_cand,pa,d_well,d_opre,d_len,d_toff,d_ent,d_src,NULL,NULL)) != DX_OK) return rc;
-      DX_CUDA(ctx,cudaMemcpyAsync(&h_tail->total,d_opre+M,8,cudaMemcpyDeviceToHost,ctx->stream));
-      DX_CUDA(ctx,cudaMemcpyAsync(&h_tail->flag,d_flag,4,cudaMemcpyDeviceToHost,ctx->stream));
-      DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
-      if (h_tail->flag) return dx_fail(ctx,DX_E_FORMAT,"unusable read length in an entry header");
-      if ((size_t) h_tail->total > cap)
-        return dx_fail_cap(ctx,(size_t) (h_tail->total),cap);
-      if ((rc = dxk_qv_assemble(ctx,d_tmp,tmp_n,d_ent,d_src,(int64_t) M,d_prefix,plen,d_out)) != DX_OK) return rc;
+      if ((rc = qv_layout(ctx,c,M,plen,d_flag,false,&total)) != DX_OK) return rc;
+      if (total > cap) return dx_fail_cap(ctx,total,cap);
+      if ((rc = dxk_qv_assemble(ctx,c.d_tmp,c.tmp_n,c.d_ent,c.d_src,(int64_t) M,d_prefix,plen,d_out)) != DX_OK) return rc;
       DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
       ph.mark("assemble");
     }
   ph.report("undexqv (entries discovered)");
   if (ctx->keep_index)
-    { std::vector<dx_index_row> &ix = *(std::vector<dx_index_row> *) ctx->last_index;
-      std::vector<QvDecEntry> he;
-      if ((rc = download(ctx,d_ent,direct ? N : M,he)) != DX_OK) return rc;     // direct: one row per candidate
-      ix.resize(M);
-      for (size_t m = 0; m < M; m++)
-        { const size_t c = (size_t) h_cand[m];
-          const QvDecEntry &d = he[direct ? c : m];
-          ix[m].stream_off = h_q[c] + 12; ix[m].end_off = h_soff[6*c + 5];
-          ix[m].text_off = d.text_off; ix[m].rlen = d.end - d.beg; ix[m].well = d.well;
+    { std::vector<QvDecEntry> he;
+      if ((rc = download(ctx,direct ? d_ent : c.d_ent,direct ? N : M,he)) != DX_OK) return rc;   // direct: one row per candidate
+      std::vector<QvDecEntry> ent(M);
+      std::vector<int64_t> stream_off(M), end_off(M);
+      for (size_t i = 0; i < M; i++)
+        { const size_t k = (size_t) c.h_cand[i];
+          ent[i] = he[direct ? k : i]; stream_off[i] = c.h_q[k] + 12; end_off[i] = c.h_soff[6*k + 5];
         }
+      set_last_index(ctx,M,ent.data(),stream_off.data(),end_off.data());
     }
-  *out_len = (size_t) h_tail->total;
+  *out_len = total;
   *handled = true;
   return DX_OK;
 }
@@ -2172,14 +2253,7 @@ extern "C" int dx_undexqv_dev(dx_ctx *ctx, const uint8_t *d_in, size_t n, int up
   DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
   if (stat) return dx_fail(ctx,DX_E_TRUNC,"Could not read more bits (Decode)");
   if (ctx->keep_index && ctx->last_index && plan.ix_fs.size() == N)
-    { std::vector<dx_index_row> &ix = *(std::vector<dx_index_row> *) ctx->last_index;
-      ix.resize(N);
-      for (size_t i = 0; i < N; i++)
-        { ix[i].stream_off = plan.ix_fs[i]; ix[i].end_off = plan.ix_end[i];
-          ix[i].text_off = plan.ent[i].text_off; ix[i].rlen = plan.ent[i].end - plan.ent[i].beg;
-          ix[i].well = plan.ent[i].well;
-        }
-    }
+    set_last_index(ctx,N,plan.ent.data(),plan.ix_fs.data(),plan.ix_end.data());
   *out_len = plan.text_len;
   return DX_OK;
 }
@@ -2208,16 +2282,12 @@ extern "C" int dx_qv_load_entries_dev(dx_ctx *ctx, const uint8_t *d_in, size_t n
   if (N == 0) return DX_OK;
   if ((size_t) toff[N] > cap)
     return dx_fail_cap(ctx,(size_t) (toff[N]),cap);
-  QvDecTables4 *h4 = (QvDecTables4 *) malloc(sizeof(QvDecTables4));
-  if (h4 == NULL) return DX_E_NOMEM;
-  if (!build_dec_tables4(coding,h4))
-    { free(h4);
-      return dx_fail(ctx,DX_E_CODING,"dx_qv_load_entries_dev: the coding has more long codes than the decode tables hold");
-    }
   QvDecTables4 *d_tab4 = (QvDecTables4 *) dx_arena_get(ctx,sizeof(QvDecTables4));
-  rc = d_tab4 ? upload(ctx,d_tab4,h4,1) : DX_E_NOMEM;
-  free(h4);
-  if (rc != DX_OK) return rc;
+  if (d_tab4 == NULL) return DX_E_NOMEM;
+  bool fits = false;
+  if ((rc = qv_tables4(ctx,coding,NULL,false,d_tab4,&fits)) != DX_OK) return rc;
+  if (!fits)
+    return dx_fail(ctx,DX_E_CODING,"dx_qv_load_entries_dev: the coding has more long codes than the decode tables hold");
   int64_t *d_start = (int64_t *) dx_arena_get(ctx,N*8);
   int32_t *d_rlen  = (int32_t *) dx_arena_get(ctx,N*4);
   int64_t *d_toff  = (int64_t *) dx_arena_get(ctx,(N+1)*8);
@@ -2343,15 +2413,9 @@ static int undexqv_pipe(dx_ctx *ctx, const uint8_t *h_in, size_t n, int upper, u
   const size_t kMinChunk = ctx->route[DXR_PIPE_CHUNK] > 0 ? (size_t) ctx->route[DXR_PIPE_CHUNK] : (size_t) 32 << 20;
   if (n < 2*kMinChunk || kMinChunk < 16384 || ctx->route[DXR_SERIAL_IO] || ctx->route[DXR_DECODER] == 1 || ctx->route[DXR_NO_SPEC] ||
       ctx->route[DXR_NO_FAST] || ctx->keep_index) return DX_OK;
-  uint16_t key; memcpy(&key,h_in,2);
-  if (key != 0x55aa) return DX_OK;
-  dx_qv_coding coding;
-  std::vector<char> prefix(100001);
-  size_t used = 0;
-  if (dx_qv_read_coding(h_in+2,n-2 < 300000 ? n-2 : 300000,&coding,prefix.data(),(int) prefix.size(),&used) != DX_OK ||
-      coding.flip) return DX_OK;
-  const size_t first = 2 + used;
-  const int plen = (int) strlen(prefix.data());
+  QvHead hd;
+  if (qv_read_head(h_in,2 + (n-2 < 300000 ? n-2 : 300000),hd) != DX_OK || hd.key != 0x55aa || hd.coding.flip) return DX_OK;
+  const int plen = hd.plen;
   // every window's decode launch lasts about as long as its longest entry (~2 ms with 60 000-position
   // entries), whatever else it holds: windows must stay large enough for the launch to hide behind the
   // text copy of the window before it
@@ -2372,6 +2436,7 @@ static int undexqv_pipe(dx_ctx *ctx, const uint8_t *h_in, size_t n, int upper, u
       DX_CUDA(ctx,cudaMemcpyAsync(ctx->io_in + a,h_in + a,b - a,cudaMemcpyHostToDevice,ctx->cs_in));
       DX_CUDA(ctx,cudaEventRecord(ctx->pev[k],ctx->cs_in));
     }
+
   auto drain = [&]() { cudaStreamSynchronize(ctx->cs_in); cudaStreamSynchronize(ctx->cs_out);
                        cudaStreamSynchronize(ctx->stream); };
 
@@ -2380,24 +2445,16 @@ static int undexqv_pipe(dx_ctx *ctx, const uint8_t *h_in, size_t n, int upper, u
   char *d_prefix = (char *) dx_arena_get(ctx,(size_t) plen + 1);
   char *h_prefix = (char *) dx_hpin_get(ctx,(size_t) plen + 1);
   int32_t *d_flag = (int32_t *) dx_arena_get(ctx,16);
-  if (!h4 || !d_tab4 || !d_prefix || !h_prefix || !d_flag) { drain(); return DX_E_NOMEM; }
-  if (!build_dec_tables4(&coding,h4)) { drain(); return DX_OK; }
-  memcpy(h_prefix,prefix.data(),(size_t) plen + 1);
-  if ((rc = dxk_fetch(ctx,d_tab4,h4,sizeof(QvDecTables4))) != DX_OK) { drain(); return rc; }
+  QvTail *h_tail = (QvTail *) dx_hpin_get(ctx,sizeof(QvTail));
+  if (!h4 || !d_tab4 || !d_prefix || !h_prefix || !d_flag || !h_tail) { drain(); return DX_E_NOMEM; }
+  bool fits = false;
+  if ((rc = qv_tables4(ctx,&hd.coding,h4,true,d_tab4,&fits)) != DX_OK || !fits) { drain(); return rc; }
+  memcpy(h_prefix,hd.prefix.data(),(size_t) plen + 1);
   if ((rc = dxk_fetch(ctx,d_prefix,h_prefix,(size_t) plen + 1)) != DX_OK) { drain(); return rc; }
   DX_CUDA(ctx,cudaMemsetAsync(d_flag,0,16,ctx->stream));
-  int minbits = 0;
-  for (int k = 2; k <= 3; k++)
-    { int mn = 32;
-      for (int x = 0; x < 256; x++)
-        if (coding.tab[k].lens[x] > 0 && coding.tab[k].lens[x] < mn) mn = coding.tab[k].lens[x];
-      minbits += (mn == 32) ? 0 : mn;
-    }
-  struct Tail { int64_t total; int32_t flag; int32_t pad; };
-  Tail *h_tail = (Tail *) dx_hpin_get(ctx,sizeof(Tail));
-  if (h_tail == NULL) { drain(); return DX_E_NOMEM; }
+  const int minbits = qv_minbits(hd.coding);
 
-  int64_t cur = (int64_t) first;           // image offset of the next entry (chain position)
+  int64_t cur = (int64_t) hd.first;        // image offset of the next entry (chain position)
   int32_t well = 0;
   size_t  tbase = 0;                       // text bytes of the windows before this one
   const size_t kBack = 4096;               // bytes before a window's first candidate the kernels may look at
@@ -2406,103 +2463,38 @@ static int undexqv_pipe(dx_ctx *ctx, const uint8_t *h_in, size_t n, int upper, u
       const size_t avail = ((size_t) (k + 2)*chunk < n) ? (size_t) (k + 2)*chunk : n;  // bytes on the device
       DX_CUDA(ctx,cudaStreamWaitEvent(ctx->stream,ctx->pev[(k + 1 < K) ? k + 1 : k],0));
       const size_t base = (k == 0) ? 0 : wa - kBack;                   // the window's own origin
-      const size_t wfirst = (k == 0) ? first : kBack;
+      const size_t wfirst = (k == 0) ? hd.first : kBack;
       const uint8_t *w_in = d_in + base;
       const size_t w_n = avail - base;
       const size_t scan_n = ((wb + 64 < avail) ? wb + 64 : avail) - base;
       int64_t *d_q = NULL, nc = 0;
       if ((rc = dxk_index_positions(ctx,DX_PRED_QVCAND,w_in,scan_n,wfirst + (k == 0 ? 1 : 0),&d_q,&nc)) != DX_OK)
         { drain(); return rc; }
-      const size_t N = (size_t) nc;
-      if (N == 0)
+      if (nc == 0)
         { if (cur < (int64_t) wb) { drain(); return DX_OK; }          // entries here, but no candidate
           continue;
         }
-      QvPlanArrays pa;
-      pa.fs   = (int64_t *)  dx_arena_get(ctx,N*8);  pa.rlen = (int32_t *)  dx_arena_get(ctx,N*4);
-      pa.delta= (uint32_t *) dx_arena_get(ctx,N*4);  pa.beg  = (int32_t *)  dx_arena_get(ctx,N*4);
-      pa.end  = (int32_t *)  dx_arena_get(ctx,N*4);  pa.qv   = (int32_t *)  dx_arena_get(ctx,N*4);
-      uint32_t *d_tlen  = (uint32_t *) dx_arena_get(ctx,N*4);
-      int64_t  *d_limit = (int64_t *)  dx_arena_get(ctx,N*8);
-      int32_t  *d_ffrun = (int32_t *)  dx_arena_get(ctx,N*4);
-      uint8_t  *d_last  = (uint8_t *)  dx_arena_get(ctx,N);
-      int64_t  *d_toff  = (int64_t *)  dx_arena_get(ctx,(N+1)*8);
-      int64_t  *d_soff  = (int64_t *)  dx_arena_get(ctx,N*48);
-      int32_t  *d_stat  = (int32_t *)  dx_arena_get(ctx,N*4);
-      int32_t  *d_order = (int32_t *)  dx_arena_get(ctx,N*4);
-      int64_t *h_q     = (int64_t *) dx_hpin_get(ctx,N*8);
-      int32_t *h_ffrun = (int32_t *) dx_hpin_get(ctx,N*4);
-      uint8_t *h_last  = (uint8_t *) dx_hpin_get(ctx,N);
-      int32_t *h_rlen  = (int32_t *) dx_hpin_get(ctx,N*4);
-      int32_t *h_order = (int32_t *) dx_hpin_get(ctx,N*4);
-      int64_t *h_soff  = (int64_t *) dx_hpin_get(ctx,N*48);
-      int32_t *h_stat  = (int32_t *) dx_hpin_get(ctx,N*4);
-      int32_t *h_cand  = (int32_t *) dx_hpin_get(ctx,N*4);
-      int32_t *h_well  = (int32_t *) dx_hpin_get(ctx,N*4);
-      if (!pa.fs || !pa.rlen || !pa.delta || !pa.beg || !pa.end || !pa.qv || !d_tlen || !d_limit || !d_ffrun ||
-          !d_last || !d_toff || !d_soff || !d_stat || !d_order || !h_q || !h_ffrun || !h_last || !h_rlen ||
-          !h_order || !h_soff || !h_stat || !h_cand || !h_well) { drain(); return DX_E_NOMEM; }
-      if ((rc = dxk_qv_cand_prep(ctx,w_in,w_n,wfirst,d_q,nc,4,minbits,pa,d_tlen,d_limit,d_ffrun,d_last)) != DX_OK ||
-          (rc = dxk_scan_u32(ctx,d_tlen,nc,d_toff)) != DX_OK) { drain(); return rc; }
-      if ((rc = dxk_fetch(ctx,h_q,d_q,N*8)) != DX_OK) { drain(); return rc; }
-      if ((rc = dxk_fetch(ctx,h_ffrun,d_ffrun,N*4)) != DX_OK) { drain(); return rc; }
-      if ((rc = dxk_fetch(ctx,h_last,d_last,N)) != DX_OK) { drain(); return rc; }
-      if ((rc = dxk_fetch(ctx,h_rlen,pa.rlen,N*4)) != DX_OK) { drain(); return rc; }
-      if ((rc = dxk_fetch(ctx,&h_tail->total,d_toff+N,8)) != DX_OK) { drain(); return rc; }
+      QvCands c;
+      if ((rc = qv_cands_prep(ctx,w_in,w_n,wfirst,d_q,nc,minbits,h_tail,c)) != DX_OK ||
+          (rc = qv_cands_plan(ctx,c,true)) != DX_OK ||
+          (rc = qv_cands_decode(ctx,w_in,w_n,d_tab4,hd.coding,upper,c)) != DX_OK ||
+          (rc = dxk_fetch(ctx,c.h_soff,c.d_soff,c.N*48)) != DX_OK ||
+          (rc = dxk_fetch(ctx,c.h_stat,c.d_stat,c.N*4)) != DX_OK) { drain(); return rc; }
       DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
-      const int64_t n_coop = ticket_plan(ctx,h_rlen,N,h_order);
-      if ((rc = dxk_fetch(ctx,d_order,h_order,N*4)) != DX_OK) { drain(); return rc; }
-      const size_t tmp_n = (size_t) h_tail->total;
-      uint8_t *d_tmp = (uint8_t *) dx_arena_get(ctx,tmp_n + 64);
-      if (d_tmp == NULL) { drain(); return DX_E_NOMEM; }
-      if ((rc = dxk_qv_decode6x(ctx,w_in,w_n,d_tab4,coding.delchar,coding.subchar,upper,2,nc,pa.fs,pa.rlen,NULL,NULL,0,
-                                d_tmp,d_soff,d_stat,d_limit,d_order,d_toff,n_coop)) != DX_OK) { drain(); return rc; }
-      if ((rc = dxk_fetch(ctx,h_soff,d_soff,N*48)) != DX_OK) { drain(); return rc; }
-      if ((rc = dxk_fetch(ctx,h_stat,d_stat,N*4)) != DX_OK) { drain(); return rc; }
-      DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
-      // the chain (see resolve_chain), in window coordinates; it stops at the window's end
-      size_t M = 0;
-      { size_t i = 0;
-        const int64_t stop = (k + 1 < K) ? (int64_t) (wb - base) : (int64_t) (n - base);
-        int64_t c = cur - (int64_t) base;
-        while (c < stop)
-          { while (i < N && h_q[i] - 1 < c) i++;
-            while (i < N && h_last[i] == 0xff && h_q[i] - 1 - c <= h_ffrun[i]) i++;
-            if (i >= N || h_stat[i] != 0) { drain(); return DX_OK; }
-            const int64_t gap = h_q[i] - 1 - c;
-            if (gap > h_ffrun[i] || h_last[i] == 0xff) { drain(); return DX_OK; }
-            const int64_t end = h_soff[6*i + 5];
-            if (end > (int64_t) w_n || end <= c) { drain(); return DX_OK; }
-            well += 255 * (int32_t) gap + h_last[i];
-            h_cand[M] = (int32_t) i; h_well[M] = well; M++;
-            c = end;
-            i++;
-          }
-        cur = c + (int64_t) base;
-      }
+      // the chain in window coordinates; it stops at the window's end
+      const DxChainIn ci = { c.h_q, c.h_ffrun, c.h_last, c.h_stat, c.h_soff, NULL, nc, (int64_t) wfirst, (int64_t) w_n,
+                             cur - (int64_t) base, (int64_t) (((k + 1 < K) ? wb : n) - base) };
+      int64_t M = 0, stop = 0;
+      bool as_assumed;
+      if (!dx_chain_walk(ci,well,c.h_cand,c.h_well,&M,&as_assumed,&stop)) { drain(); return DX_OK; }
+      cur = stop + (int64_t) base;
       if (M == 0) continue;
-      int32_t *d_cand = (int32_t *) dx_arena_get(ctx,M*4 + 4);
-      int32_t *d_wells = (int32_t *) dx_arena_get(ctx,M*4 + 4);
-      int32_t *d_well = (int32_t *) dx_arena_get(ctx,M*4 + 4);
-      uint32_t *d_len = (uint32_t *) dx_arena_get(ctx,M*4 + 4);
-      int64_t *d_opre = (int64_t *) dx_arena_get(ctx,(M+1)*8);
-      int64_t *d_src  = (int64_t *) dx_arena_get(ctx,M*8 + 8);
-      QvDecEntry *d_ent = (QvDecEntry *) dx_arena_get(ctx,(M+1)*sizeof(QvDecEntry));
-      if (!d_cand || !d_wells || !d_well || !d_len || !d_opre || !d_src || !d_ent) { drain(); return DX_E_NOMEM; }
-      if ((rc = dxk_fetch(ctx,d_cand,h_cand,M*4)) != DX_OK) { drain(); return rc; }
-      if ((rc = dxk_fetch(ctx,d_wells,h_well,M*4)) != DX_OK) { drain(); return rc; }
-      if ((rc = dxk_qv_text_len(ctx,(int64_t) M,d_cand,pa,NULL,d_wells,0,plen,d_len,d_well,d_flag)) != DX_OK ||
-          (rc = dxk_scan_u32(ctx,d_len,(int64_t) M,d_opre)) != DX_OK ||
-          (rc = dxk_qv_build_ent(ctx,(int64_t) M,d_cand,pa,d_well,d_opre,d_len,d_toff,d_ent,d_src,NULL,NULL)) != DX_OK)
-        { drain(); return rc; }
-      if ((rc = dxk_fetch(ctx,&h_tail->total,d_opre+M,8)) != DX_OK) { drain(); return rc; }
-      if ((rc = dxk_fetch(ctx,&h_tail->flag,d_flag,4)) != DX_OK) { drain(); return rc; }
-      DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
-      if (h_tail->flag) { drain(); return dx_fail(ctx,DX_E_FORMAT,"unusable read length in an entry header"); }
-      const size_t wtext = (size_t) h_tail->total;
+      well = c.h_well[M-1];
+      size_t wtext = 0;
+      if ((rc = qv_layout(ctx,c,(size_t) M,plen,d_flag,true,&wtext)) != DX_OK) { drain(); return rc; }
       if (tbase + wtext > cap)
         { drain(); return dx_fail(ctx,DX_E_CAP,"output needs more than %zu bytes",cap); }
-      if ((rc = dxk_qv_assemble(ctx,d_tmp,tmp_n,d_ent,d_src,(int64_t) M,d_prefix,plen,d_out + tbase)) != DX_OK)
+      if ((rc = dxk_qv_assemble(ctx,c.d_tmp,c.tmp_n,c.d_ent,c.d_src,M,d_prefix,plen,d_out + tbase)) != DX_OK)
         { drain(); return rc; }
       // this window's text leaves while the next window is decoded
       DX_CUDA(ctx,cudaEventRecord(ctx->pev[K + k],ctx->stream));

@@ -38,22 +38,26 @@ struct DxChainIn
   const int32_t *stat;     // [N] != 0: the candidate did not decode
   const int64_t *soff;     // [N][6] stream offsets of the decode; [5] = first byte behind the entry
   const uint8_t *keep;     // [N] part of the layout assumed in advance (NULL: nothing was assumed)
-  int64_t N, first, n;     // candidates, first byte behind the coding header, image length
+  int64_t N, first, n;     // candidates, first byte behind the coding header, bytes every entry ends within
+  int64_t start = first,   // the walk's first entry and its bound (entries start below it); left out: the
+          stop = n;        // whole image
 };
 
-// One step of the reference's loop for every entry of the image.  cand[m] / well[m] (m < *M): the
-// candidate that is entry m and its well number.  *as_assumed: the entries are exactly the kept
-// candidates and no entry but the first has 0xff delta bytes.  Returns false when the chain breaks
-// (an entry the candidates miss, a candidate that did not decode): the caller takes the general path.
+// One step of the reference's loop for every entry that starts in [start, stop).  cand[m] / well[m]
+// (m < *M): the candidate that is entry m and its well number.  *as_assumed: the entries are exactly
+// the kept candidates and no entry but the first has 0xff delta bytes.  *cur_out (if asked for): where
+// the next entry starts (windows that carry it and the last well walk the chain of one whole walk).
+// Returns false when the chain breaks (an entry the candidates miss, a candidate that did not decode):
+// the caller takes the general path.
 static inline bool dx_chain_walk(const DxChainIn &c, int32_t well_in, int32_t *cand, int32_t *well_out,
-                                 int64_t *M_out, bool *as_assumed)
+                                 int64_t *M_out, bool *as_assumed, int64_t *cur_out = NULL)
 { int64_t M = 0, kept = 0;
   bool same = true;
   if (c.keep != NULL)
     for (int64_t i = 0; i < c.N; i++) kept += (c.keep[i] != 0);
-  int64_t cur = c.first, i = 0;
+  int64_t cur = c.start, i = 0;
   int32_t well = well_in;
-  while (cur < c.n)
+  while (cur < c.stop)
     { while (i < c.N && c.q[i] - 1 < cur) i++;
       // a candidate whose terminator byte is 0xff is no terminator: part of a longer delta
       while (i < c.N && c.last[i] == 0xff && c.q[i] - 1 - cur <= c.ffrun[i]) i++;
@@ -71,6 +75,7 @@ static inline bool dx_chain_walk(const DxChainIn &c, int32_t well_in, int32_t *c
   if (M != kept) same = false;
   *M_out = M;
   *as_assumed = same;
+  if (cur_out != NULL) *cur_out = cur;
   return true;
 }
 

@@ -43,9 +43,9 @@ struct QvDecTables
   int32_t type[6];
 };
 
-// Compact two-level decode tables for the parallel decoder (dx_qv_decode2.cu): the top 11 bits of
-// the 16-bit window index prim; codes longer than 11 bits go through a 32-entry sub-table.
-// entry = symbol | length << 8 ; bit 15 of a prim entry = "low 15 bits are a sub-table index".
+// Compact two-level decode tables for the parallel decoders (dx_qv_decode5.cu, dx_qv_decode6.cu): the
+// top 11 bits of the 16-bit window index prim; codes longer than 11 bits go through a 32-entry
+// sub-table.  entry = symbol | length << 8 ; bit 15 of a prim entry = "low 15 bits are a sub-table index".
 #define DX_DEC2_MAXSUB 64
 struct QvDecTables2
 { uint16_t prim[6][2048];
@@ -53,8 +53,8 @@ struct QvDecTables2
   int32_t  type[6];
 };
 
-// Tables of the fourth-generation decoder (dx_qv_decode4.cu): 12-bit primary tables that are copied
-// to shared memory per stream.  multi: plain streams, up to two symbols per entry (bits 0-4 total
+// Tables of the parallel decoders (dx_qv_decode5.cu, dx_qv_decode6.cu): 12-bit primary tables that are
+// copied to shared memory per stream.  multi: plain streams, up to two symbols per entry (bits 0-4 total
 // length incl. the 8 literal bits of an escape, 5-6 symbol count, bit 7 escape, 8-12 length of the
 // first code, 16-23 / 24-31 the symbols); single: sym | len << 8.  0 = code longer than 12 bits
 // (or no code): look in t2.  abits: predicted stream bits per output position.

@@ -15,7 +15,11 @@
 //   2. (there is a kept candidate and all of them pass dx_chain_check_one)  <=>  (the walk succeeds and
 //      reports as_assumed);
 //   3. when as_assumed holds, the wells the layout assumed (first delta 255*ffrun + d, later ones d)
-//      are the walk's wells.
+//      are the walk's wells;
+//   4. the walk cut into windows at random bounds, each window starting at the cursor the one before
+//      stopped at and carrying the last well (as the pipelined host decode walks): every window stops
+//      at the first entry that starts at or past its bound, and together they find the same entries and
+//      wells as the whole walk and end at n -- or, when the whole walk fails, a window fails.
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -34,7 +38,7 @@ struct Cand { int64_t q; int64_t end; int32_t stat; bool truth; int32_t well; };
 
 int main(int argc, char **argv)
 { const int rounds = (argc > 1) ? atoi(argv[1]) : 20000;
-  long assumed = 0, broken = 0, walked = 0;
+  long assumed = 0, broken = 0, walked = 0, windowed = 0;
   for (int round = 0; round < rounds; round++)
     { rng_state += 0x632be59bd9b4e019ull * (uint64_t) (round + 1);
       const int style = (int) rnd(4);                  // 0: tidy files, 3: everything at once
@@ -116,9 +120,11 @@ int main(int argc, char **argv)
         }
       DxChainIn ci = { q.data(), ffrun.data(), last.data(), stat.data(), soff.data(), keep.data(), N, first, n };
       std::vector<int32_t> cand(N + 1), wells(N + 1);
-      int64_t M = 0;
+      int64_t M = 0, stop = 0;
       bool as_assumed = false;
-      const bool ok = dx_chain_walk(ci,well_in,cand.data(),wells.data(),&M,&as_assumed);
+      const bool ok = dx_chain_walk(ci,well_in,cand.data(),wells.data(),&M,&as_assumed,&stop);
+      if (ok && stop != n)
+        { fprintf(stderr,"round %d: the walk stopped at %lld, image length %lld\n",round,(long long) stop,(long long) n); return 1; }
 
       // 1. the walk against the truth
       bool all_decoded = true;
@@ -167,7 +173,43 @@ int main(int argc, char **argv)
             }
           assumed++;
         }
+
+      // 4. window by window (the bounds are drawn without changing the images of the later rounds)
+      { const uint64_t image_rng = rng_state;
+        std::vector<int64_t> bounds;                                      // the windows' stops, the last one n
+        const int nwin = 2 + (int) rnd(6);
+        for (int w = 0; w + 1 < nwin; w++) bounds.push_back(first + (int64_t) rnd((uint32_t) (n - first)));
+        std::sort(bounds.begin(),bounds.end());
+        bounds.push_back(n);
+        DxChainIn wi = ci;
+        wi.keep = NULL;                                                   // the pipelined decode assumes no layout
+        std::vector<int32_t> wc(N + 1), ww(N + 1), allc, allw;
+        int32_t wwell = well_in;
+        bool wok = true, dummy;
+        int busy = 0;                                                     // windows with an entry (or the break)
+        for (const int64_t b : bounds)
+          { int64_t m = 0, cur = 0;
+            wi.stop = b;
+            if (!dx_chain_walk(wi,wwell,wc.data(),ww.data(),&m,&dummy,&cur)) { wok = false; busy++; break; }
+            const int64_t last_start = (m > 1) ? soff[6*wc[m-2] + 5] : wi.start;    // where its last entry starts
+            if (cur < b || (m > 0 && last_start >= b))
+              { fprintf(stderr,"round %d: a window bounded by %lld stopped at %lld, its last entry starts at %lld\n",
+                        round,(long long) b,(long long) cur,(long long) last_start); return 1; }
+            if (m > 0) { wwell = ww[m-1]; busy++; }
+            allc.insert(allc.end(),wc.begin(),wc.begin() + m);
+            allw.insert(allw.end(),ww.begin(),ww.begin() + m);
+            wi.start = cur;
+          }
+        if (wok != ok ||
+            (ok && (wi.start != n || allc != std::vector<int32_t>(cand.begin(),cand.begin() + M) ||
+                    allw != std::vector<int32_t>(wells.begin(),wells.begin() + M))))
+          { fprintf(stderr,"round %d: windowed walk ok %d, whole walk ok %d (%zu windows, %zu / %lld entries)\n",round,
+                    (int) wok,(int) ok,bounds.size(),allc.size(),(long long) M); return 1; }
+        if (busy >= 2) windowed++;
+        rng_state = image_rng;
+      }
     }
-  printf("ok %d images: %ld walked to the truth, %ld as assumed, %ld broken chains refused\n",rounds,walked,assumed,broken);
+  printf("ok %d images: %ld walked to the truth, %ld as assumed, %ld broken chains refused, %ld walked in windows\n",
+         rounds,walked,assumed,broken,windowed);
   return 0;
 }

@@ -7,7 +7,8 @@ make -> write -> read.  Any report from a sanitizer fails the test.  CPU only.
 Also here: the entry-chain decision of csrc/dx_chain.h (which candidates of a .dexqv image are its
 entries), whose two forms -- the host's walk and the per-candidate predicate the device evaluates after
 an in-place decode -- are driven on 100 000 random images by tests/hostfuzz/fz_chain.cpp: the walk
-against the truth, the two forms against each other, the assumed wells against the walk's."""
+against the truth, the two forms against each other, the assumed wells against the walk's, and the
+walk cut into windows (as the pipelined host decode walks) against the whole walk."""
 import os
 import shutil
 import subprocess
@@ -78,5 +79,6 @@ def test_entry_chain_walk_and_device_predicate_agree(tmp_path):
         pytest.skip("sanitizer build not possible here: " + r.stderr[-300:])
     out = _run([str(exe), "100000"])
     assert out.startswith("ok 100000 images"), out
-    walked, assumed, broken = [int(x) for x in out.replace(":", " ").split() if x.isdigit()][1:4]
+    walked, assumed, broken, windowed = [int(x) for x in out.replace(":", " ").split() if x.isdigit()][1:5]
     assert walked > 80000 and assumed > 30000 and broken > 1000, out      # every branch was exercised
+    assert windowed > 60000, out                                          # ... the windowed walk too
