@@ -35,7 +35,7 @@ extern "C" {
 #define DX_E_TRUNC    (-3)   /* compressed input ends early (SYSTEM_READ_ERROR, DB.h:136-139)     */
 #define DX_E_KEY      (-4)   /* endian key invalid (undexta.c:156-159, undexar.c:142-145)         */
 #define DX_E_LINELEN  (-5)   /* lines of a .quiva entry differ in length (QV.c:792-795)           */
-#define DX_E_TOOLONG  (-6)   /* fasta/arrow line longer than MAX_BUFFER-2 (dexta.c:168-172)       */
+#define DX_E_TOOLONG  (-6)   /* fasta/arrow line longer than MAX_BUFFER-2 (dexta.c:168-172), .quiva entry of >= 2^24 positions */
 #define DX_E_ARG      (-7)   /* bad argument                                                      */
 #define DX_E_NOMEM    (-8)   /* host or device allocation failed                                  */
 #define DX_E_NOGPU    (-9)   /* no usable CUDA device: there is no CPU fallback                   */
@@ -169,7 +169,8 @@ typedef struct
 /* Pass 1.  Replaces QVcoding_Scan / QVcoding_Scan1 (QV.c:922-1023 / 866-920) over a whole
  * .quiva text (or one shard of it starting at an entry boundary): frames the entries, checks
  * them the way Read_Lines does (QV.c:751-798), and histograms the five streams.  The framing is
- * kept in the context and reused by dx_qv_encode_dev on the same buffer. */
+ * kept in the context and reused by dx_qv_encode_dev on the same buffer.  An entry of 2^24 positions
+ * or more is refused with DX_E_TOOLONG (the reference takes it; DESIGN section 2). */
 int dx_qv_scan_dev(dx_ctx *ctx, const uint8_t *d_text, size_t n, const dx_qv_carry *carry,
                    dx_qv_stats *stats);
 
@@ -214,7 +215,8 @@ int dx_text_lines_dev(dx_ctx *ctx, const uint8_t *d_text, size_t n, int64_t skip
                       int64_t *nlines, int64_t *skip_off);
 
 /* The whole tool on one GPU: scan, make coding, 0x55aa key + coding header, encode.
- * Replaces dexqv.c:59-147. */
+ * Replaces dexqv.c:59-147.  Like dx_qv_scan_dev, refuses an entry of 2^24 positions or more
+ * (DX_E_TOOLONG). */
 int dx_dexqv_dev (dx_ctx *ctx, const uint8_t *d_text, size_t n, int lossy,
                   uint8_t *d_out, size_t cap, size_t *out_len);
 int dx_dexqv_host(dx_ctx *ctx, const uint8_t *h_text, size_t n, int lossy,
