@@ -13,6 +13,7 @@
 #include <vector>
 #include <algorithm>
 #include <chrono>
+#include <new>
 #include "dx_internal.h"
 #include "dx_chain.h"
 
@@ -79,6 +80,7 @@ void dx_arena_reset(dx_ctx *ctx)
   for (int i = 0; i < ctx->nblk; i++)
     ctx->blk[i].top = 0;
   ctx->hpin_top = 0;
+  ctx->qv_range_live = 0;                               // its scratch is gone
 }
 
 // Pinned host scratch.  Pointers stay valid until the next dx_arena_reset: when the block is too
@@ -230,6 +232,8 @@ extern "C" int dx_open(int device, dx_ctx **out)
   return DX_OK;
 }
 
+static void qv_range_free(dx_ctx *ctx);
+
 extern "C" void dx_close(dx_ctx *ctx)
 { if (ctx == NULL) return;
   cudaSetDevice(ctx->device);
@@ -239,6 +243,7 @@ extern "C" void dx_close(dx_ctx *ctx)
   if (ctx->io_out)   cudaFree(ctx->io_out);
   if (ctx->qv_store) cudaFree(ctx->qv_store);
   if (ctx->last_index) delete (std::vector<dx_index_row> *) ctx->last_index;
+  qv_range_free(ctx);
   if (ctx->hpin)     cudaFreeHost(ctx->hpin);
   while (ctx->hpin_extra)
     { DxPinExtra *e = (DxPinExtra *) ctx->hpin_extra; ctx->hpin_extra = e->next; cudaFreeHost(e->p); free(e); }
@@ -2387,14 +2392,286 @@ extern "C" int dx_dexqv_host(dx_ctx *ctx, const uint8_t *h_text, size_t n, int l
 }
 
 // ------------------------------------------------------------------------------------------------
+//  One byte range of a .dexqv image: the entries whose FIRST byte (the first well-delta byte,
+//  undexqv.c:119-208 reads the delta first) lies in [a, b).  Three steps, so that callers with one
+//  range per GPU run the expensive one everywhere at once and hand on only the chain's position:
+//    qv_range_decode  the range's candidates, decoded speculatively (qv_cands_prep / plan / decode);
+//    qv_range_chain   the host walk from the carried position and well, bounded to the range
+//                     (dx_chain_walk_general: an entry the candidates miss is read and decoded by
+//                     itself, as plan_undexqv's general path does);
+//    qv_range_text    the text of the chain (qv_layout + k_qv_assemble); after a walk that needed the
+//                     slow path, the chain's entries are decoded once more as the only candidates.
+//  The kernels see the image bytes [base, base + w_n) at w_in, base at most 4096 bytes in front of
+//  the range (as far back as they look) and 16-byte aligned.  undexqv_pipe runs its windows through
+//  these steps; dx_undexqv_range_* expose them.
+// ------------------------------------------------------------------------------------------------
+struct QvRange
+{ dx_qv_coding  coding;             // set-up, the same for every range of one image
+  int           plen, minbits, upper;
+  int64_t       first;              // first byte behind the coding header
+  QvDecTables4 *d_tab4;
+  char         *d_prefix;
+  int32_t      *d_flag;
+  QvTail       *h_tail;
+  bool          by_kernel;          // small transfers through dxk_fetch (qv_copy)
+  const uint8_t *w_in;              // the range
+  size_t        w_n;
+  int64_t       base, a, b;
+  QvCands       c;
+  std::vector<DxChainEntry> ent;    // the chain, in window coordinates
+  bool          slow;               // some entry of it is no candidate of c
+};
+
+static void qv_range_free(dx_ctx *ctx)
+{ delete (QvRange *) ctx->qv_range;
+  ctx->qv_range = NULL;
+}
+
+// d_tab4 == NULL after a successful call: the coding has more long codes than the 12-bit tables hold
+static int qv_range_setup(dx_ctx *ctx, const QvHead &hd, int upper, bool by_kernel, QvRange &R)
+{ R.coding = hd.coding; R.plen = hd.plen; R.first = (int64_t) hd.first; R.upper = upper;
+  R.by_kernel = by_kernel; R.minbits = qv_minbits(hd.coding);
+  QvDecTables4 *h4 = (QvDecTables4 *) dx_hpin_get(ctx,sizeof(QvDecTables4));
+  char *h_prefix = (char *) dx_hpin_get(ctx,(size_t) R.plen + 1);
+  R.d_tab4   = (QvDecTables4 *) dx_arena_get(ctx,sizeof(QvDecTables4));
+  R.d_prefix = (char *) dx_arena_get(ctx,(size_t) R.plen + 1);
+  R.d_flag   = (int32_t *) dx_arena_get(ctx,16);
+  R.h_tail   = (QvTail *) dx_hpin_get(ctx,sizeof(QvTail));
+  if (!h4 || !h_prefix || !R.d_tab4 || !R.d_prefix || !R.d_flag || !R.h_tail) return DX_E_NOMEM;
+  bool fits = false;
+  int rc;
+  if ((rc = qv_tables4(ctx,&hd.coding,h4,by_kernel,R.d_tab4,&fits)) != DX_OK) return rc;
+  if (!fits) { R.d_tab4 = NULL; return DX_OK; }
+  memcpy(h_prefix,hd.prefix.data(),(size_t) R.plen + 1);
+  if ((rc = qv_copy(ctx,by_kernel,R.d_prefix,h_prefix,(size_t) R.plen + 1)) != DX_OK) return rc;
+  DX_CUDA(ctx,cudaMemsetAsync(R.d_flag,0,16,ctx->stream));
+  return DX_OK;
+}
+
+// the window origin of a range whose entries start at a >= first, in a buffer starting at image offset buf_off
+static int64_t qv_range_base(int64_t a, int64_t buf_off)
+{ const int64_t lo = (a > 4096) ? a - 4096 : 0;
+  return buf_off + ((lo - buf_off) & ~(int64_t) 15);
+}
+
+static int qv_range_decode(dx_ctx *ctx, QvRange &R, const uint8_t *w_in, size_t w_n, int64_t base, int64_t a, int64_t b)
+{ R.w_in = w_in; R.w_n = w_n; R.base = base; R.a = a; R.b = b;
+  R.c = QvCands();
+  R.ent.clear(); R.slow = false;
+  if (b <= a) return DX_OK;
+  const int64_t wfirst = a - base;
+  const int64_t scan_end = (b + 64 < base + (int64_t) w_n) ? b + 64 : base + (int64_t) w_n;
+  int64_t *d_q = NULL, nc = 0;
+  int rc;
+  if ((rc = dxk_index_positions(ctx,DX_PRED_QVCAND,w_in,(size_t) (scan_end - base),(size_t) wfirst + 1,&d_q,&nc)) != DX_OK)
+    return rc;
+  if (nc == 0) return DX_OK;
+  if ((rc = qv_cands_prep(ctx,w_in,w_n,(size_t) wfirst,d_q,nc,R.minbits,R.h_tail,R.c)) != DX_OK ||
+      (rc = qv_cands_plan(ctx,R.c,R.by_kernel)) != DX_OK ||
+      (rc = qv_cands_decode(ctx,w_in,w_n,R.d_tab4,R.coding,R.upper,R.c)) != DX_OK ||
+      (rc = qv_copy(ctx,R.by_kernel,R.c.h_soff,R.c.d_soff,R.c.N*48)) != DX_OK ||
+      (rc = qv_copy(ctx,R.by_kernel,R.c.h_stat,R.c.d_stat,R.c.N*4)) != DX_OK) return rc;
+  return DX_OK;
+}
+
+// Bytes an entry of rlen positions takes behind its fields, at most: in a run-length coded stream every
+// position a run code and a symbol code, both escaped; two bits per tag; each stream padded to words.
+static int64_t qv_entry_bound(const dx_qv_coding &cd, int64_t rlen)
+{ auto maxlen = [&](int k) { int m = 0; for (int x = 0; x < 256; x++) m = std::max(m,(int) cd.tab[k].lens[x]); return (int64_t) m; };
+  const int64_t bits[4] = { maxlen(0) + 8 + (cd.delchar >= 0 ? maxlen(1) + 16 : 0), maxlen(2) + 8, maxlen(3) + 8,
+                            maxlen(4) + 8 + (cd.subchar >= 0 ? maxlen(5) + 16 : 0) };
+  int64_t bytes = (rlen + 3) / 4 + 8;
+  for (int s = 0; s < 4; s++) bytes += (rlen * bits[s] + 7) / 8 + 8;
+  return bytes;
+}
+
+// DX_E_CAP: the range's buffer ends before the entry at image offset `at` does; it needs the image up to `need`
+static int qv_range_short(dx_ctx *ctx, const QvRange &R, int64_t at, int64_t need)
+{ dx_fail(ctx,DX_E_CAP,"the entry at image offset %lld runs past the end of the buffer (%lld): it needs the image up to %lld",
+          (long long) at,(long long) (R.base + (int64_t) R.w_n),(long long) need);
+  ctx->need_bytes = (size_t) need;
+  return DX_E_CAP;
+}
+
+struct QvSlowUser { dx_ctx *ctx; QvRange *R; };
+
+// dx_chain_walk_general's slow path: the entry at cur (window coordinates) read and decoded by itself
+static int qv_range_slow(void *user, int64_t cur, int64_t *q, int64_t *end, int32_t *delta)
+{ dx_ctx *ctx = ((QvSlowUser *) user)->ctx;
+  const QvRange &R = *((QvSlowUser *) user)->R;
+  const int64_t n = (int64_t) R.w_n;
+  std::vector<uint8_t> win;
+  int64_t p = cur;
+  int32_t add = 0;
+  int rc;
+  for (;;)                                                  // the delta bytes: 0xff ... 0xff, d
+    { if ((rc = peek(ctx,R.w_in,R.w_n,(size_t) p,4096,win)) != DX_OK) return rc;
+      size_t k = 0;
+      while (k < win.size() && win[k] == 0xff) k++;
+      add += 255 * (int32_t) k; p += (int64_t) k;
+      if (k < win.size()) { add += win[k]; p += 1; break; }
+      if (p >= n)                                           // a delta is at most 2^31 wells: 8 421 505 bytes
+        return qv_range_short(ctx,R,R.base + cur,R.base + cur + 8421505 + 12);
+    }
+  if ((rc = peek(ctx,R.w_in,R.w_n,(size_t) p,12,win)) != DX_OK) return rc;
+  if (win.size() < 12) return qv_range_short(ctx,R,R.base + cur,R.base + p + 12 + 65536);
+  const int32_t rlen = le32(win.data() + 4) - le32(win.data());
+  if (rlen < 0 || rlen >= (1 << 24))
+    return dx_fail(ctx,DX_E_FORMAT,"unusable read length %d in the entry header at image offset %lld",rlen,
+                   (long long) (R.base + p));
+  int64_t *d_start = (int64_t *) dx_arena_get(ctx,8);
+  int32_t *d_rlen  = (int32_t *) dx_arena_get(ctx,4);
+  int64_t *d_soff  = (int64_t *) dx_arena_get(ctx,48);
+  int32_t *d_stat  = (int32_t *) dx_arena_get(ctx,4);
+  if (!d_start || !d_rlen || !d_soff || !d_stat) return DX_E_NOMEM;
+  const int64_t start = p + 12;
+  if ((rc = upload(ctx,d_start,&start,1)) != DX_OK || (rc = upload(ctx,d_rlen,&rlen,1)) != DX_OK) return rc;
+  if ((rc = dxk_qv_decode5(ctx,R.w_in,R.w_n,R.d_tab4,R.coding.delchar,R.coding.subchar,0,0,1,d_start,d_rlen,
+                           NULL,NULL,0,NULL,d_soff,d_stat)) != DX_OK) return rc;
+  std::vector<int64_t> so; std::vector<int32_t> st;
+  if ((rc = download(ctx,d_soff,6,so)) != DX_OK || (rc = download(ctx,d_stat,1,st)) != DX_OK) return rc;
+  if (st[0] != 0 || so[5] > n || so[5] <= cur)
+    { const int64_t need = R.base + start + qv_entry_bound(R.coding,rlen);
+      if (need > R.base + n) return qv_range_short(ctx,R,R.base + cur,need);
+      return dx_fail(ctx,DX_E_TRUNC,"Could not read more bits (Decode), entry at image offset %lld",(long long) (R.base + cur));
+    }
+  *q = p; *end = so[5]; *delta = add;
+  return DX_OK;
+}
+
+static int qv_range_chain(dx_ctx *ctx, QvRange &R, int64_t cur_in, int32_t well_in, int64_t *cur_out, int32_t *well_out)
+{ DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));          // the candidates' ends and status
+  const QvCands &c = R.c;
+  const DxChainIn ci = { c.h_q, c.h_ffrun, c.h_last, c.h_stat, c.h_soff, NULL, (int64_t) c.N, R.a - R.base,
+                         (int64_t) R.w_n, cur_in - R.base, R.b - R.base };
+  QvSlowUser u = { ctx, &R };
+  int64_t stop = 0;
+  const int rc = dx_chain_walk_general(ci,well_in,qv_range_slow,&u,R.ent,&stop);
+  if (rc != DX_OK) { R.ent.clear(); return rc; }
+  R.slow = false;
+  for (const DxChainEntry &e : R.ent) R.slow = R.slow || (e.cand < 0);
+  *cur_out = stop + R.base;
+  *well_out = R.ent.empty() ? well_in : R.ent.back().well;
+  if (ctx->route[DXR_DEBUG] && R.slow)
+    fprintf(stderr,"[dexb200 debug] undexqv range [%lld, %lld): %zu entries, some found by the slow path\n",
+            (long long) R.a,(long long) R.b,R.ent.size());
+  return DX_OK;
+}
+
+static int qv_range_text(dx_ctx *ctx, QvRange &R, uint8_t *d_out, size_t cap, size_t *out_len)
+{ const size_t M = R.ent.size();
+  *out_len = 0;
+  if (M == 0) return DX_OK;
+  int rc;
+  bool redo = false;
+  if (R.slow)
+    { // entries the candidates did not give: the chain's own entries, decoded as the only candidates and
+      // without the speculative decode's limit (which also gives up on entries that synchronise late)
+      int64_t *h_q = (int64_t *) dx_hpin_get(ctx,M*8);
+      int64_t *d_q = (int64_t *) dx_arena_get(ctx,M*8);
+      if (!h_q || !d_q) return DX_E_NOMEM;
+      for (size_t m = 0; m < M; m++) { h_q[m] = R.ent[m].q; R.ent[m].cand = (int32_t) m; }
+      R.c = QvCands();
+      QvCands &c = R.c;
+      if ((rc = qv_copy(ctx,R.by_kernel,d_q,h_q,M*8)) != DX_OK ||
+          (rc = qv_cands_prep(ctx,R.w_in,R.w_n,(size_t) (R.a - R.base),d_q,(int64_t) M,0,R.h_tail,c)) != DX_OK ||
+          (rc = qv_cands_plan(ctx,c,R.by_kernel)) != DX_OK) return rc;
+      if ((c.d_tmp = (uint8_t *) dx_arena_get(ctx,c.tmp_n + 64)) == NULL) return DX_E_NOMEM;
+      if ((rc = dxk_qv_decode6x(ctx,R.w_in,R.w_n,R.d_tab4,R.coding.delchar,R.coding.subchar,R.upper,2,(int64_t) M,c.pa.fs,
+                                c.pa.rlen,NULL,NULL,0,c.d_tmp,c.d_soff,c.d_stat,NULL,c.d_order,c.d_toff,c.n_coop)) != DX_OK ||
+          (rc = qv_copy(ctx,R.by_kernel,c.h_stat,c.d_stat,M*4)) != DX_OK) return rc;
+      R.slow = false;
+      redo = true;
+    }
+  for (size_t m = 0; m < M; m++) { R.c.h_cand[m] = R.ent[m].cand; R.c.h_well[m] = R.ent[m].well; }
+  size_t total = 0;
+  if ((rc = qv_layout(ctx,R.c,M,R.plen,R.d_flag,R.by_kernel,&total)) != DX_OK) return rc;
+  for (size_t m = 0; redo && m < M; m++)                     // (qv_layout waited for the stream)
+    if (R.c.h_stat[m] != 0)
+      return dx_fail(ctx,DX_E_TRUNC,"Could not read more bits (Decode), entry at image offset %lld",
+                     (long long) (R.base + R.ent[m].q));
+  if (total > cap) return dx_fail_cap(ctx,total,cap);
+  if ((rc = dxk_qv_assemble(ctx,R.c.d_tmp,R.c.tmp_n,R.c.d_ent,R.c.d_src,(int64_t) M,R.d_prefix,R.plen,d_out)) != DX_OK)
+    return rc;
+  *out_len = total;
+  return DX_OK;
+}
+
+extern "C" int dx_undexqv_range_dev(dx_ctx *ctx, const uint8_t *h_head, size_t head_n, const uint8_t *d_buf,
+                                    size_t buf_n, int64_t buf_off, int64_t a, int64_t b, int upper, int64_t *first)
+{ if (ctx == NULL) return DX_E_ARG;
+  int rc;
+  if (h_head == NULL) return dx_fail(ctx,DX_E_ARG,"dx_undexqv_range_dev: h_head is NULL");
+  if ((rc = check_buf(ctx,d_buf,"range buffer")) != DX_OK) return rc;
+  QvHead hd;
+  if ((rc = qv_read_head(h_head,head_n,hd)) == DX_E_KEY)
+    return dx_fail(ctx,DX_E_KEY,"not a .dexqv file (endian key 0x%04x)",(unsigned) hd.key);
+  if (rc != DX_OK)
+    return dx_fail(ctx,rc,"Could not read the coding header (Read_QVcoding) from the %zu head bytes",head_n);
+  if (!hd.newv || hd.coding.flip)
+    return dx_fail(ctx,DX_E_FORMAT,"%s image: byte ranges take images of the 0x55aa layout in the native byte "
+                   "order; decode it whole with dx_undexqv_dev",hd.newv ? "a foreign-endian" : "an old-layout (key-less)");
+  if (first != NULL) *first = (int64_t) hd.first;
+  const int64_t A = std::max(a,(int64_t) hd.first), B = std::max(b,A);     // no entry starts inside the header
+  const int64_t base = qv_range_base(A,buf_off), buf_end = buf_off + (int64_t) buf_n;
+  if (a < 0 || a > b)
+    return dx_fail(ctx,DX_E_ARG,"dx_undexqv_range_dev: bad range [%lld, %lld)",(long long) a,(long long) b);
+  if (buf_off < 0 || base < buf_off || buf_end < b)
+    return dx_fail(ctx,DX_E_ARG,"dx_undexqv_range_dev: the buffer holds the image bytes [%lld, %lld), the range [%lld, %lld) "
+                   "needs at least [%lld, %lld)",(long long) buf_off,(long long) buf_end,(long long) a,(long long) b,
+                   (long long) (A > 4096 ? A - 4096 : 0),(long long) B);
+  cudaSetDevice(ctx->device);
+  dx_arena_reset(ctx);
+  if (ctx->qv_range == NULL) ctx->qv_range = new (std::nothrow) QvRange();
+  if (ctx->qv_range == NULL) return DX_E_NOMEM;
+  QvRange &R = *(QvRange *) ctx->qv_range;
+  if ((rc = qv_range_setup(ctx,hd,upper,false,R)) != DX_OK) return rc;
+  if (R.d_tab4 == NULL)
+    return dx_fail(ctx,DX_E_CODING,"the coding has more long codes than the parallel decode tables hold; decode this "
+                   "image whole with dx_undexqv_dev");
+  if (B == A)                                             // a range inside the header: no entry starts there
+    rc = qv_range_decode(ctx,R,d_buf,0,buf_off,A,B);
+  else
+    rc = qv_range_decode(ctx,R,d_buf + (base - buf_off),(size_t) (buf_end - base),base,A,B);
+  if (rc != DX_OK) return rc;
+  ctx->qv_range_live = 1;
+  return DX_OK;
+}
+
+extern "C" int dx_undexqv_range_chain(dx_ctx *ctx, int64_t cur_in, int32_t well_in, int64_t *cur_out, int32_t *well_out)
+{ if (ctx == NULL || cur_out == NULL || well_out == NULL) return DX_E_ARG;
+  if (!ctx->qv_range_live) return dx_fail(ctx,DX_E_ARG,"dx_undexqv_range_chain: no range decoded (dx_undexqv_range_dev)");
+  QvRange &R = *(QvRange *) ctx->qv_range;
+  if (cur_in < R.a)
+    return dx_fail(ctx,DX_E_ARG,"dx_undexqv_range_chain: the chain position %lld lies in front of the range [%lld, %lld)",
+                   (long long) cur_in,(long long) R.a,(long long) R.b);
+  cudaSetDevice(ctx->device);
+  const int rc = qv_range_chain(ctx,R,cur_in,well_in,cur_out,well_out);
+  if (rc != DX_OK) ctx->qv_range_live = (rc == DX_E_CAP) ? 0 : ctx->qv_range_live;
+  return rc;
+}
+
+extern "C" int dx_undexqv_range_text_dev(dx_ctx *ctx, uint8_t *d_out, size_t cap, size_t *out_len)
+{ if (ctx == NULL || out_len == NULL) return DX_E_ARG;
+  *out_len = 0;
+  if (!ctx->qv_range_live) return dx_fail(ctx,DX_E_ARG,"dx_undexqv_range_text_dev: no range decoded (dx_undexqv_range_dev)");
+  if (d_out == NULL && cap > 0) return dx_fail(ctx,DX_E_ARG,"dx_undexqv_range_text_dev: d_out is NULL");
+  cudaSetDevice(ctx->device);
+  int rc;
+  if ((rc = qv_range_text(ctx,*(QvRange *) ctx->qv_range,d_out,cap,out_len)) != DX_OK) return rc;
+  DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
+  return DX_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
 //  dx_undexqv_host as a pipeline: the image goes to the device in chunks (copy stream cs_in), every
-//  chunk is a WINDOW whose entries are found, decoded, verified and assembled as soon as it and its
+//  chunk is a WINDOW -- a byte range, through the three steps above -- decoded as soon as it and its
 //  successor have arrived (an entry may run over the boundary), and a window's text leaves for the
 //  host (copy stream cs_out) while the next window is decoded: PCIe is busy in both directions and
-//  the kernels hide behind the copies.  Same kernels and the same chain rule as undexqv_fast; the
-//  chain just carries its position, well number and text offset from window to window.  Anything
-//  unusual (legacy layout, a missed entry, tables that do not fit) -> *handled = false after the
-//  copies have drained, and the caller runs the plain path on the complete image.
+//  the kernels hide behind the copies.  The chain carries its position, well number and text offset
+//  from window to window.  Anything unusual (legacy layout, tables that do not fit, an entry longer
+//  than the bytes that have arrived, a malformed image) -> *handled = false after the copies have
+//  drained, and the caller runs the plain path on the complete image.
 // ------------------------------------------------------------------------------------------------
 static int pipe_setup(dx_ctx *ctx, int nev)
 { if (ctx->cs_in == NULL)  DX_CUDA(ctx,cudaStreamCreateWithFlags(&ctx->cs_in,cudaStreamNonBlocking));
@@ -2415,7 +2692,6 @@ static int undexqv_pipe(dx_ctx *ctx, const uint8_t *h_in, size_t n, int upper, u
       ctx->route[DXR_NO_FAST] || ctx->keep_index) return DX_OK;
   QvHead hd;
   if (qv_read_head(h_in,2 + (n-2 < 300000 ? n-2 : 300000),hd) != DX_OK || hd.key != 0x55aa || hd.coding.flip) return DX_OK;
-  const int plen = hd.plen;
   // every window's decode launch lasts about as long as its longest entry (~2 ms with 60 000-position
   // entries), whatever else it holds: windows must stay large enough for the launch to hide behind the
   // text copy of the window before it
@@ -2440,62 +2716,29 @@ static int undexqv_pipe(dx_ctx *ctx, const uint8_t *h_in, size_t n, int upper, u
   auto drain = [&]() { cudaStreamSynchronize(ctx->cs_in); cudaStreamSynchronize(ctx->cs_out);
                        cudaStreamSynchronize(ctx->stream); };
 
-  QvDecTables4 *h4 = (QvDecTables4 *) dx_hpin_get(ctx,sizeof(QvDecTables4));
-  QvDecTables4 *d_tab4 = (QvDecTables4 *) dx_arena_get(ctx,sizeof(QvDecTables4));
-  char *d_prefix = (char *) dx_arena_get(ctx,(size_t) plen + 1);
-  char *h_prefix = (char *) dx_hpin_get(ctx,(size_t) plen + 1);
-  int32_t *d_flag = (int32_t *) dx_arena_get(ctx,16);
-  QvTail *h_tail = (QvTail *) dx_hpin_get(ctx,sizeof(QvTail));
-  if (!h4 || !d_tab4 || !d_prefix || !h_prefix || !d_flag || !h_tail) { drain(); return DX_E_NOMEM; }
-  bool fits = false;
-  if ((rc = qv_tables4(ctx,&hd.coding,h4,true,d_tab4,&fits)) != DX_OK || !fits) { drain(); return rc; }
-  memcpy(h_prefix,hd.prefix.data(),(size_t) plen + 1);
-  if ((rc = dxk_fetch(ctx,d_prefix,h_prefix,(size_t) plen + 1)) != DX_OK) { drain(); return rc; }
-  DX_CUDA(ctx,cudaMemsetAsync(d_flag,0,16,ctx->stream));
-  const int minbits = qv_minbits(hd.coding);
+  QvRange R;
+  if ((rc = qv_range_setup(ctx,hd,upper,true,R)) != DX_OK || R.d_tab4 == NULL) { drain(); return rc; }
 
   int64_t cur = (int64_t) hd.first;        // image offset of the next entry (chain position)
   int32_t well = 0;
   size_t  tbase = 0;                       // text bytes of the windows before this one
-  const size_t kBack = 4096;               // bytes before a window's first candidate the kernels may look at
   for (int k = 0; k < K; k++)
-    { const size_t wa = (size_t) k*chunk, wb = (wa + chunk < n) ? wa + chunk : n;      // candidates of [wa, wb)
+    { const size_t wa = (size_t) k*chunk, wb = (wa + chunk < n) ? wa + chunk : n;      // entries starting in [wa, wb)
       const size_t avail = ((size_t) (k + 2)*chunk < n) ? (size_t) (k + 2)*chunk : n;  // bytes on the device
       DX_CUDA(ctx,cudaStreamWaitEvent(ctx->stream,ctx->pev[(k + 1 < K) ? k + 1 : k],0));
-      const size_t base = (k == 0) ? 0 : wa - kBack;                   // the window's own origin
-      const size_t wfirst = (k == 0) ? hd.first : kBack;
-      const uint8_t *w_in = d_in + base;
-      const size_t w_n = avail - base;
-      const size_t scan_n = ((wb + 64 < avail) ? wb + 64 : avail) - base;
-      int64_t *d_q = NULL, nc = 0;
-      if ((rc = dxk_index_positions(ctx,DX_PRED_QVCAND,w_in,scan_n,wfirst + (k == 0 ? 1 : 0),&d_q,&nc)) != DX_OK)
-        { drain(); return rc; }
-      if (nc == 0)
-        { if (cur < (int64_t) wb) { drain(); return DX_OK; }          // entries here, but no candidate
-          continue;
-        }
-      QvCands c;
-      if ((rc = qv_cands_prep(ctx,w_in,w_n,wfirst,d_q,nc,minbits,h_tail,c)) != DX_OK ||
-          (rc = qv_cands_plan(ctx,c,true)) != DX_OK ||
-          (rc = qv_cands_decode(ctx,w_in,w_n,d_tab4,hd.coding,upper,c)) != DX_OK ||
-          (rc = dxk_fetch(ctx,c.h_soff,c.d_soff,c.N*48)) != DX_OK ||
-          (rc = dxk_fetch(ctx,c.h_stat,c.d_stat,c.N*4)) != DX_OK) { drain(); return rc; }
-      DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
-      // the chain in window coordinates; it stops at the window's end
-      const DxChainIn ci = { c.h_q, c.h_ffrun, c.h_last, c.h_stat, c.h_soff, NULL, nc, (int64_t) wfirst, (int64_t) w_n,
-                             cur - (int64_t) base, (int64_t) (((k + 1 < K) ? wb : n) - base) };
-      int64_t M = 0, stop = 0;
-      bool as_assumed;
-      if (!dx_chain_walk(ci,well,c.h_cand,c.h_well,&M,&as_assumed,&stop)) { drain(); return DX_OK; }
-      cur = stop + (int64_t) base;
-      if (M == 0) continue;
-      well = c.h_well[M-1];
+      const int64_t a = std::max((int64_t) wa,(int64_t) hd.first), b = std::max((int64_t) wb,a);
+      const int64_t base = qv_range_base(a,0);
+      if ((rc = qv_range_decode(ctx,R,d_in + base,avail - (size_t) base,base,a,b)) != DX_OK) { drain(); return rc; }
+      int64_t stop = 0;
+      int32_t wlast = 0;
+      rc = qv_range_chain(ctx,R,cur,well,&stop,&wlast);
+      if (rc == DX_E_CAP || rc == DX_E_TRUNC || rc == DX_E_FORMAT) { drain(); return DX_OK; }    // the plain path decides
+      if (rc != DX_OK) { drain(); return rc; }
+      cur = stop; well = wlast;
+      if (R.ent.empty()) continue;
       size_t wtext = 0;
-      if ((rc = qv_layout(ctx,c,(size_t) M,plen,d_flag,true,&wtext)) != DX_OK) { drain(); return rc; }
-      if (tbase + wtext > cap)
-        { drain(); return dx_fail(ctx,DX_E_CAP,"output needs more than %zu bytes",cap); }
-      if ((rc = dxk_qv_assemble(ctx,c.d_tmp,c.tmp_n,c.d_ent,c.d_src,M,d_prefix,plen,d_out + tbase)) != DX_OK)
-        { drain(); return rc; }
+      if ((rc = qv_range_text(ctx,R,d_out + tbase,cap - tbase,&wtext)) != DX_OK)
+        { drain(); return (rc == DX_E_CAP) ? dx_fail(ctx,DX_E_CAP,"output needs more than %zu bytes",cap) : rc; }
       // this window's text leaves while the next window is decoded
       DX_CUDA(ctx,cudaEventRecord(ctx->pev[K + k],ctx->stream));
       DX_CUDA(ctx,cudaStreamWaitEvent(ctx->cs_out,ctx->pev[K + k],0));

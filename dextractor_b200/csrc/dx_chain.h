@@ -16,7 +16,10 @@
 //                       but the first below 255: there IS a kept candidate and ALL of them pass  <=>
 //                       the walk accepts exactly the kept candidates with no 0xff delta byte except
 //                       in front of the first (tests/hostfuzz/fz_chain.cpp drives both on random
-//                       images; it found the "there is one" half).
+//                       images; it found the "there is one" half);
+//   dx_chain_walk_general  the walk over one byte range of an image, which has no whole image to fall
+//                       back to: where the candidates break the chain, the entry is read by a slow path
+//                       (tests/hostfuzz/fz_chain_ranges.cpp walks random images range after range).
 //
 // Plain C++ (no CUDA types) so that the host, the kernel (dx_qv_plan.cu) and the fuzz harness share it.
 
@@ -24,6 +27,7 @@
 #define DX_CHAIN_H
 
 #include <stdint.h>
+#include <vector>
 
 #if defined(__CUDACC__)
 #define DX_CHAIN_HD __host__ __device__ __forceinline__
@@ -77,6 +81,47 @@ static inline bool dx_chain_walk(const DxChainIn &c, int32_t well_in, int32_t *c
   *as_assumed = same;
   if (cur_out != NULL) *cur_out = cur;
   return true;
+}
+
+// The walk without a way out, for a caller that has no whole image to fall back to (one byte range of
+// an image, dx_undexqv_range_*): wherever dx_chain_walk would return false, the entry at cur is taken
+// from `slow`, which reads its delta bytes and fields at cur and decodes that one entry by itself (the
+// reference's loop for a single entry): *q its fields, *end the first byte behind it (> cur), *delta
+// its well delta.  A candidate the filter missed, one whose speculative decode was cut short, a 0xff
+// run whose terminator lies beyond the candidates: none of them stops the walk.  Entry m is ent[m]
+// (cand -1: found by `slow`).  Returns 0, or the first non-zero status of `slow`.
+struct DxChainEntry { int64_t q, end; int32_t cand, well; };
+typedef int (*DxChainSlow)(void *user, int64_t cur, int64_t *q, int64_t *end, int32_t *delta);
+
+static inline int dx_chain_walk_general(const DxChainIn &c, int32_t well_in, DxChainSlow slow, void *user,
+                                        std::vector<DxChainEntry> &ent, int64_t *cur_out)
+{ int64_t cur = c.start, i = 0;
+  int32_t well = well_in;
+  ent.clear();
+  while (cur < c.stop)
+    { while (i < c.N && c.q[i] - 1 < cur) i++;
+      while (i < c.N && c.last[i] == 0xff && c.q[i] - 1 - cur <= c.ffrun[i]) i++;
+      DxChainEntry e;
+      const int64_t gap = (i < c.N) ? c.q[i] - 1 - cur : 0;
+      if (i < c.N && c.stat[i] == 0 && gap <= c.ffrun[i] && c.last[i] != 0xff &&
+          c.soff[6*i + 5] <= c.n && c.soff[6*i + 5] > cur)
+        { e.q = c.q[i]; e.end = c.soff[6*i + 5]; e.cand = (int32_t) i;
+          well += 255 * (int32_t) gap + c.last[i];
+          i++;
+        }
+      else
+        { int32_t delta = 0;
+          const int rc = slow(user,cur,&e.q,&e.end,&delta);
+          if (rc != 0) return rc;
+          e.cand = -1;
+          well += delta;
+        }
+      e.well = well;
+      ent.push_back(e);
+      cur = e.end;
+    }
+  *cur_out = cur;
+  return 0;
 }
 
 // Kept candidate i confirms the assumed layout: it decoded, its terminator is one, it ends exactly

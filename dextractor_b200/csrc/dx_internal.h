@@ -133,6 +133,11 @@ struct dx_ctx
   QvEntries      qv_ent;
   uint8_t       *qv_store;     // cudaMalloc'ed backing of qv_ent
   size_t         qv_store_cap;
+
+  // the byte range of a .dexqv image between dx_undexqv_range_dev and its _chain / _text_dev calls
+  // (QvRange*, dx_api.cpp); live until the next call that resets the arena
+  void          *qv_range;
+  int            qv_range_live;
 };
 
 int   dx_fail(dx_ctx *ctx, int code, const char *fmt, ...);

@@ -27,6 +27,7 @@ SYMBOLS = [
     "dx_qv_encode_dev", "dx_dexqv_dev", "dx_dexqv_host", "dx_undexqv_dev", "dx_undexqv_host",
     "dx_undexqv_size_dev", "dx_keep_index", "dx_last_index", "dx_qv_forget", "dx_qv_last_well",
     "dx_text_lines_dev", "dx_qv_load_entries_dev",
+    "dx_undexqv_range_dev", "dx_undexqv_range_chain", "dx_undexqv_range_text_dev",
 ]
 
 
@@ -138,6 +139,9 @@ def load_library():
         "dx_qv_last_well": (C.c_int, [vp, C.POINTER(i32)]),
         "dx_text_lines_dev": (C.c_int, [vp, vp, sz, i64, C.POINTER(i64), C.POINTER(i64)]),
         "dx_last_index": (C.c_int, [vp, vp, i64, C.POINTER(i64)]),
+        "dx_undexqv_range_dev": (C.c_int, [vp, vp, sz, vp, sz, i64, i64, i64, C.c_int, C.POINTER(i64)]),
+        "dx_undexqv_range_chain": (C.c_int, [vp, i64, i32, C.POINTER(i64), C.POINTER(i32)]),
+        "dx_undexqv_range_text_dev": (C.c_int, [vp, vp, sz, szp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -393,6 +397,32 @@ class Context:
         rows = (IndexRow * max(cnt.value, 1))()
         self._check(self.L.dx_last_index(self.h, rows, cnt.value, C.byref(cnt)))
         return [(r.stream_off, r.end_off, r.text_off, r.rlen, r.well) for r in rows[: cnt.value]]
+
+    def needed_bytes(self) -> int:
+        """what the last call that failed with DX_E_CAP needed (dx_needed_bytes)"""
+        return int(self.L.dx_needed_bytes(self.h))
+
+    # ---- one byte range of a .dexqv image (dx_undexqv_range_*): decode, chain, text ----------------
+    def undexqv_range_dev(self, head: bytes, d_buf, buf_n, buf_off, a, b, upper=False) -> int:
+        """speculative decode of the range [a, b) from the image bytes [buf_off, buf_off + buf_n) at
+        d_buf; head: the image's first bytes (key and coding header).  -> the first entry's offset"""
+        _wait_for_torch()
+        first = C.c_int64(0)
+        src = np.frombuffer(head, dtype=np.uint8)
+        self._check(self.L.dx_undexqv_range_dev(self.h, src.ctypes.data, len(head), d_buf, buf_n, buf_off,
+                                                a, b, int(upper), C.byref(first)))
+        return first.value
+
+    def undexqv_range_chain(self, cur_in: int, well_in: int):
+        """-> (where the next range's chain starts, the well of this range's last entry)"""
+        cur, well = C.c_int64(0), C.c_int32(0)
+        self._check(self.L.dx_undexqv_range_chain(self.h, cur_in, well_in, C.byref(cur), C.byref(well)))
+        return cur.value, well.value
+
+    def undexqv_range_text_dev(self, d_out, cap) -> int:
+        m = C.c_size_t(0)
+        self._check(self.L.dx_undexqv_range_text_dev(self.h, d_out, cap, C.byref(m)))
+        return m.value
 
     def undexqv_size_dev(self, d_in, n) -> int:
         _wait_for_torch()

@@ -237,6 +237,41 @@ int dx_undexqv_host(dx_ctx *ctx, const uint8_t *h_in, size_t n, int upper,
 /* size of the .quiva text dx_undexqv_* would produce for this file */
 int dx_undexqv_size_dev(dx_ctx *ctx, const uint8_t *d_in, size_t n, size_t *out_len);
 
+/* One byte range of a .dexqv image, for callers that cut an image into ranges and decode each on its own
+ * GPU (tools/undexqv_mg).  Entry e belongs to the range [a, b) that holds its FIRST byte, its first
+ * well-delta byte (undexqv.c:119-208 reads the delta first).  Three calls on one context, in this order,
+ * with no other call of the context in between:
+ *
+ *   dx_undexqv_range_dev       decodes every entry candidate the range needs, speculatively (no chain
+ *                              decision yet).  h_head / head_n: the image's first bytes on the host, at
+ *                              least its key and coding header (min(image size, 2 + 16384 + 100001)
+ *                              bytes are always enough).  d_buf (16-byte aligned) holds the image bytes
+ *                              [buf_off, buf_off + buf_n); it must cover [max(a', 4096) - 4096, b) with
+ *                              a' = max(a, first) and should hold the tails of the entries that start in
+ *                              [a, b).  *first (if not NULL): the byte behind the coding header, where
+ *                              the first entry starts.  upper = -U.
+ *   dx_undexqv_range_chain     the host walk from the chain position the range before it ended at:
+ *                              cur_in / well_in (first / 0 for the range that holds the first entry).
+ *                              *cur_out: where the next range's chain starts (>= b; cur_in if no entry
+ *                              starts in [cur_in, b)), *well_out: the well of the range's last entry
+ *                              (well_in if none).  An entry the candidates miss is read and decoded by
+ *                              itself, never an error of a valid image.  DX_E_CAP: an entry's tail lies
+ *                              behind the buffer; dx_needed_bytes() is the image offset the buffer has to
+ *                              reach -- read that much and start again with dx_undexqv_range_dev.
+ *   dx_undexqv_range_text_dev  the text of the range's entries into d_out; DX_E_CAP with
+ *                              dx_needed_bytes() = the text's size when cap is smaller (d_out may be
+ *                              NULL with cap 0 to ask).  Waits for the context's stream.
+ *
+ * The text of consecutive ranges, each chained from where the one before it ended, concatenated, is the
+ * text of dx_undexqv_dev on the whole image.  Images of the old layout or the other byte order, and codings
+ * whose long codes do not fit the parallel decoder's tables, are refused (DX_E_FORMAT / DX_E_CODING):
+ * decode them whole with dx_undexqv_dev. */
+int dx_undexqv_range_dev(dx_ctx *ctx, const uint8_t *h_head, size_t head_n, const uint8_t *d_buf,
+                         size_t buf_n, int64_t buf_off, int64_t a, int64_t b, int upper, int64_t *first);
+int dx_undexqv_range_chain(dx_ctx *ctx, int64_t cur_in, int32_t well_in, int64_t *cur_out,
+                           int32_t *well_out);
+int dx_undexqv_range_text_dev(dx_ctx *ctx, uint8_t *d_out, size_t cap, size_t *out_len);
+
 /* Batched Load_QVentry (DB.c:2575-2621, and Load_All... style loaders built on it): the caller knows
  * where every entry's streams start (DAZZ_READ.coff of a Dazzler .qvs, which stores bare streams;
  * or the byte behind beg/end/qv of a .dexqv entry) and how long it is.  Entry i's five lines (del,
