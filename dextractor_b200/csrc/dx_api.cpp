@@ -14,6 +14,7 @@
 #include <algorithm>
 #include <chrono>
 #include <new>
+#include <unordered_map>
 #include "dx_internal.h"
 #include "dx_chain.h"
 
@@ -126,10 +127,19 @@ void *dx_arena_get(dx_ctx *ctx, size_t bytes)
       return NULL;
     }
   size_t cap = round_up(bytes > ((size_t) 32 << 20) ? bytes : ((size_t) 32 << 20),(size_t) 1 << 20);
+  if (ctx->route[DXR_ARENA_CAP] > 0)
+    { size_t have = 0;
+      for (int i = 0; i < ctx->nblk; i++) have += ctx->blk[i].cap;
+      if (have + cap > (size_t) ctx->route[DXR_ARENA_CAP])
+        { dx_fail(ctx,DX_E_NOMEM,"scratch arena capped at %lld bytes (arena_cap)",(long long) ctx->route[DXR_ARENA_CAP]);
+          return NULL;
+        }
+    }
   uint8_t *p = NULL;
   cudaError_t e = cudaMalloc((void **) &p,cap);
   if (e != cudaSuccess)
-    { dx_cuda_fail(ctx,e,"cudaMalloc(scratch)");
+    { cudaGetLastError();                               // not left behind for the next launch check
+      dx_cuda_fail(ctx,e,"cudaMalloc(scratch)");
       return NULL;
     }
   DxBlock &b = ctx->blk[ctx->nblk++];
@@ -228,6 +238,9 @@ extern "C" int dx_open(int device, dx_ctx **out)
     }
   ctx->sm_count = prop.multiProcessorCount;
   ctx->route[DXR_DEBUG] = (getenv("DEXB200_DEBUG") != NULL);      // read once, here; never in a call
+  { const char *cap = getenv("DEXB200_ARENA_CAP");                  // tests: out-of-memory in a subprocess
+    if (cap != NULL) ctx->route[DXR_ARENA_CAP] = strtoll(cap,NULL,10);
+  }
   *out = ctx;
   return DX_OK;
 }
@@ -243,6 +256,7 @@ extern "C" void dx_close(dx_ctx *ctx)
   if (ctx->io_out)   cudaFree(ctx->io_out);
   if (ctx->qv_store) cudaFree(ctx->qv_store);
   if (ctx->last_index) delete (std::vector<dx_index_row> *) ctx->last_index;
+  delete (std::unordered_map<void *,size_t> *) ctx->dev_blocks;
   qv_range_free(ctx);
   if (ctx->hpin)     cudaFreeHost(ctx->hpin);
   while (ctx->hpin_extra)
@@ -267,12 +281,14 @@ extern "C" void       *dx_stream(dx_ctx *ctx) { return ctx ? (void *) ctx->strea
 extern "C" int dx_route(dx_ctx *ctx, const char *name, int64_t value)
 { static const char *names[DXR_COUNT] = { "no_fast", "no_spec", "exact_index", "exact_pack", "pack2", "two_pass",
                                           "chain_scan", "decoder", "lane_max_rlen", "lane_min_entries", "debug",
-                                          "serial_io", "pipe_chunk", "no_direct", "index_bulk", "hist_mode" };
+                                          "serial_io", "pipe_chunk", "no_direct", "index_bulk", "hist_mode",
+                                          "arena_cap" };
   if (ctx == NULL || name == NULL) return DX_E_ARG;
   if (strcmp(name,"default") == 0)
-    { const int64_t dbg = ctx->route[DXR_DEBUG];
+    { const int64_t dbg = ctx->route[DXR_DEBUG], cap = ctx->route[DXR_ARENA_CAP];
       memset(ctx->route,0,sizeof(ctx->route));
       ctx->route[DXR_DEBUG] = dbg;
+      ctx->route[DXR_ARENA_CAP] = cap;
       return DX_OK;
     }
   for (int k = 0; k < DXR_COUNT; k++)
@@ -310,11 +326,41 @@ extern "C" uint64_t dx_launch_count(dx_ctx *ctx, int reset)
 extern "C" void *dx_device_alloc(dx_ctx *ctx, size_t bytes)
 { void *p = NULL;
   cudaSetDevice(ctx->device);
-  cudaError_t e = cudaMalloc(&p,round_up(bytes + 64,256));
-  if (e != cudaSuccess) { dx_cuda_fail(ctx,e,"cudaMalloc"); return NULL; }
+  const size_t sz = round_up(bytes + 64,256);
+  cudaError_t e = cudaMalloc(&p,sz);
+  if (e != cudaSuccess) { cudaGetLastError(); dx_cuda_fail(ctx,e,"cudaMalloc"); return NULL; }
+  if (ctx->dev_blocks == NULL) ctx->dev_blocks = new std::unordered_map<void *,size_t>();
+  (*(std::unordered_map<void *,size_t> *) ctx->dev_blocks)[p] = sz;
   return p;
 }
-extern "C" void dx_device_free(dx_ctx *ctx, void *p) { (void) ctx; if (p) cudaFree(p); }
+extern "C" void dx_device_free(dx_ctx *ctx, void *p)
+{ if (p == NULL) return;
+  if (ctx != NULL && ctx->dev_blocks != NULL) ((std::unordered_map<void *,size_t> *) ctx->dev_blocks)->erase(p);
+  cudaFree(p);
+}
+
+extern "C" int dx_mem_info(dx_ctx *ctx, size_t *free_bytes, size_t *total_bytes, size_t *held)
+{ if (ctx == NULL) return DX_E_ARG;
+  cudaSetDevice(ctx->device);
+  size_t f = 0, t = 0;
+  DX_CUDA(ctx,cudaMemGetInfo(&f,&t));
+  size_t h = ctx->io_in_cap + ctx->io_out_cap + ctx->qv_store_cap;
+  for (int i = 0; i < ctx->nblk; i++) h += ctx->blk[i].cap;
+  if (ctx->dev_blocks != NULL)
+    for (const auto &b : *(std::unordered_map<void *,size_t> *) ctx->dev_blocks) h += b.second;
+  if (free_bytes)  *free_bytes = f;
+  if (total_bytes) *total_bytes = t;
+  if (held)        *held = h;
+  return DX_OK;
+}
+
+extern "C" int dx_set_origin(dx_ctx *ctx, int64_t line0, int64_t entry0)
+{ if (ctx == NULL || line0 < 0 || entry0 < 0) return DX_E_ARG;
+  ctx->origin_line = line0; ctx->origin_entry = entry0;
+  return DX_OK;
+}
+
+extern "C" int64_t dx_last_entries(const dx_ctx *ctx) { return ctx ? ctx->last_entries : 0; }
 
 extern "C" void *dx_pinned_alloc(dx_ctx *ctx, size_t bytes)
 { void *p = NULL;
@@ -384,7 +430,10 @@ static int ensure_io(dx_ctx *ctx, uint8_t **buf, size_t *cap, size_t need)
   if (*cap >= need) return DX_OK;
   if (*buf) cudaFree(*buf);
   *buf = NULL; *cap = 0;
-  DX_CUDA(ctx,cudaMalloc((void **) buf,need));
+  if (cudaMalloc((void **) buf,need) != cudaSuccess)
+    { *buf = NULL; cudaGetLastError();
+      return dx_fail(ctx,DX_E_NOMEM,"device allocation of %zu bytes (staging) failed",need);
+    }
   *cap = need;
   return DX_OK;
 }
@@ -499,25 +548,32 @@ static int pk_walk_one(dx_ctx *ctx, void *user, int64_t q, int64_t *end, int64_t
   return DX_OK;
 }
 
-static int dexta_impl(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n,
-                      uint8_t *d_out, size_t cap, size_t *out_len, bool exact, bool *redo);
+static int dexta_impl(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n, int32_t lwell_in, int with_header,
+                      uint8_t *d_out, size_t cap, size_t *out_len, int32_t *last_well, bool exact, bool *redo);
 
-extern "C" int dx_dexta_dev(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n,
-                            uint8_t *d_out, size_t cap, size_t *out_len)
-{ // first the vectorised kernels, which take the symbol counts from the line lattice and verify them
+extern "C" int dx_dexta_part_dev(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n, int32_t lwell_in,
+                                 int with_header, uint8_t *d_out, size_t cap, size_t *out_len, int32_t *last_well)
+{ if (ctx == NULL) return DX_E_ARG;
+  // first the vectorised kernels, which take the symbol counts from the line lattice and verify them
   // while packing; a file whose lines do not form the lattice is redone with the exact counts
   bool redo = false;
-  int rc = dexta_impl(ctx,kind,d_text,n,d_out,cap,out_len,ctx->route[DXR_EXACT_PACK] != 0,&redo);
-  if (rc == DX_OK && redo) rc = dexta_impl(ctx,kind,d_text,n,d_out,cap,out_len,true,&redo);
+  int rc = dexta_impl(ctx,kind,d_text,n,lwell_in,with_header,d_out,cap,out_len,last_well,
+                      ctx->route[DXR_EXACT_PACK] != 0,&redo);
+  if (rc == DX_OK && redo) rc = dexta_impl(ctx,kind,d_text,n,lwell_in,with_header,d_out,cap,out_len,last_well,true,&redo);
   return rc;
 }
 
-static int dexta_impl(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n,
-                      uint8_t *d_out, size_t cap, size_t *out_len, bool exact, bool *redo)
+extern "C" int dx_dexta_dev(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n,
+                            uint8_t *d_out, size_t cap, size_t *out_len)
+{ return dx_dexta_part_dev(ctx,kind,d_text,n,0,1,d_out,cap,out_len,NULL); }
+
+static int dexta_impl(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n, int32_t lwell_in, int with_header,
+                      uint8_t *d_out, size_t cap, size_t *out_len, int32_t *last_well, bool exact, bool *redo)
 { *redo = false;
   if (ctx == NULL || out_len == NULL || (kind != DX_FASTA && kind != DX_ARROW)) return DX_E_ARG;
   *out_len = 0;
   ctx->err_line = 0;
+  ctx->last_entries = 0;
   int rc;
   if ((rc = check_buf(ctx,d_text,"text")) != DX_OK) return rc;
   if (d_out == NULL) return dx_fail(ctx,DX_E_ARG,"output is NULL");
@@ -525,24 +581,30 @@ static int dexta_impl(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n,
   cudaSetDevice(ctx->device);
   dx_arena_reset(ctx);
 
-  // first header line: endian key + prefix (dexta.c:108-129)
+  // first header line: endian key + prefix (dexta.c:108-129); a later part only has to start at a header
   std::vector<uint8_t> head;
-  if ((rc = peek(ctx,d_text,n,0,100000,head)) != DX_OK) return rc;
-  const uint8_t *nl = (const uint8_t *) memchr(head.data(),'\n',head.size());
-  if (nl == NULL || nl - head.data() > 99998)
-    { ctx->err_line = 1;
-      return dx_fail(ctx,DX_E_TOOLONG,"Line 1: %s line is too long (> 99998 chars)",
-                     kind == DX_FASTA ? "Fasta" : "Arrow");
+  int32_t plen = 0;
+  size_t  hbytes = 0;
+  if ((rc = peek(ctx,d_text,n,0,with_header ? 100000 : 1,head)) != DX_OK) return rc;
+  if (with_header)
+    { const uint8_t *nl = (const uint8_t *) memchr(head.data(),'\n',head.size());
+      if (nl == NULL || nl - head.data() > 99998)
+        { ctx->err_line = 1;
+          return dx_fail(ctx,DX_E_TOOLONG,"Line 1: %s line is too long (> 99998 chars)",
+                         kind == DX_FASTA ? "Fasta" : "Arrow");
+        }
+      if (head[0] != '>')
+        { ctx->err_line = 1;
+          return dx_fail(ctx,DX_E_FORMAT,"Line 1: First header in %s file is missing",
+                         kind == DX_FASTA ? "fasta" : "arrow");
+        }
+      const uint8_t *slash = (const uint8_t *) memchr(head.data(),'/',(size_t) (nl - head.data()));
+      if (slash == NULL) return dx_fail(ctx,DX_E_FORMAT,"Header line incorrectly formatted ?");
+      plen = (int32_t) (slash - head.data());
+      hbytes = 2 + 4 + (size_t) plen;
     }
-  if (head[0] != '>')
-    { ctx->err_line = 1;
-      return dx_fail(ctx,DX_E_FORMAT,"Line 1: First header in %s file is missing",
-                     kind == DX_FASTA ? "fasta" : "arrow");
-    }
-  const uint8_t *slash = (const uint8_t *) memchr(head.data(),'/',(size_t) (nl - head.data()));
-  if (slash == NULL) return dx_fail(ctx,DX_E_FORMAT,"Header line incorrectly formatted ?");
-  const int32_t plen = (int32_t) (slash - head.data());
-  const size_t  hbytes = 2 + 4 + (size_t) plen;
+  else if (head[0] != '>')
+    return dx_fail(ctx,DX_E_ARG,"dx_dexta_part_dev: a part without the file header must start at an entry header ('>')");
 
   int64_t *d_hdr = NULL, nent = 0;
   if ((rc = dxk_index_positions(ctx,DX_PRED_FASTA_HDR,d_text,n,0,&d_hdr,&nent)) != DX_OK) return rc;
@@ -585,8 +647,8 @@ static int dexta_impl(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n,
     flag.assign(N,0);
   for (size_t e = 0; e < N && anyflag; e++)
     { if (flag[e] & 4)
-        return dx_fail(ctx,DX_E_TOOLONG,"%s line is too long (> 99998 chars) or unterminated (entry %zu)",
-                       kind == DX_FASTA ? "Fasta" : "Arrow",e+1);
+        return dx_fail(ctx,DX_E_TOOLONG,"%s line is too long (> 99998 chars) or unterminated (entry %lld)",
+                       kind == DX_FASTA ? "Fasta" : "Arrow",(long long) (ctx->origin_entry + (int64_t) e + 1));
       if (!(flag[e] & 1)) continue;
       int64_t h0 = 0;
       DX_CUDA(ctx,cudaMemcpyAsync(&h0,ent.hdr+e,8,cudaMemcpyDeviceToHost,ctx->stream));
@@ -594,7 +656,8 @@ static int dexta_impl(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n,
       std::vector<uint8_t> line;
       if ((rc = peek(ctx,d_text,n,(size_t) h0,100000,line)) != DX_OK) return rc;
       const uint8_t *e1 = (const uint8_t *) memchr(line.data(),'\n',line.size());
-      if (e1 == NULL) return dx_fail(ctx,DX_E_TOOLONG,"header line too long (entry %zu)",e+1);
+      if (e1 == NULL)
+        return dx_fail(ctx,DX_E_TOOLONG,"header line too long (entry %lld)",(long long) (ctx->origin_entry + (int64_t) e + 1));
       std::vector<char> txt(line.begin(),line.begin() + (e1 - line.data()) + 1);
       txt.push_back('\0');
       char *sl = strchr(txt.data()+1,'/');
@@ -623,27 +686,29 @@ static int dexta_impl(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n,
     }
 
   int64_t body = 0;
-  if ((rc = dxk_fa_offsets(ctx,kind,ent,0,&body)) != DX_OK) return rc;
+  if ((rc = dxk_fa_offsets(ctx,kind,ent,lwell_in,&body)) != DX_OK) return rc;
   if (hbytes + (size_t) body > cap)
     return dx_fail_cap(ctx,(size_t) (hbytes + (size_t) body),cap);
 
-  std::vector<uint8_t> fh(hbytes);
-  const uint16_t key = 0x55aa;
-  memcpy(fh.data(),&key,2);
-  memcpy(fh.data()+2,&plen,4);
-  memcpy(fh.data()+6,head.data(),(size_t) plen);
-  if ((rc = upload(ctx,d_out,fh.data(),hbytes)) != DX_OK) return rc;
+  if (with_header)
+    { std::vector<uint8_t> fh(hbytes);
+      const uint16_t key = 0x55aa;
+      memcpy(fh.data(),&key,2);
+      memcpy(fh.data()+2,&plen,4);
+      memcpy(fh.data()+6,head.data(),(size_t) plen);
+      if ((rc = upload(ctx,d_out,fh.data(),hbytes)) != DX_OK) return rc;
+    }
   if (exact)
-    { if ((rc = dxk_fa_pack(ctx,kind,d_text,n,ent,0,d_out + hbytes)) != DX_OK) return rc;
+    { if ((rc = dxk_fa_pack(ctx,kind,d_text,n,ent,lwell_in,d_out + hbytes)) != DX_OK) return rc;
       DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
     }
   else
     { // d_flags: [1] pack error, [2..3] ticket, [4] entries left to k_fa_pack2, [6..7] its ticket
       int32_t res[4] = { 0, 0, 0, 0 };
       if (ctx->route[DXR_PACK2])
-        rc = dxk_fa_pack2(ctx,kind,d_text,ent,0,d_out + hbytes,d_flags + 1,(unsigned long long *) (d_flags + 2),0);
+        rc = dxk_fa_pack2(ctx,kind,d_text,ent,lwell_in,d_out + hbytes,d_flags + 1,(unsigned long long *) (d_flags + 2),0);
       else
-        rc = dxk_fa_pack3(ctx,kind,d_text,n,ent,0,d_out + hbytes,d_flags + 1,d_flags + 4,
+        rc = dxk_fa_pack3(ctx,kind,d_text,n,ent,lwell_in,d_out + hbytes,d_flags + 1,d_flags + 4,
                           (unsigned long long *) (d_flags + 2));
       if (rc != DX_OK) return rc;
       DX_CUDA(ctx,cudaMemcpyAsync(res,d_flags + 1,16,cudaMemcpyDeviceToHost,ctx->stream));
@@ -651,7 +716,7 @@ static int dexta_impl(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n,
       if (res[0] == 2) return dx_fail(ctx,DX_E_TOOLONG,"%s line is too long (> 99998 chars)",kind == DX_FASTA ? "Fasta" : "Arrow");
       if (res[0]) { *redo = true; return DX_OK; }
       if (res[3])                                   // entries off the lattice (or narrower than 16)
-        { if ((rc = dxk_fa_pack2(ctx,kind,d_text,ent,0,d_out + hbytes,d_flags + 1,
+        { if ((rc = dxk_fa_pack2(ctx,kind,d_text,ent,lwell_in,d_out + hbytes,d_flags + 1,
                                  (unsigned long long *) (d_flags + 6),1)) != DX_OK) return rc;
           DX_CUDA(ctx,cudaMemcpyAsync(res,d_flags + 1,4,cudaMemcpyDeviceToHost,ctx->stream));
           DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
@@ -659,6 +724,14 @@ static int dexta_impl(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n,
           if (res[0]) { *redo = true; return DX_OK; }
         }
     }
+  if (last_well != NULL)
+    { *last_well = lwell_in;
+      if (N > 0)
+        { DX_CUDA(ctx,cudaMemcpyAsync(last_well,ent.well + (N - 1),4,cudaMemcpyDeviceToHost,ctx->stream));
+          DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
+        }
+    }
+  ctx->last_entries = nent;
   *out_len = hbytes + (size_t) body;
   return DX_OK;
 }
@@ -938,6 +1011,153 @@ extern "C" int dx_undexta_size_dev(dx_ctx *ctx, int kind, const uint8_t *d_in, s
   return DX_OK;
 }
 
+// ---- one window of a .dexta / .dexar image ----------------------------------------------------------
+// The chain is walked from a carried position and well (dx_chain_walk_general); an entry the candidates
+// do not give is read by itself, and the walk ends in front of the first entry that does not lie wholly
+// in the buffer.
+
+struct PkWinSlow { dx_ctx *ctx; const uint8_t *d_buf; size_t n; int fieldbytes; int64_t need; };
+
+// the entry at buffer offset cur read by itself; DX_E_CAP (u.need: the buffer offset it needs) when its
+// delta bytes, fields or payload reach past the buffer
+static int pk_win_slow(void *user, int64_t cur, int64_t *q, int64_t *end, int32_t *delta)
+{ PkWinSlow &u = *(PkWinSlow *) user;
+  std::vector<uint8_t> win;
+  int64_t p = cur;
+  int32_t add = 0;
+  int rc;
+  for (;;)
+    { if ((rc = peek(u.ctx,u.d_buf,u.n,(size_t) p,4096,win)) != DX_OK) return rc;
+      size_t k = 0;
+      while (k < win.size() && win[k] == 0xff) k++;
+      add += 255 * (int32_t) k; p += (int64_t) k;
+      if (k < win.size()) { add += win[k]; p += 1; break; }
+      if (p >= (int64_t) u.n)                               // a delta is at most 2^31 wells: 8 421 505 bytes
+        { u.need = cur + 8421505 + u.fieldbytes; return DX_E_CAP; }
+    }
+  if ((rc = peek(u.ctx,u.d_buf,u.n,(size_t) p,(size_t) u.fieldbytes,win)) != DX_OK) return rc;
+  if ((int) win.size() < u.fieldbytes) { u.need = p + u.fieldbytes; return DX_E_CAP; }
+  const int64_t rlen = (int64_t) le32(win.data()+4) - le32(win.data());
+  if (rlen < 0) return dx_fail(u.ctx,DX_E_FORMAT,"negative read length in entry header");
+  *q = p; *end = p + u.fieldbytes + ((rlen + 3) >> 2); *delta = add;
+  if (*end > (int64_t) u.n) { u.need = *end; return DX_E_CAP; }
+  return DX_OK;
+}
+
+extern "C" int dx_undexta_window_dev(dx_ctx *ctx, int kind, const uint8_t *h_head, size_t head_n,
+                                     const uint8_t *d_buf, size_t buf_n, int64_t buf_off, int64_t cur_in,
+                                     int32_t well_in, int is_last, int width, int upper, uint8_t *d_out, size_t cap,
+                                     size_t *out_len, int64_t *cur_out, int32_t *well_out)
+{ if (ctx == NULL || out_len == NULL || cur_out == NULL || well_out == NULL || (kind != DX_FASTA && kind != DX_ARROW))
+    return DX_E_ARG;
+  *out_len = 0; *cur_out = cur_in; *well_out = well_in;
+  ctx->last_entries = 0;
+  int rc;
+  if (h_head == NULL) return dx_fail(ctx,DX_E_ARG,"dx_undexta_window_dev: h_head is NULL");
+  if (width <= 0) return dx_fail(ctx,DX_E_ARG,"line width must be positive");
+  if (head_n < 6) return dx_fail(ctx,DX_E_TRUNC,"System error, read failed!");
+  uint16_t key; memcpy(&key,h_head,2);
+  int32_t  plen; memcpy(&plen,h_head+2,4);
+  if (!(key == 0x55aa || key == 0xaa55 || (kind == DX_FASTA && (key == 0x33cc || key == 0xcc33))))
+    return dx_fail(ctx,DX_E_KEY,"Not a %s file, endian key invalid",kind == DX_FASTA ? ".dexta" : ".dexar");
+  if (key != 0x55aa)
+    return dx_fail(ctx,DX_E_FORMAT,"%s image: windows take images of the 0x55aa layout in the native byte order; "
+                   "decode it whole with dx_undexta_dev",key == 0xaa55 ? "a foreign-endian" : "an old-layout (0x33cc)");
+  if (plen < 0 || (size_t) plen + 6 > head_n) return dx_fail(ctx,DX_E_TRUNC,"System error, read failed!");
+  if ((rc = check_buf(ctx,d_buf,"window buffer")) != DX_OK) return rc;
+  const int64_t first = 6 + (int64_t) plen, buf_end = buf_off + (int64_t) buf_n;
+  if (buf_off < 0 || cur_in < first || cur_in < buf_off || cur_in > buf_end)
+    return dx_fail(ctx,DX_E_ARG,"dx_undexta_window_dev: the chain position %lld is not in the buffer [%lld, %lld) "
+                   "behind the header (%lld bytes)",(long long) cur_in,(long long) buf_off,(long long) buf_end,(long long) first);
+  cudaSetDevice(ctx->device);
+  dx_arena_reset(ctx);
+  const int fieldbytes = (kind == DX_FASTA) ? 12 : 16;
+  const int64_t s = cur_in - buf_off;
+
+  int64_t *d_q = NULL, nc = 0;
+  if (s < (int64_t) buf_n &&
+      (rc = dxk_index_positions(ctx,kind == DX_FASTA ? DX_PRED_QVCAND : DX_PRED_ARCAND,d_buf,buf_n,(size_t) s + 1,
+                                &d_q,&nc)) != DX_OK) return rc;
+  const size_t N = (size_t) nc;
+  int64_t *d_end   = (int64_t *) dx_arena_get(ctx,N*8);
+  int32_t *d_ffrun = (int32_t *) dx_arena_get(ctx,N*4);
+  uint8_t *d_last  = (uint8_t *) dx_arena_get(ctx,N);
+  int64_t *h_q     = (int64_t *) dx_hpin_get(ctx,N*8);
+  int64_t *h_end   = (int64_t *) dx_hpin_get(ctx,N*8);
+  int32_t *h_ffrun = (int32_t *) dx_hpin_get(ctx,N*4);
+  uint8_t *h_last  = (uint8_t *) dx_hpin_get(ctx,N);
+  if (!d_end || !d_ffrun || !d_last || !h_q || !h_end || !h_ffrun || !h_last) return DX_E_NOMEM;
+  if (N > 0)
+    { if ((rc = dxk_pk_cand_prep(ctx,d_buf,buf_n,(size_t) s,fieldbytes,d_q,nc,d_end,d_ffrun,d_last)) != DX_OK) return rc;
+      DX_CUDA(ctx,cudaMemcpyAsync(h_q,d_q,N*8,cudaMemcpyDeviceToHost,ctx->stream));
+      DX_CUDA(ctx,cudaMemcpyAsync(h_end,d_end,N*8,cudaMemcpyDeviceToHost,ctx->stream));
+      DX_CUDA(ctx,cudaMemcpyAsync(h_ffrun,d_ffrun,N*4,cudaMemcpyDeviceToHost,ctx->stream));
+      DX_CUDA(ctx,cudaMemcpyAsync(h_last,d_last,N,cudaMemcpyDeviceToHost,ctx->stream));
+      DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
+    }
+  std::vector<int32_t> stat(N);                         // the walk's view of a candidate: did it end in the buffer
+  std::vector<int64_t> soff(6*N);
+  for (size_t i = 0; i < N; i++) { stat[i] = (h_end[i] < 0); soff[6*i + 5] = h_end[i]; }
+  const DxChainIn ci = { h_q, h_ffrun, h_last, stat.data(), soff.data(), NULL, (int64_t) N, s, (int64_t) buf_n,
+                         s, (int64_t) buf_n };
+  PkWinSlow u = { ctx, d_buf, buf_n, fieldbytes, 0 };
+  std::vector<DxChainEntry> ent;
+  int64_t stop = s;
+  rc = dx_chain_walk_general(ci,well_in,pk_win_slow,&u,ent,&stop);
+  if (rc == DX_E_CAP)                                   // the walk stopped in front of an entry the buffer cuts
+    { if (is_last) return dx_fail(ctx,DX_E_TRUNC,"System error, read failed!");
+      if (ent.empty())
+        { dx_fail(ctx,DX_E_CAP,"the entry at image offset %lld runs past the end of the buffer (%lld): it needs the image "
+                  "up to %lld",(long long) cur_in,(long long) buf_end,(long long) (buf_off + u.need));
+          ctx->need_bytes = (size_t) (buf_off + u.need);
+          return DX_E_CAP;
+        }
+      stop = ent.back().end;
+    }
+  else if (rc != DX_OK)
+    return rc;
+
+  const size_t M = ent.size();
+  *cur_out = buf_off + stop;
+  *well_out = (M > 0) ? ent.back().well : well_in;
+  ctx->last_entries = (int64_t) M;
+  if (M == 0) return DX_OK;
+  int64_t *h_qm  = (int64_t *) dx_hpin_get(ctx,M*8);
+  int32_t *h_cw  = (int32_t *) dx_hpin_get(ctx,M*8);     // [0, M) candidate = m, [M, 2M) well
+  int64_t *h_total = (int64_t *) dx_hpin_get(ctx,8);
+  int64_t *d_qm  = (int64_t *) dx_arena_get(ctx,M*8);
+  int32_t *d_cw  = (int32_t *) dx_arena_get(ctx,M*8);
+  uint32_t *d_len = (uint32_t *) dx_arena_get(ctx,M*4);
+  int64_t *d_opre = (int64_t *) dx_arena_get(ctx,(M+1)*8);
+  PkDecEntry *d_ent = (PkDecEntry *) dx_arena_get(ctx,(M+1)*sizeof(PkDecEntry));
+  char *d_prefix = (char *) dx_arena_get(ctx,(size_t) plen + 1);
+  unsigned long long *d_ticket = (unsigned long long *) dx_arena_get(ctx,8);
+  if (!h_qm || !h_cw || !h_total || !d_qm || !d_cw || !d_len || !d_opre || !d_ent || !d_prefix || !d_ticket)
+    return DX_E_NOMEM;
+  for (size_t m = 0; m < M; m++) { h_qm[m] = ent[m].q; h_cw[m] = (int32_t) m; h_cw[M + m] = ent[m].well; }
+  DX_CUDA(ctx,cudaMemcpyAsync(d_qm,h_qm,M*8,cudaMemcpyHostToDevice,ctx->stream));
+  DX_CUDA(ctx,cudaMemcpyAsync(d_cw,h_cw,M*8,cudaMemcpyHostToDevice,ctx->stream));
+  if (plen > 0) DX_CUDA(ctx,cudaMemcpyAsync(d_prefix,h_head + 6,(size_t) plen,cudaMemcpyHostToDevice,ctx->stream));
+  DX_CUDA(ctx,cudaMemsetAsync(d_ticket,0,8,ctx->stream));
+  if ((rc = dxk_pk_layout(ctx,kind,d_buf,d_qm,d_cw,d_cw + M,(int64_t) M,fieldbytes,plen,width,d_len,d_opre,d_ent)) != DX_OK)
+    return rc;
+  DX_CUDA(ctx,cudaMemcpyAsync(h_total,d_opre + M,8,cudaMemcpyDeviceToHost,ctx->stream));
+  DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
+  const size_t total = (size_t) *h_total;
+  if (total > cap) return dx_fail_cap(ctx,total,cap);
+  if (d_out == NULL) return dx_fail(ctx,DX_E_ARG,"output is NULL");
+  if (width < 16)
+    rc = dxk_unpack(ctx,kind,upper,width,d_buf,d_ent,(int64_t) M,d_prefix,plen,d_out);
+  else if (ctx->route[DXR_PACK2])
+    rc = dxk_unpack2(ctx,kind,upper,width,d_buf,buf_n,d_ent,(int64_t) M,d_prefix,plen,d_out,d_ticket);
+  else
+    rc = dxk_unpack3(ctx,kind,upper,width,d_buf,buf_n,d_ent,(int64_t) M,d_prefix,plen,d_out,d_ticket);
+  if (rc != DX_OK) return rc;
+  DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
+  *out_len = total;
+  return DX_OK;
+}
+
 extern "C" int dx_compress_reads_dev(dx_ctx *ctx, int kind, const uint8_t *d_src,
                                      const int64_t *d_src_off, const int32_t *d_len, int64_t nreads,
                                      uint8_t *d_dst, const int64_t *d_dst_off)
@@ -980,19 +1200,22 @@ static int qv_frame(dx_ctx *ctx, const uint8_t *d_text, size_t n, uint64_t *totc
         { DX_CUDA(ctx,cudaMemcpyAsync(&last,d_nl+nlines-1,8,cudaMemcpyDeviceToHost,ctx->stream));
           DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
         }
-      ctx->err_line = nlines + 1;
+      ctx->err_line = ctx->origin_line + nlines + 1;
       if (last != (int64_t) n - 1)
         return dx_fail(ctx,DX_E_FORMAT,"Line %lld: Last line does not end with a newline !",
-                       (long long) nlines + 1);
+                       (long long) ctx->err_line);
       return dx_fail(ctx,DX_E_FORMAT,"Line %lld: incomplete last entry of .quiv file",
-                     (long long) nlines + 1);
+                     (long long) ctx->err_line);
     }
   const int64_t nent = nlines / 6;
   const size_t need = round_up((size_t) nent*8,256)*2 + round_up((size_t) nent*4,256)*7 + 256;
   if (ctx->qv_store_cap < need)
     { if (ctx->qv_store) cudaFree(ctx->qv_store);
       ctx->qv_store = NULL; ctx->qv_store_cap = 0;
-      DX_CUDA(ctx,cudaMalloc((void **) &ctx->qv_store,need));
+      if (cudaMalloc((void **) &ctx->qv_store,need) != cudaSuccess)
+        { ctx->qv_store = NULL; cudaGetLastError();
+          return dx_fail(ctx,DX_E_NOMEM,"device allocation of %zu bytes (entry table) failed",need);
+        }
       ctx->qv_store_cap = need;
     }
   QvEntries ent;
@@ -1012,17 +1235,17 @@ static int qv_frame(dx_ctx *ctx, const uint8_t *d_text, size_t n, uint64_t *totc
   int64_t noncanon = 0, last = -1;
   if ((rc = dxk_qv_entries(ctx,d_text,n,d_nl,nlines,ent,err,totchar,&noncanon,&last)) != DX_OK) return rc;
   if (last != (int64_t) n - 1)
-    { ctx->err_line = nlines + 1;
+    { ctx->err_line = ctx->origin_line + nlines + 1;
       return dx_fail(ctx,DX_E_FORMAT,"Line %lld: Last line does not end with a newline !",
-                     (long long) nlines + 1);
+                     (long long) ctx->err_line);
     }
   if (err[0] != 0)
-    { ctx->err_line = err[1];
+    { const long long line = (long long) (ctx->err_line = ctx->origin_line + err[1]);
       if (err[0] == 5)
-        return dx_fail(ctx,DX_E_LINELEN,"Line %d: Lines for an entry are not the same length",err[1]);
+        return dx_fail(ctx,DX_E_LINELEN,"Line %lld: Lines for an entry are not the same length",line);
       if (err[0] == 6)
-        return dx_fail(ctx,DX_E_TOOLONG,"Line %d: entry longer than 2^24 symbols",err[1]);
-      return dx_fail(ctx,DX_E_FORMAT,"Line %d: Header in quiva file is missing",err[1]);
+        return dx_fail(ctx,DX_E_TOOLONG,"Line %lld: entry longer than 2^24 symbols",line);
+      return dx_fail(ctx,DX_E_FORMAT,"Line %lld: Header in quiva file is missing",line);
     }
 
   // headers the device parser did not recognise as canonical: the host's sscanf decides
@@ -1042,9 +1265,9 @@ static int qv_frame(dx_ctx *ctx, const uint8_t *d_text, size_t n, uint64_t *totc
       char *sl = strchr(txt.data()+1,'/');
       int well, beg, en, qv;
       if (sl == NULL || sscanf(sl+1,"%d/%d_%d RQ=0.%d\n",&well,&beg,&en,&qv) != 4)   // QV.c:958-968
-        { ctx->err_line = 6*e + 1;
+        { ctx->err_line = ctx->origin_line + 6*e + 1;
           return dx_fail(ctx,DX_E_FORMAT,"Line %lld: Header line incorrectly formatted ?",
-                         (long long) (6*e + 1));
+                         (long long) ctx->err_line);
         }
       if ((rc = upload(ctx,ent.well+e,&well,1)) != DX_OK) return rc;
       if ((rc = upload(ctx,ent.beg+e,&beg,1)) != DX_OK) return rc;

@@ -87,6 +87,7 @@ enum { DXR_NO_FAST = 0, DXR_NO_SPEC, DXR_EXACT_INDEX, DXR_EXACT_PACK, DXR_PACK2,
        DXR_NO_DIRECT,          // discovered entries: always decode into the scratch image, then assemble
        DXR_INDEX_BULK,         // newline index with cp.async.bulk tiles (experiment); > 1: CTAs per SM
        DXR_HIST_MODE,          // k_qv_hist_run: 0 shared atomics, 1 match.any groups, 2 / 3 one of each, 4 no queue
+       DXR_ARENA_CAP,          // > 0: the scratch arena grows to at most this many bytes (DX_E_NOMEM beyond)
        DXR_COUNT };
 
 struct dx_ctx
@@ -138,6 +139,12 @@ struct dx_ctx
   // (QvRange*, dx_api.cpp); live until the next call that resets the arena
   void          *qv_range;
   int            qv_range_live;
+
+  // dx_set_origin: added to the line and entry numbers of error texts and dx_error_line, so that a caller
+  // that feeds one file window by window reports what the whole-file call reports
+  int64_t        origin_line, origin_entry;
+  int64_t        last_entries;  // entries of the last dx_dexta_part_dev / dx_undexta_window_dev
+  void          *dev_blocks;    // std::unordered_map<void*, size_t>*: live dx_device_alloc blocks (dx_mem_info)
 };
 
 int   dx_fail(dx_ctx *ctx, int code, const char *fmt, ...);

@@ -28,6 +28,7 @@ SYMBOLS = [
     "dx_undexqv_size_dev", "dx_keep_index", "dx_last_index", "dx_qv_forget", "dx_qv_last_well",
     "dx_text_lines_dev", "dx_qv_load_entries_dev",
     "dx_undexqv_range_dev", "dx_undexqv_range_chain", "dx_undexqv_range_text_dev",
+    "dx_mem_info", "dx_set_origin", "dx_dexta_part_dev", "dx_last_entries", "dx_undexta_window_dev",
 ]
 
 
@@ -142,6 +143,12 @@ def load_library():
         "dx_undexqv_range_dev": (C.c_int, [vp, vp, sz, vp, sz, i64, i64, i64, C.c_int, C.POINTER(i64)]),
         "dx_undexqv_range_chain": (C.c_int, [vp, i64, i32, C.POINTER(i64), C.POINTER(i32)]),
         "dx_undexqv_range_text_dev": (C.c_int, [vp, vp, sz, szp]),
+        "dx_mem_info": (C.c_int, [vp, szp, szp, szp]),
+        "dx_set_origin": (C.c_int, [vp, i64, i64]),
+        "dx_dexta_part_dev": (C.c_int, [vp, C.c_int, vp, sz, i32, C.c_int, vp, sz, szp, C.POINTER(i32)]),
+        "dx_last_entries": (i64, [vp]),
+        "dx_undexta_window_dev": (C.c_int, [vp, C.c_int, vp, sz, vp, sz, i64, i64, i32, C.c_int, C.c_int, C.c_int,
+                                            vp, sz, szp, C.POINTER(i64), C.POINTER(i32)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -423,6 +430,38 @@ class Context:
         m = C.c_size_t(0)
         self._check(self.L.dx_undexqv_range_text_dev(self.h, d_out, cap, C.byref(m)))
         return m.value
+
+    # ---- files window by window: 2-bit parts and windows, origin, memory --------------------------------
+    def mem_info(self):
+        """-> (free, total, held) device bytes (dx_mem_info)"""
+        f, t, h = C.c_size_t(0), C.c_size_t(0), C.c_size_t(0)
+        self._check(self.L.dx_mem_info(self.h, C.byref(f), C.byref(t), C.byref(h)))
+        return f.value, t.value, h.value
+
+    def set_origin(self, line0: int = 0, entry0: int = 0):
+        self._check(self.L.dx_set_origin(self.h, line0, entry0))
+
+    def last_entries(self) -> int:
+        return int(self.L.dx_last_entries(self.h))
+
+    def dexta_part_dev(self, kind, d_text, n, lwell_in, with_header, d_out, cap):
+        """-> (output bytes, well of the part's last entry)"""
+        _wait_for_torch()
+        m, lastw = C.c_size_t(0), C.c_int32(0)
+        self._check(self.L.dx_dexta_part_dev(self.h, kind, d_text, n, lwell_in, int(with_header), d_out, cap,
+                                             C.byref(m), C.byref(lastw)))
+        return m.value, lastw.value
+
+    def undexta_window_dev(self, kind, head: bytes, d_buf, buf_n, buf_off, cur_in, well_in, is_last, width,
+                           upper, d_out, cap):
+        """-> (text bytes, next chain position, well in front of it)"""
+        _wait_for_torch()
+        m, cur, well = C.c_size_t(0), C.c_int64(0), C.c_int32(0)
+        src = np.frombuffer(head, dtype=np.uint8)
+        self._check(self.L.dx_undexta_window_dev(self.h, kind, src.ctypes.data, len(head), d_buf, buf_n, buf_off,
+                                                 cur_in, well_in, int(is_last), width, int(upper), d_out, cap,
+                                                 C.byref(m), C.byref(cur), C.byref(well)))
+        return m.value, cur.value, well.value
 
     def undexqv_size_dev(self, d_in, n) -> int:
         _wait_for_torch()

@@ -65,6 +65,16 @@ int   dx_h2d(dx_ctx *ctx, void *d_dst, const void *h_src, size_t bytes);   /* as
 int   dx_d2h(dx_ctx *ctx, void *h_dst, const void *d_src, size_t bytes);   /* async on stream */
 int   dx_d2d(dx_ctx *ctx, void *d_dst, const void *d_src, size_t bytes);   /* async; no overlap */
 
+/* Device memory for sizing windows.  free / total: cudaMemGetInfo of the context's device.  held: the
+ * device bytes this context holds now -- its scratch arena, its staging and framing buffers and the live
+ * dx_device_alloc blocks.  Any pointer may be NULL. */
+int dx_mem_info(dx_ctx *ctx, size_t *free, size_t *total, size_t *held);
+
+/* Where the text of the following calls starts in its file: line0 lines and entry0 entries lie in front
+ * of it.  Added to the line and entry numbers of error texts and of dx_error_line, so that a caller that
+ * feeds a file window by window reports an error exactly as the whole-file call does.  0, 0 at dx_open. */
+int dx_set_origin(dx_ctx *ctx, int64_t line0, int64_t entry0);
+
 /* launches issued by this context since the last reset (for the bench's gpu_launches claim) */
 uint64_t dx_launch_count(dx_ctx *ctx, int reset);
 
@@ -77,7 +87,9 @@ uint64_t dx_launch_count(dx_ctx *ctx, int reset);
  * discovered entries decodes into a scratch image and moves the lines, instead of straight into
  * place), "index_bulk" (the newline index fetches its tiles with cp.async.bulk + mbarrier instead of
  * vector loads: an experiment, value = CTAs per SM), "hist_mode" (how k_qv_hist_run counts a batch: 0 shared atomics, 1 match.any groups, 2 / 3
- * one of each, 4 without the item queue), "debug"; "default" resets all.
+ * one of each, 4 without the item queue), "arena_cap" (the scratch arena grows to at most this many bytes;
+ * beyond, DX_E_NOMEM: how a caller's out-of-memory handling is tested), "debug"; "default" resets all but
+ * "debug" and "arena_cap", which dx_open takes from DEXB200_DEBUG and DEXB200_ARENA_CAP.
  * No reference counterpart; nothing in the library reads the environment inside a call. */
 int dx_route(dx_ctx *ctx, const char *name, int64_t value);
 
@@ -102,6 +114,19 @@ int dx_dexta_dev (dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n,
 int dx_dexta_host(dx_ctx *ctx, int kind, const uint8_t *h_text, size_t n,
                   uint8_t *h_out, size_t cap, size_t *out_len);
 
+/* One part of a file: the entries of d_text[0..n), which starts at an entry header ('>').  lwell_in is
+ * the well of the entry in front of the part (0 for the first part), *last_well (if not NULL) returns the
+ * well of the part's last entry, for the next part's lwell_in.  with_header = 1 (the first part only):
+ * the part also gets the 0x55aa key, plen and prefix, and its first line is checked as dx_dexta_dev
+ * checks it.  The parts' outputs concatenated, each part cut in front of a line that starts with '>',
+ * are the bytes of dx_dexta_dev on the whole file, which is this call with 0 and 1.  DX_E_CAP and
+ * dx_needed_bytes as for dx_dexta_dev. */
+int dx_dexta_part_dev(dx_ctx *ctx, int kind, const uint8_t *d_text, size_t n, int32_t lwell_in,
+                      int with_header, uint8_t *d_out, size_t cap, size_t *out_len, int32_t *last_well);
+/* entries encoded by the last dx_dexta_part_dev / dx_dexta_dev, or decoded by the last
+ * dx_undexta_window_dev (the entry0 of the next window's dx_set_origin) */
+int64_t dx_last_entries(const dx_ctx *ctx);
+
 /* Whole-file decode.  Replaces undexta.c:130-271 / undexar.c:130-229: endian key (0x55aa,
  * 0xaa55 and, fasta only, the old 0x33cc/0xcc33 16-bit layout), per-entry header text,
  * Uncompress_Read (DB.c:342-363) + Lower_/Upper_Read/Letter_Arrow, `width` symbols per line
@@ -115,6 +140,23 @@ int dx_undexta_size_host(dx_ctx *ctx, int kind, const uint8_t *h_in, size_t n, i
                          size_t *out_len);
 int dx_undexta_size_dev (dx_ctx *ctx, int kind, const uint8_t *d_in, size_t n, int width,
                          size_t *out_len);
+
+/* One window of a .dexta / .dexar image, for callers that hold only part of the file.  h_head: the image's
+ * first min(image size, 6 + plen) bytes on the host (key, plen, prefix).  d_buf (16-byte aligned) holds the
+ * image bytes [buf_off, buf_off + buf_n).  The chain starts at image offset cur_in (6 + plen for the first
+ * window) with the well well_in (0 for the first); the call decodes every entry from there on that lies
+ * wholly in the buffer and stops in front of the first that does not: *cur_out / *well_out are where that
+ * entry starts and the well in front of it (the next window's cur_in / well_in).  is_last = 1: the buffer
+ * reaches the end of the image, and an entry cut short is DX_E_TRUNC, as for the whole file.
+ * DX_E_CAP with *cur_out == cur_in: no entry lies wholly in the buffer (is_last = 0); dx_needed_bytes() is
+ * the image offset the buffer has to reach.  DX_E_CAP with *cur_out > cur_in: the text needs
+ * dx_needed_bytes() bytes of d_out (d_out may be NULL with cap 0 to ask).  The texts of consecutive windows
+ * concatenated are the text of dx_undexta_dev.  Images of the old 0x33cc layout or the other byte order are
+ * refused (DX_E_FORMAT): decode them whole. */
+int dx_undexta_window_dev(dx_ctx *ctx, int kind, const uint8_t *h_head, size_t head_n, const uint8_t *d_buf,
+                          size_t buf_n, int64_t buf_off, int64_t cur_in, int32_t well_in, int is_last,
+                          int width, int upper, uint8_t *d_out, size_t cap, size_t *out_len,
+                          int64_t *cur_out, int32_t *well_out);
 
 /* Batched in-memory form of the same codec for callers that already hold reads in memory
  * (the Dazzler DB loaders, DB.c:1279-1286, 1414-1432, 1533-1540, 1592-1600 and the dex2DB

@@ -20,10 +20,12 @@ static int run(dx_ctx *ctx, const dx_opts *o, const uint8_t *d_in, size_t n,
   return rc;
 }
 
+static int stream(dx_win *w) { return dx_stream_pack(w,DX_ARROW); }
+
 int main(int argc, char *argv[])
 { static const dx_tool tool =
     { "dexar", "[-vk] ( -i | <path:arrow> ... )", "vki", 0, ".arrow", ".dexar",
       { "      -i: source is on standard input.",
-        "      -k: do *not* remove the .arrow file on completion.", NULL, NULL, NULL }, run };
+        "      -k: do *not* remove the .arrow file on completion.", NULL, NULL, NULL }, run, stream, 4.0 };
   return dx_cli_main(&tool,argc,argv);
 }

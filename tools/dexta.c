@@ -20,11 +20,13 @@ static int run(dx_ctx *ctx, const dx_opts *o, const uint8_t *d_in, size_t n,
   return rc;
 }
 
+static int stream(dx_win *w) { return dx_stream_pack(w,DX_FASTA); }
+
 int main(int argc, char *argv[])
 { static const dx_tool tool =
     { "dexta", "[-vk] ( -i | <path:fasta> ... )", "vki", 0, ".fasta", ".dexta",
       { "      -i: source is on standard input.",
         "      -k: do *not* remove the .fasta file on completion.",
-        "      -w: line width for sequence lines.", NULL, NULL }, run };
+        "      -w: line width for sequence lines.", NULL, NULL }, run, stream, 4.0 };
   return dx_cli_main(&tool,argc,argv);
 }

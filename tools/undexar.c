@@ -13,11 +13,13 @@ static int run(dx_ctx *ctx, const dx_opts *o, const uint8_t *d_in, size_t n,
   return dx_undexta_dev(ctx,DX_ARROW,d_in,n,o->width,0,*d_out,cap + 64,out_len);
 }
 
+static int stream(dx_win *w) { return dx_stream_unpack(w,DX_ARROW); }
+
 int main(int argc, char *argv[])
 { static const dx_tool tool =
     { "undexar", "[-vk] [-w<int(80)>] ( -i | <path:dexar> ... )", "vki", 1, ".dexar", ".arrow",
       { "      -i: source is on standard input.",
         "      -k: do *not* remove the .dexar file on completion.",
-        "      -w: line width for arrow lines.", NULL, NULL }, run };
+        "      -w: line width for arrow lines.", NULL, NULL }, run, stream, 10.0 };
   return dx_cli_main(&tool,argc,argv);
 }

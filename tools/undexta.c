@@ -13,12 +13,14 @@ static int run(dx_ctx *ctx, const dx_opts *o, const uint8_t *d_in, size_t n,
   return dx_undexta_dev(ctx,DX_FASTA,d_in,n,o->width,o->upper,*d_out,cap + 64,out_len);
 }
 
+static int stream(dx_win *w) { return dx_stream_unpack(w,DX_FASTA); }
+
 int main(int argc, char *argv[])
 { static const dx_tool tool =
     { "undexta", "[-vkU] [-w<int(80)>] ( -i | <path:dexta> ... )", "vkiU", 1, ".dexta", ".fasta",
       { "      -i: source is on standard input.",
         "      -k: do *not* remove the .dexta file on completion.",
         "      -U: use uppercase letters (default is lower case).",
-        "      -w: line width for sequence lines.", NULL }, run };
+        "      -w: line width for sequence lines.", NULL }, run, stream, 10.0 };
   return dx_cli_main(&tool,argc,argv);
 }
