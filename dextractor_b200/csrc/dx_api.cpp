@@ -1466,9 +1466,9 @@ static void build_dec_tables(const dx_qv_coding *c, QvDecTables *t)
     }
 }
 
-// Two-level tables for the parallel decoder.  false if a table needs more sub-tables than fit
-// (then the sequential kernels of dx_qv_decode.cu take over).
-static bool build_dec_tables2(const dx_qv_coding *c, QvDecTables2 *t)
+// Two-level tables for the warp-per-entry decoder.  A scheme has at most 256 codes, so it never
+// needs more than DX_DEC2_MAXSUB sub-tables.
+static void build_dec_tables2(const dx_qv_coding *c, QvDecTables2 *t)
 { memset(t,0,sizeof(*t));
   for (int k = 0; k < 6; k++)
     { const dx_scheme &s = c->tab[k];
@@ -1486,8 +1486,7 @@ static bool build_dec_tables2(const dx_qv_coding *c, QvDecTables2 *t)
             { const uint32_t pre = (s.bits[i] >> (len - 11)) & 0x7ffu;
               uint16_t &pe = t->prim[k][pre];
               if (!(pe & 0x8000u))
-                { if (nsub >= DX_DEC2_MAXSUB) return false;
-                  pe = (uint16_t) (0x8000u | nsub);
+                { pe = (uint16_t) (0x8000u | nsub);
                   nsub++;
                 }
               const uint32_t idx = pe & 0x7fffu;
@@ -1496,16 +1495,15 @@ static bool build_dec_tables2(const dx_qv_coding *c, QvDecTables2 *t)
             }
         }
     }
-  return true;
 }
 
 // 12-bit shared-memory tables for the parallel decoders.  A code of at most 12 bits owns the range
 // of 12-bit windows it is a prefix of; filling the ranges in ascending symbol order resolves the
 // ties of a type-2 scheme (symbols folded onto the escape share its code) exactly as the
 // reference's 16-bit LUT does: 255 wins (QV.c:365-372).
-static bool build_dec_tables4(const dx_qv_coding *c, QvDecTables4 *t)
+static void build_dec_tables4(const dx_qv_coding *c, QvDecTables4 *t)
 { memset(t,0,sizeof(*t));
-  if (!build_dec_tables2(c,&t->t2)) return false;
+  build_dec_tables2(c,&t->t2);
   double ab[6], erun[6];
   for (int k = 0; k < 6; k++)
     { const dx_scheme &s = c->tab[k];
@@ -1573,7 +1571,6 @@ static bool build_dec_tables4(const dx_qv_coding *c, QvDecTables4 *t)
   t->abits[2] = (float) ab[2];
   t->abits[3] = (float) ab[3];
   t->abits[4] = (float) (c->subchar >= 0 ? (ab[4] + ab[5]) / (erun[5] + 1.0) : ab[4]);
-  return true;
 }
 
 // bits a position takes at least: the shortest ins code plus the shortest mrg code (never run-length coded)
@@ -1597,21 +1594,19 @@ static int qv_copy(dx_ctx *ctx, bool by_kernel, void *dst, const void *src, size
 }
 
 // The 12-bit decode tables of a coding, copied to d_tab4 through a temporary buffer (h4 == NULL, synchronous)
-// or by qv_copy from pinned h4.  *fits = false: more long codes than the tables hold, nothing is copied.
-static int qv_tables4(dx_ctx *ctx, const dx_qv_coding *c, QvDecTables4 *h4, bool by_kernel,
-                      QvDecTables4 *d_tab4, bool *fits)
+// or by qv_copy from pinned h4.
+static int qv_tables4(dx_ctx *ctx, const dx_qv_coding *c, QvDecTables4 *h4, bool by_kernel, QvDecTables4 *d_tab4)
 { QvDecTables4 *h = h4 ? h4 : (QvDecTables4 *) malloc(sizeof(QvDecTables4));
   if (h == NULL) return DX_E_NOMEM;
-  int rc = DX_OK;
-  *fits = build_dec_tables4(c,h);
-  if (*fits) rc = h4 ? qv_copy(ctx,by_kernel,d_tab4,h,sizeof(QvDecTables4)) : upload(ctx,d_tab4,h,1);
+  build_dec_tables4(c,h);
+  const int rc = h4 ? qv_copy(ctx,by_kernel,d_tab4,h,sizeof(QvDecTables4)) : upload(ctx,d_tab4,h,1);
   if (h4 == NULL) free(h);
   return rc;
 }
 
 struct QvPlan
 { std::vector<QvDecEntry> ent;
-  bool         v2;            // parallel decoders usable (tables fit shared memory)
+  bool         v2;            // the parallel decoders (not the sequential kernels of dx_qv_decode.cu)
   QvDecTables4 *d_tab4;
   int64_t     *d_soff;        // v1 only: [count][6] device
   int64_t     *d_start;       // v2: first stream byte of every entry
@@ -1809,12 +1804,11 @@ static int plan_undexqv(dx_ctx *ctx, const uint8_t *d_in, size_t n, const int64_
   plan.d_soff = NULL; plan.d_start = NULL; plan.d_rlen = NULL; plan.d_tab = NULL;
   plan.spec = false; plan.d_tmp = NULL; plan.tmp_n = 0; plan.src.clear();
 
-  plan.v2 = false; plan.d_tab4 = NULL;
-  if (ctx->route[DXR_DECODER] != 1 && !legacy)
-    { // 12-bit shared-memory tables for the parallel kernels; a coding they cannot hold (more long
-      // codes than the sub-tables take) is decoded by the sequential kernels of dx_qv_decode.cu
-      if ((plan.d_tab4 = (QvDecTables4 *) dx_arena_get(ctx,sizeof(QvDecTables4))) == NULL) return DX_E_NOMEM;
-      if ((rc = qv_tables4(ctx,&plan.coding,NULL,false,plan.d_tab4,&plan.v2)) != DX_OK) return rc;
+  plan.v2 = (ctx->route[DXR_DECODER] != 1 && !legacy);
+  plan.d_tab4 = NULL;
+  if (plan.v2)
+    { if ((plan.d_tab4 = (QvDecTables4 *) dx_arena_get(ctx,sizeof(QvDecTables4))) == NULL) return DX_E_NOMEM;
+      if ((rc = qv_tables4(ctx,&plan.coding,NULL,false,plan.d_tab4)) != DX_OK) return rc;
     }
   if (!plan.v2)
     { QvDecTables *h_tab = (QvDecTables *) malloc(sizeof(QvDecTables));
@@ -2179,8 +2173,7 @@ static void set_last_index(dx_ctx *ctx, size_t N, const QvDecEntry *ent, const i
 //  The usual case of dx_undexqv_dev with everything but the verification of the entry chain on the
 //  device (dx_qv_plan.cu): well numbers and text offsets are prefix sums, the host sees a few
 //  bytes per entry through pinned memory.  Returns *handled = false (nothing written) when the
-//  file needs the general path below: decode tables that do not fit the one-warp-per-entry
-//  kernel, or an entry the candidate filter missed.
+//  file needs the general path below: an entry the candidate filter missed.
 // ------------------------------------------------------------------------------------------------
 static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, uint8_t *d_out, size_t cap,
                         size_t *out_len, const int64_t *h_entry_off, int64_t nentries, int32_t well_in,
@@ -2204,8 +2197,7 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
   if (!d_tab4 || !d_prefix || !d_flag) return DX_E_NOMEM;
   // the decode tables are host work (~0.1 ms): with a known entry index they are built while the
   // planning kernels run
-  bool tables_ok = true;
-  auto make_tables = [&]() -> int { return qv_tables4(ctx,&coding,h4,false,d_tab4,&tables_ok); };
+  auto make_tables = [&]() -> int { return qv_tables4(ctx,&coding,h4,false,d_tab4); };
   // ... and while the candidate index runs when there is none
   struct Deferred { decltype(make_tables) *fn; int rc; } deferred = { &make_tables, DX_OK };
   char *h_prefix = (char *) dx_hpin_get(ctx,(size_t) plen + 1);
@@ -2251,7 +2243,6 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
       DX_CUDA(ctx,cudaMemcpyAsync(&h_tail->flag,d_flag,4,cudaMemcpyDeviceToHost,ctx->stream));
       DX_CUDA(ctx,cudaStreamSynchronize(ctx->stream));
       ph.mark("plan");
-      if (!tables_ok) return DX_OK;                          // tables that need the general path
       if (h_tail->flag == 1) return dx_fail(ctx,DX_E_TRUNC,"compressed image ends inside an entry header");
       if (h_tail->flag == 2) return dx_fail(ctx,DX_E_FORMAT,"unusable read length in an entry header");
       if ((size_t) h_tail->total > cap)
@@ -2289,7 +2280,6 @@ static int undexqv_fast(dx_ctx *ctx, const uint8_t *d_in, size_t n, int upper, u
     }
   if (rc != DX_OK) return rc;
   if (deferred.rc != DX_OK) return deferred.rc;
-  if (!tables_ok) return DX_OK;
   ph.mark("index");
   const size_t N = (size_t) nc;
   if (N == 0) return DX_OK;                             // empty or all entries missed: general path
@@ -2512,10 +2502,7 @@ extern "C" int dx_qv_load_entries_dev(dx_ctx *ctx, const uint8_t *d_in, size_t n
     return dx_fail_cap(ctx,(size_t) (toff[N]),cap);
   QvDecTables4 *d_tab4 = (QvDecTables4 *) dx_arena_get(ctx,sizeof(QvDecTables4));
   if (d_tab4 == NULL) return DX_E_NOMEM;
-  bool fits = false;
-  if ((rc = qv_tables4(ctx,coding,NULL,false,d_tab4,&fits)) != DX_OK) return rc;
-  if (!fits)
-    return dx_fail(ctx,DX_E_CODING,"dx_qv_load_entries_dev: the coding has more long codes than the decode tables hold");
+  if ((rc = qv_tables4(ctx,coding,NULL,false,d_tab4)) != DX_OK) return rc;
   int64_t *d_start = (int64_t *) dx_arena_get(ctx,N*8);
   int32_t *d_rlen  = (int32_t *) dx_arena_get(ctx,N*4);
   int64_t *d_toff  = (int64_t *) dx_arena_get(ctx,(N+1)*8);
@@ -2650,7 +2637,6 @@ static void qv_range_free(dx_ctx *ctx)
   ctx->qv_range = NULL;
 }
 
-// d_tab4 == NULL after a successful call: the coding has more long codes than the 12-bit tables hold
 static int qv_range_setup(dx_ctx *ctx, const QvHead &hd, int upper, bool by_kernel, QvRange &R)
 { R.coding = hd.coding; R.plen = hd.plen; R.first = (int64_t) hd.first; R.upper = upper;
   R.by_kernel = by_kernel; R.minbits = qv_minbits(hd.coding);
@@ -2661,10 +2647,8 @@ static int qv_range_setup(dx_ctx *ctx, const QvHead &hd, int upper, bool by_kern
   R.d_flag   = (int32_t *) dx_arena_get(ctx,16);
   R.h_tail   = (QvTail *) dx_hpin_get(ctx,sizeof(QvTail));
   if (!h4 || !h_prefix || !R.d_tab4 || !R.d_prefix || !R.d_flag || !R.h_tail) return DX_E_NOMEM;
-  bool fits = false;
   int rc;
-  if ((rc = qv_tables4(ctx,&hd.coding,h4,by_kernel,R.d_tab4,&fits)) != DX_OK) return rc;
-  if (!fits) { R.d_tab4 = NULL; return DX_OK; }
+  if ((rc = qv_tables4(ctx,&hd.coding,h4,by_kernel,R.d_tab4)) != DX_OK) return rc;
   memcpy(h_prefix,hd.prefix.data(),(size_t) R.plen + 1);
   if ((rc = qv_copy(ctx,by_kernel,R.d_prefix,h_prefix,(size_t) R.plen + 1)) != DX_OK) return rc;
   DX_CUDA(ctx,cudaMemsetAsync(R.d_flag,0,16,ctx->stream));
@@ -2849,9 +2833,6 @@ extern "C" int dx_undexqv_range_dev(dx_ctx *ctx, const uint8_t *h_head, size_t h
   if (ctx->qv_range == NULL) return DX_E_NOMEM;
   QvRange &R = *(QvRange *) ctx->qv_range;
   if ((rc = qv_range_setup(ctx,hd,upper,false,R)) != DX_OK) return rc;
-  if (R.d_tab4 == NULL)
-    return dx_fail(ctx,DX_E_CODING,"the coding has more long codes than the parallel decode tables hold; decode this "
-                   "image whole with dx_undexqv_dev");
   if (B == A)                                             // a range inside the header: no entry starts there
     rc = qv_range_decode(ctx,R,d_buf,0,buf_off,A,B);
   else
@@ -2892,9 +2873,9 @@ extern "C" int dx_undexqv_range_text_dev(dx_ctx *ctx, uint8_t *d_out, size_t cap
 //  successor have arrived (an entry may run over the boundary), and a window's text leaves for the
 //  host (copy stream cs_out) while the next window is decoded: PCIe is busy in both directions and
 //  the kernels hide behind the copies.  The chain carries its position, well number and text offset
-//  from window to window.  Anything unusual (legacy layout, tables that do not fit, an entry longer
-//  than the bytes that have arrived, a malformed image) -> *handled = false after the copies have
-//  drained, and the caller runs the plain path on the complete image.
+//  from window to window.  Anything unusual (legacy layout, an entry longer than the bytes that have
+//  arrived, a malformed image) -> *handled = false after the copies have drained, and the caller runs
+//  the plain path on the complete image.
 // ------------------------------------------------------------------------------------------------
 static int pipe_setup(dx_ctx *ctx, int nev)
 { if (ctx->cs_in == NULL)  DX_CUDA(ctx,cudaStreamCreateWithFlags(&ctx->cs_in,cudaStreamNonBlocking));
@@ -2940,7 +2921,7 @@ static int undexqv_pipe(dx_ctx *ctx, const uint8_t *h_in, size_t n, int upper, u
                        cudaStreamSynchronize(ctx->stream); };
 
   QvRange R;
-  if ((rc = qv_range_setup(ctx,hd,upper,true,R)) != DX_OK || R.d_tab4 == NULL) { drain(); return rc; }
+  if ((rc = qv_range_setup(ctx,hd,upper,true,R)) != DX_OK) { drain(); return rc; }
 
   int64_t cur = (int64_t) hd.first;        // image offset of the next entry (chain position)
   int32_t well = 0;

@@ -46,7 +46,9 @@ struct QvDecTables
 // Compact two-level decode tables for the parallel decoders (dx_qv_decode5.cu, dx_qv_decode6.cu): the
 // top 11 bits of the 16-bit window index prim; codes longer than 11 bits go through a 32-entry
 // sub-table.  entry = symbol | length << 8 ; bit 15 of a prim entry = "low 15 bits are a sub-table index".
-#define DX_DEC2_MAXSUB 64
+// One sub-table per distinct 11-bit prefix of a code of 12..16 bits: a scheme has at most 256 codes,
+// so 256 sub-tables hold every coding.
+#define DX_DEC2_MAXSUB 256
 struct QvDecTables2
 { uint16_t prim[6][2048];
   uint16_t sub[6][DX_DEC2_MAXSUB*32];

@@ -305,9 +305,9 @@ int dx_undexqv_size_dev(dx_ctx *ctx, const uint8_t *d_in, size_t n, size_t *out_
  *                              NULL with cap 0 to ask).  Waits for the context's stream.
  *
  * The text of consecutive ranges, each chained from where the one before it ended, concatenated, is the
- * text of dx_undexqv_dev on the whole image.  Images of the old layout or the other byte order, and codings
- * whose long codes do not fit the parallel decoder's tables, are refused (DX_E_FORMAT / DX_E_CODING):
- * decode them whole with dx_undexqv_dev. */
+ * text of dx_undexqv_dev on the whole image.  Every coding is taken, codes of up to 16 bits included.
+ * Images of the old layout or the other byte order are refused (DX_E_FORMAT): decode them whole with
+ * dx_undexqv_dev. */
 int dx_undexqv_range_dev(dx_ctx *ctx, const uint8_t *h_head, size_t head_n, const uint8_t *d_buf,
                          size_t buf_n, int64_t buf_off, int64_t a, int64_t b, int upper, int64_t *first);
 int dx_undexqv_range_chain(dx_ctx *ctx, int64_t cur_in, int32_t well_in, int64_t *cur_out,

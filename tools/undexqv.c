@@ -46,7 +46,6 @@ static int stream(dx_win *w)
           if (b <= a) { lim *= 2; dx_win_fill(w,lim); continue; }
           rc = dx_undexqv_range_dev(ctx,head,head_n,w->d,buf_n,w->off,a,b,w->o->upper,&first);
           if (rc == DX_OK) rc = dx_sync(ctx);
-          if (rc == DX_E_CODING && cur < 0) return DX_WHOLE;   /* long codes: the whole-image decoder */
           if (rc == DX_E_NOMEM && w->size > ((size_t) 64 << 10)) { w->size /= 2; lim = w->size; continue; }
           if (rc != DX_OK) dx_cli_die(ctx,rc);
           rc = dx_undexqv_range_chain(ctx,cur < 0 ? first : cur,well,&cur_out,&well_out);

@@ -13,8 +13,8 @@
  *                                 memory and a condition variable: a few scalars, no NCCL);
  *   3. dx_undexqv_range_text_dev  every rank at once: its text, written with pwrite at the sum of the
  *                                 text sizes of the ranks before it.
- * An image of the old layout or the other byte order, one whose coding the parallel decoder cannot
- * hold, and a file smaller than N MB are decoded by rank 0 alone (dx_undexqv_dev).
+ * An image of the old layout or the other byte order, and a file smaller than N MB, are decoded by
+ * rank 0 alone (dx_undexqv_dev).
  * Same file naming, flags, messages and exit codes as undexqv; the source is removed only after the
  * output is completely written.  Host code is plain C; every codec step runs on the GPUs.
  */
@@ -50,7 +50,7 @@ typedef struct                               /* one file, shared by its ranks */
     size_t          head_n;
     pthread_mutex_t mu;
     pthread_cond_t  cv;
-    int             chain_ready[MAXGPU+1], text_ready[MAXGPU+1], whole;
+    int             chain_ready[MAXGPU+1], text_ready[MAXGPU+1];
     int64_t         cur[MAXGPU+1], tsize[MAXGPU+1];
     int32_t         well[MAXGPU+1];
   } Job;
@@ -136,11 +136,6 @@ static void *rank_main(void *arg)
       R->t_read += now() - t0; t0 = now();
       rc = dx_undexqv_range_dev(ctx,J->head,J->head_n,d_buf,(size_t) (to - from),from,a,b,J->o->upper,&first);
       if (rc == DX_OK) rc = dx_sync(ctx);
-      if (rc == DX_E_CODING)                               /* the same coding on every rank: all get here */
-        { pthread_mutex_lock(&J->mu); J->whole = 1; pthread_cond_broadcast(&J->cv); pthread_mutex_unlock(&J->mu);
-          dx_device_free(ctx,d_buf); dx_pinned_free(ctx,stage); dx_close(ctx);
-          return NULL;
-        }
       if (rc != DX_OK) die(ctx,rc);
       R->t_decode += now() - t0; t0 = now();
 
@@ -148,11 +143,9 @@ static void *rank_main(void *arg)
       if (r == 0) { cur = first; well = 0; }
       else
         { pthread_mutex_lock(&J->mu);
-          while (!J->chain_ready[r] && !J->whole) pthread_cond_wait(&J->cv,&J->mu);
+          while (!J->chain_ready[r]) pthread_cond_wait(&J->cv,&J->mu);
           cur = J->cur[r]; well = J->well[r];
-          const int whole = J->whole;
           pthread_mutex_unlock(&J->mu);
-          if (whole) { dx_device_free(ctx,d_buf); dx_pinned_free(ctx,stage); dx_close(ctx); return NULL; }
         }
       const double tw = now();
       rc = dx_undexqv_range_chain(ctx,cur,well,&cur_out,&well_out);
@@ -298,26 +291,26 @@ int main(int argc, char *argv[])
       if (o.verbose) { fprintf(stderr,"Processing '%s' ...\n",root); fflush(stderr); }
       pthread_mutex_init(&J.mu,NULL); pthread_cond_init(&J.cv,NULL);
       /* rank 0 alone: not the native 0x55aa layout (the old layout, the other byte order), or too small */
-      J.whole = !(J.head_n >= 2 && J.head[0] == 0xaa && J.head[1] == 0x55) || J.fsize < (int64_t) o.world << 20;
-      if (!J.whole)
+      const int whole = !(J.head_n >= 2 && J.head[0] == 0xaa && J.head[1] == 0x55) || J.fsize < (int64_t) o.world << 20;
+      if (whole)
+        { if (o.verbose)
+            { fprintf(stderr,"  %s: rank 0 decodes the file alone\n",
+                      J.fsize < (int64_t) o.world << 20 ? "smaller than 1 MB per GPU" : "old layout or other byte order");
+              fflush(stderr);
+            }
+          decode_whole(&J);
+        }
+      else
         { for (k = 0; k < o.world; k++)
             { memset(&R[k],0,sizeof(Rank));
               R[k].rank = k; R[k].J = &J;
               if (pthread_create(&th[k],NULL,rank_main,&R[k]) != 0) { fprintf(stderr,"%s: pthread_create failed\n",Prog); exit (1); }
             }
           for (k = 0; k < o.world; k++) pthread_join(th[k],NULL);
-          if (J.whole && ftruncate(J.fd_out,0) != 0) { fprintf(stderr,"%s: System error, write failed!\n",Prog); exit (2); }
-          if (J.whole && o.verbose) fprintf(stderr,"  the coding does not fit the parallel decoder's tables: ");
-        }
-      else if (o.verbose)
-        fprintf(stderr,"  %s: ",J.fsize < (int64_t) o.world << 20 ? "smaller than 1 MB per GPU" : "old layout or other byte order");
-      if (J.whole)
-        { if (o.verbose) { fprintf(stderr,"rank 0 decodes the file alone\n"); fflush(stderr); }
-          decode_whole(&J);
         }
       close(fd_in);
       if (close(J.fd_out) != 0) { fprintf(stderr,"%s: System error, write failed!\n",Prog); exit (2); }
-      if (o.verbose && !J.whole)
+      if (o.verbose && !whole)
         { double tr = 0, td = 0, tc = 0, tt = 0, tw = 0; int64_t rb = 0, wb = 0;
           for (k = 0; k < o.world; k++)
             { if (R[k].t_read > tr)   tr = R[k].t_read;
